@@ -2,7 +2,7 @@
 """bench.py - env-steps/s of the fused batched GridEnvironment.step on B200.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload ieee123|ieee13|ieee34|...] [--lanes L]
-                  [--scaling weak|strong] [--no-configs] [--no-cpu]
+                  [--scaling weak|strong] [--no-configs] [--no-cpu] [--dump-outputs DIR]
   python bench.py --impl reference ...      # the CPU oracle (port of the reference path) on host cores
 
 One JSON line on stdout (rank 0).  A "step" is one pass of the hot path over one batch of
@@ -350,9 +350,10 @@ def measure_device(m, lib, name, B, dev, world, rank, lanes, seed, K, W, max_ove
     R = 4
     actions = [env.sample_actions(gen) for _ in range(R)]
     E = len(envs)
+    last = [None]
 
     def dev_step(i):
-        envs[i % E].step(actions[i % R])
+        last[0] = envs[i % E].step(actions[i % R])
 
     for i in range(max(W, E)):
         dev_step(i)
@@ -389,7 +390,33 @@ def measure_device(m, lib, name, B, dev, world, rank, lanes, seed, K, W, max_ove
                      "kernel": f"step_kernel<{li['lanes']},{solver}>", "kernel_ms": ms / K},
         "gpu_launches": int(launches),
     }
-    return res, envs, actions
+    return res, envs, actions, last[0]
+
+
+DUMP_BYTES = 60_000_000      # array data of one --dump-outputs directory (64 MB with the .npy headers, with room)
+
+
+def dump_outputs(out_dir, outputs, limit=DUMP_BYTES):
+    """Writes one step's outputs - what ``BatchedGridEnvironment.step`` returns: observation, reward, the two done
+    flags and every tensor of ``info`` - as ``<out_dir>/<name>.npy``, so that two builds can be compared output for
+    output.  Every array keeps the same instances (rows): all of them when they fit in ``limit`` bytes, else a sorted
+    sample drawn with a fixed seed; ``rows.npy`` lists them.  fp32 / fp64 arrays keep their type, flags and counters
+    become fp64 (exactly)."""
+    import numpy as np
+    import torch
+    obs, reward, terminated, truncated, info = outputs
+    arrays = {"obs": obs, "reward": reward, "terminated": terminated, "truncated": truncated}
+    arrays.update((k, v) for k, v in info.items() if isinstance(v, torch.Tensor))
+    arrays = {k: v if v.dtype in (torch.float32, torch.float64) else v.to(torch.float64) for k, v in arrays.items()}
+    B = obs.shape[0]
+    row_bytes = 8 + sum(v[0].numel() * v.element_size() for v in arrays.values())
+    n = min(B, limit // row_bytes)
+    rows = np.arange(B) if n == B else np.sort(np.random.default_rng(0).choice(B, size=n, replace=False))
+    idx = torch.as_tensor(rows, device=obs.device)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "rows.npy"), rows.astype(np.float64))
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v.index_select(0, idx).cpu().numpy())
 
 
 def run_gpu(args):
@@ -423,8 +450,10 @@ def run_gpu(args):
 
     sampler = ClockSampler(physical_gpu_index(local))
     sampler.start()
-    main, envs, actions = measure_device(m, lib, args.workload, B, dev, world, rank, args.lanes, args.seed, K, W,
-                                         max_over_ranks, peak, facts)
+    main, envs, actions, last = measure_device(m, lib, args.workload, B, dev, world, rank, args.lanes, args.seed, K, W,
+                                               max_over_ranks, peak, facts)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)       # before the end-to-end arms step the environment again
     env = envs[0]
     value, ms = main["value"], main["ms_per_step"] * K
     if args.kernel_only:                 # tuning aid (tools/): the device-resident arm only
@@ -508,7 +537,7 @@ def run_gpu(args):
                 continue
             Bn = WORKLOADS[name][1]
             Kn = max(20, min(K, 200))
-            res, es, _ = measure_device(m, lib, name, Bn, dev, world, rank, 0, args.seed, Kn, W, max_over_ranks, peak, facts)
+            res, es, _, _ = measure_device(m, lib, name, Bn, dev, world, rank, 0, args.seed, Kn, W, max_over_ranks, peak, facts)
             for e in es:
                 e.close()
             others[name] = res
@@ -594,7 +623,9 @@ def measure_rollout(m, dev, world, rank, max_over_ranks, args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200,
+                    help="timed steps of the headline workload (its device-resident and end-to-end arms); the other "
+                         "configurations and the observation arms report their own step counts")
     ap.add_argument("--warmup", type=int, default=10)
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default="ieee123", choices=sorted(WORKLOADS))
@@ -607,7 +638,14 @@ def main():
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="weak: the workload's per-GPU size on every GPU; strong: --total-envs (1,048,576) split over the GPUs")
     ap.add_argument("--total-envs", type=int, default=0, help="instances in total for --scaling strong")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the headline workload's last timed step to DIR/<name>.npy (rank 0's "
+                         "instances; a fixed sample of them when they exceed 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's outputs; --impl reference has none")
     if args.impl == "reference":
         run_reference(args)
     else:
