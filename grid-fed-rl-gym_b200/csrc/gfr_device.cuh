@@ -45,7 +45,8 @@ enum { GEN_SOLAR = 0, GEN_WIND = 1 };
 //            (L D^-1 U, L D^-1 r) and its branch's share of the parent's calculated injection stay in
 //            REGISTERS, and the parent's correction comes back down the same way.  Only the other
 //            children go through a pool slot (planned by the host: held from the child's row up to the
-//            parent's; field 0 carries the correction on the way down).  D^-1 U and D^-1 r, only needed
+//            row that reads it - the sibling that absorbs it into its chain, or the parent; field 0 of a
+//            slot planned for the back-substitution carries the correction on the way down).  D^-1 U and D^-1 r, only needed
 //            again in the back-substitution, and the specified injections live in a per-slot scratch
 //            in global memory, by position, that stays L2 resident; the back-substitution loads them
 //            two rows ahead into registers.
@@ -63,7 +64,7 @@ enum { FL_PQ = 1, FL_FROM_IS_PARENT = 2, FL_FIXED_VM = 4, FL_THETA = 8,     // P
        FL_VALID = 128,                                                    // the schedule position holds a bus
        FL_POOL_SHIFT = 8, FL_POOL_MASK = 0xFFF,                           // bits 8..19: the bus's pool slot
        FL_XSLOT_SHIFT = 20,                                               // bits 20..31: the slot its parent's correction arrives in
-       REC_LIST_MASK = 0xFFFFF, REC_KIDX_SHIFT = 20 };                    // word y: child list begin | slot this bus puts ITS correction in << 20
+       REC_LIST_MASK = 0xFFFFF, REC_KIDX_SHIFT = 20 };                    // word y: tail list begin | 1 + slot this bus puts ITS correction in << 20
 // record (persistent per-instance state) slots, in doubles
 enum { R_TIME = 0, R_FREQ, R_WIND, R_TEMP, R_CLOUD, R_TOTAL_LOSSES, R_EPISODE_REWARD, R_SEED,
        R_DRAWS, R_COUNTS, R_BAT };   // soc[Bt] then bpow[Bt] from R_BAT on
@@ -72,18 +73,26 @@ struct alignas(16) D2 { double x, y; };
 struct alignas(16) I4 { int x, y, z, w; };   // per-bus topology: parent, child list begin, end, flags
 GFR_HD int pool_slot_of(int w) { return (w >> FL_POOL_SHIFT) & FL_POOL_MASK; }
 // A schedule record (one per position p = row * lanes + lane, 16 bytes):
-//   x = bus k | parent's k << 16 (indices into ef)      y = first entry of the bus's child list | slot for its correction << 20
-//   z = flags | pool slot << 8 | correction slot << 20   w = children handed over through the pool | all children << 16
-// The child list (child_ent, child_slot) holds the heir first - if there is one - then the others.
-// On the way down a bus with children behind pool slots writes its correction ONCE, into the slot of the child
-// that holds its slot longest (the one eliminated first); every such child reads it there (z: correction slot).
+//   x = bus k | parent's k << 16 (indices into ef)      y = first entry of the bus's tail list | 1 + slot for its correction << 20
+//   z = flags | pool slot << 8 | correction slot << 20   w = chain tails it gathers | 1 + slot it absorbs << 16
+// The children handed over through the pool are summed along sibling chains (the host's plan): a child may
+// ABSORB the partial sum of one sibling eliminated in an earlier row (add that sibling's slot to its own
+// hand-off), and the bus gathers only the chain tails nobody absorbed, listed in child_slot.
+// On the way down a bus with children behind pool slots writes its correction ONCE, into a slot planned for
+// the back-substitution alone; every such child reads it there (z: correction slot).  0 in a "1 + slot" = none.
 GFR_HD int rec_bus(const I4& t) { return (int)((unsigned)t.x & 0xFFFFu); }
 GFR_HD int rec_parent(const I4& t) { return (int)((unsigned)t.x >> 16); }
 GFR_HD int rec_list(const I4& t) { return t.y & REC_LIST_MASK; }
-GFR_HD int rec_kids_x_slot(const I4& t) { return (int)((unsigned)t.y >> REC_KIDX_SHIFT); }
+GFR_HD int rec_kids_x_slot(const I4& t) { return (int)((unsigned)t.y >> REC_KIDX_SHIFT) - 1; }
 GFR_HD int x_slot_of(int z) { return (int)((unsigned)z >> FL_XSLOT_SHIFT); }
-GFR_HD int rec_pool_kids(const I4& t) { return (int)((unsigned)t.w & 0xFFFFu); }
-GFR_HD int rec_all_kids(const I4& t) { return (int)((unsigned)t.w >> 16); }
+GFR_HD int rec_tails(const I4& t) { return (int)((unsigned)t.w & 0xFFFFu); }
+GFR_HD int rec_absorb(const I4& t) { return (int)((unsigned)t.w >> 16) - 1; }
+// Groups of 8 lanes and more sum along sibling chains: there a warp holds at most four groups, and a hub's pool
+// children gathered on one lane kept the others waiting.  Smaller groups keep the parent gathering every pool child
+// (no absorb step compiled in, no chains planned): measured on a B200, the absorb step cost IEEE-13 on 2 lanes 2.2 %
+// and IEEE-34 on 2 lanes 0.4 %, more than their few gather iterations saved.
+enum { CHAIN_MIN_LANES = 8 };
+template <int LANES> GFR_HD constexpr bool sibling_chains() { return LANES >= CHAIN_MIN_LANES; }
 
 // Where everything is inside the feeder image (ints / doubles counted from the image base)
 // plus the sizes; passed as a kernel parameter (constant bank).
@@ -97,7 +106,7 @@ struct Layout {
   int o_gb, o_rating, o_vm_set;
   // Newton
   int o_child_ent, o_child_slot, o_gbd, o_f0;
-  int o_kids;                    // CTA-wide groups: the pool slots of a position's first 8 pool children, 16 bits each (one I4)
+  int o_kids;                    // CTA-wide groups: the pool slots of a position's first 8 chain tails, 16 bits each (one I4)
   // sweep (compact per-bus arrays)
   int o_topo, o_child_idx, o_rx;
   int o_rowrec, sw_rows;         // several lanes: one record per (row, lane) = (bus | parent << 16, child list begin, end, flags)
@@ -620,13 +629,13 @@ GFR_HD BranchT branch_terms(const D2 vk, const D2 vp, const D2 y) {
   return t;
 }
 
-// The pool slots of a position's children behind pool slots, one after the other in `slot` for the body given last.  CTA-wide groups
+// The pool slots of a position's chain tails, one after the other in `slot` for the body given last.  CTA-wide groups
 // read their image from global memory: there the first 8 slots come packed in a record (kq_) that travels one row
 // ahead with the position's own record, which takes the list's L2 round trip off every row's critical path.
 GFR_HD unsigned shr16_pair(unsigned lo, unsigned hi) { return (lo >> 16) | (hi << 16); }
 #define GFR_POOL_GATHER(t_, kq_, ...)                                                                              \
   do {                                                                                                             \
-    const int npk_ = rec_pool_kids(t_);                                                                            \
+    const int npk_ = rec_tails(t_);                                                                                \
     if (wide_group<LANES>() && npk_ <= 8) {                                                                       \
       unsigned w0_ = (unsigned)(kq_).x, w1_ = (unsigned)(kq_).y, w2_ = (unsigned)(kq_).z, w3_ = (unsigned)(kq_).w; \
       _Pragma("unroll 1")                                                                                          \
@@ -636,9 +645,9 @@ GFR_HD unsigned shr16_pair(unsigned lo, unsigned hi) { return (lo >> 16) | (hi <
         __VA_ARGS__                                                                                                \
       }                                                                                                            \
     } else {                                                                                                       \
-      const int q1_ = rec_list(t_) + rec_all_kids(t_);                                                             \
+      const int q0_ = rec_list(t_);                                                                                \
       _Pragma("unroll 1")                                                                                          \
-      for (int q_ = q1_ - npk_; q_ < q1_; ++q_) {                                                                  \
+      for (int q_ = q0_; q_ < q0_ + npk_; ++q_) {                                                                  \
         const int slot = child_slot[q_];                                                                           \
         __VA_ARGS__                                                                                                \
       }                                                                                                            \
@@ -713,6 +722,10 @@ GFR_HD double newton_mismatch(const NGrp<LANES>& g, const Layout& lay, const int
       const double loc = (aQ > aP || aQ != aQ) ? aQ : aP;
       mm = (loc > mm || loc != loc) ? loc : mm;
       hf.x = bt.gl; hf.y = bt.ll;
+      if (sibling_chains<LANES>() && rec_absorb(t) >= 0) {                         // the partial of an earlier sibling's chain
+        const D2 fl = g.poolp[3 * np + rec_absorb(t)];
+        hf.x += fl.x; hf.y += fl.y;
+      }
       if (!(t.z & FL_P_REG)) g.poolp[3 * np + pool_slot_of(t.z)] = hf;
     }
     g.sync();
@@ -767,7 +780,7 @@ GFR_HD void newton_back_update(const NGrp<LANES>& g, const Layout& lay, const in
       if (!(t.z & FL_P_REG)) x = g.poolp[x_slot_of(t.z)];                  \
       v.x = fma(-m0.x, x.x, fma(-m0.y, x.y, v.x));                         \
       v.y = fma(-m1.x, x.x, fma(-m1.y, x.y, v.y));                         \
-      if (rec_pool_kids(t)) g.poolp[rec_kids_x_slot(t)] = v;               \
+      if (rec_kids_x_slot(t) >= 0) g.poolp[rec_kids_x_slot(t)] = v;        \
       hx = v;                                                              \
       double sn, cs;                                                       \
       sincos_small(accel * v.x, &sn, &cs);                                 \
@@ -882,6 +895,10 @@ GFR_HD void newton_solve(const NGrp<LANES>& g, const Layout& lay, const int* sim
           v.y = fma(i1.x, r0, i1.y * r1);
           hc.x = fma(lp.x, v.x, lp.y * v.y);
           hc.y = fma(-lp.y, v.x, lp.x * v.y);
+          if (sibling_chains<LANES>() && rec_absorb(t) >= 0) {
+            const D2 cc = g.poolp[2 * np + rec_absorb(t)];
+            hc.x += cc.x; hc.y += cc.y;
+          }
           st_scratch(g.mg + 2 * P + p, v, g.pol);
           if (!(t.z & FL_P_REG)) g.poolp[2 * np + pool_slot_of(t.z)] = hc;
         }
@@ -959,9 +976,6 @@ GFR_HD void newton_solve(const NGrp<LANES>& g, const Layout& lay, const int* sim
           m1.y = fma(i10, u01, i11 * u11);
           v.x = fma(i00, r.x, i01 * r.y);
           v.y = fma(i10, r.x, i11 * r.y);
-          st_scratch(g.mg + p, m0, g.pol);               // needed again in the back-substitution only
-          st_scratch(g.mg + P + p, m1, g.pol);
-          st_scratch(g.mg + 2 * P + p, v, g.pol);
           // handed to the parent: L M, L v, (gl, ll)
           h0.x = fma(bt.ll, m0.x, bt.gl * m1.x);
           h0.y = fma(bt.ll, m0.y, bt.gl * m1.y);
@@ -970,6 +984,15 @@ GFR_HD void newton_solve(const NGrp<LANES>& g, const Layout& lay, const int* sim
           hc.x = fma(bt.ll, v.x, bt.gl * v.y);
           hc.y = fma(-bt.gl, v.x, bt.ll * v.y);
           hf.x = bt.gl; hf.y = bt.ll;
+          if (sibling_chains<LANES>() && rec_absorb(t) >= 0) {                     // the partial of an earlier sibling's chain
+            const D2* e = g.poolp + rec_absorb(t);
+            const D2 c0 = e[0], c1 = e[np], cc = e[2 * np], fl = e[3 * np];
+            h0.x += c0.x; h0.y += c0.y; h1.x += c1.x; h1.y += c1.y; hc.x += cc.x; hc.y += cc.y;
+            hf.x += fl.x; hf.y += fl.y;
+          }
+          st_scratch(g.mg + p, m0, g.pol);               // needed again in the back-substitution only
+          st_scratch(g.mg + P + p, m1, g.pol);
+          st_scratch(g.mg + 2 * P + p, v, g.pol);
           if (!(t.z & FL_P_REG)) {
             D2* const own = g.poolp + pool_slot_of(t.z);
             own[0] = h0; own[np] = h1; own[2 * np] = hc; own[3 * np] = hf;

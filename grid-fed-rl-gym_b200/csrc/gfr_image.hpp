@@ -296,25 +296,71 @@ inline std::string build_feeder_image(const gfr_feeder_desc* d, int lanes, int s
     }
     flags[0] |= FL_P_REG;               // the root has no parent: its "correction from above" is the zero its lane starts with
   }
-  // ---- pool plan (Newton): a slot for every bus whose hand-off goes through shared memory, held from its
-  //      own row up to its parent's.  Slots are handed out row by row; a slot read (released) in one row is
-  //      reused by LATER rows only, and a bus never takes over a slot of its own children - so on the way
-  //      down, when a parent's correction waits in a child's slot for all the children behind slots, nothing
-  //      can overwrite it before the last of them has read it.
+  // ---- sibling chains (Newton): the children handed over through shared memory ("pool children") are summed
+  //      along chains instead of by their parent alone.  Taken in elimination order (rows nrows-1 .. 0), each
+  //      pool child ABSORBS the partial sum of one sibling eliminated in a strictly earlier row - it adds that
+  //      sibling's slot to its own hand-off and writes the sum into its own slot - and the heir absorbs one more
+  //      into the hand-off it passes in registers.  Siblings of one row run in parallel and cannot chain; each
+  //      starts or continues its own chain.  The parent gathers only the chain TAILS nobody absorbed: at most as
+  //      many as it has pool children in one row, instead of all of them on one lane.
+  //      Groups of fewer than CHAIN_MIN_LANES lanes run without chains: every pool child is a tail of its own.
+  std::vector<int> absorb(n, -1), reader_row(n, -1);       // the sibling whose partial a bus absorbs; row its slot is read in
+  std::vector<std::vector<int>> tails(n);                  // per bus: the chain tails it gathers, in summation order
+  if (newton) {
+    std::vector<int> kids;
+    for (int k = 0; k < n; ++k) {
+      kids.clear();
+      for (int q = d->child_ptr[k]; q < d->child_ptr[k + 1]; ++q)
+        if (d->child_idx[q] != heir[k]) kids.push_back(d->child_idx[q]);
+      if (lanes < CHAIN_MIN_LANES) {
+        tails[k] = kids;
+        for (int c : kids) reader_row[c] = sch.row[k];
+        continue;
+      }
+      std::stable_sort(kids.begin(), kids.end(), [&](int a, int b) { return sch.row[a] > sch.row[b]; });
+      std::vector<int>& open = tails[k];                   // chain tails so far, oldest first
+      for (size_t i = 0; i < kids.size();) {
+        const int r = sch.row[kids[i]];
+        size_t j = i;
+        size_t avail = open.size();                        // tails of earlier rows: the ones open before this row
+        std::vector<int> started;
+        for (; j < kids.size() && sch.row[kids[j]] == r; ++j) {
+          const int c = kids[j];
+          if (avail > 0) {
+            absorb[c] = open.front();
+            reader_row[open.front()] = r;
+            open.erase(open.begin());
+            --avail;
+          }
+          started.push_back(c);
+        }
+        open.insert(open.end(), started.begin(), started.end());
+        i = j;
+      }
+      // the heir (row of k + 1, the last row before k's) absorbs the oldest tail unless that one shares its row
+      if (heir[k] >= 0 && !open.empty() && sch.row[open.front()] > sch.row[heir[k]]) {
+        absorb[heir[k]] = open.front();
+        reader_row[open.front()] = sch.row[heir[k]];
+        open.erase(open.begin());
+      }
+      for (int c : open) reader_row[c] = sch.row[k];
+    }
+  }
+  // ---- pool plan (Newton): a slot for every bus whose hand-off goes through shared memory, held from its own
+  //      row up to the row that reads it (the next link of its chain, or its parent).  Slots are handed out row by
+  //      row; a slot read (released) in one row is reused by LATER rows only, so the group barrier that ends a row
+  //      orders every read before the next write.
   std::vector<int32_t> pool_slot(n, 0);
   lay.n_pool = 1;
   if (newton) {
-    std::vector<std::vector<int>> by_row(sch.nrows);
-    for (int k = 0; k < n; ++k) by_row[sch.row[k]].push_back(k);
+    std::vector<std::vector<int>> by_row(sch.nrows), read_in(sch.nrows);
+    for (int k = 0; k < n; ++k) {
+      by_row[sch.row[k]].push_back(k);
+      if (reader_row[k] >= 0) read_in[reader_row[k]].push_back(k);
+    }
     std::vector<int> free_slots;
     int np = 0;
     for (int r = sch.nrows - 1; r >= 0; --r) {
-      std::vector<int> released;
-      for (int k : by_row[r])
-        for (int q = d->child_ptr[k]; q < d->child_ptr[k + 1]; ++q) {
-          const int c = d->child_idx[q];
-          if (c != heir[k]) released.push_back(pool_slot[c]);
-        }
       for (int k : by_row[r]) {
         if (flags[k] & FL_P_REG) continue;            // handed over in registers (or the root)
         if (!free_slots.empty()) {
@@ -325,58 +371,62 @@ inline std::string build_feeder_image(const gfr_feeder_desc* d, int lanes, int s
           pool_slot[k] = np++;
         }
       }
-      free_slots.insert(free_slots.end(), released.begin(), released.end());
+      for (int k : read_in[r]) free_slots.push_back(pool_slot[k]);
     }
     lay.n_pool = std::max(np, 1);
+  }
+  // ---- correction plan (Newton, back-substitution, root -> leaf): a bus with pool children writes its correction
+  //      once, into a slot every such child reads in its own row.  The slot is held from the parent's row to the
+  //      last of those children's rows, and reused from the row after that on.  This pass writes nothing else
+  //      into the pool, and group barriers separate it from the leaf -> root passes.
+  std::vector<int32_t> kids_x_slot(n, -1), x_slot(n, 0);
+  if (newton) {
+    std::vector<int> last_read(n, -1);
+    for (int k = 1; k < n; ++k)
+      if (k != heir[d->parent[k]]) last_read[d->parent[k]] = std::max(last_read[d->parent[k]], sch.row[k]);
+    std::vector<std::vector<int>> by_row(sch.nrows), freed_after(sch.nrows);
+    for (int k = 0; k < n; ++k)
+      if (last_read[k] >= 0) { by_row[sch.row[k]].push_back(k); freed_after[last_read[k]].push_back(k); }
+    std::vector<int> free_slots;
+    int np = 0;
+    for (int r = 0; r < sch.nrows; ++r) {
+      if (r > 0)
+        for (int k : freed_after[r - 1]) free_slots.push_back(kids_x_slot[k]);
+      for (int k : by_row[r]) {
+        if (!free_slots.empty()) {
+          auto it = std::min_element(free_slots.begin(), free_slots.end());
+          kids_x_slot[k] = *it;
+          free_slots.erase(it);
+        } else {
+          kids_x_slot[k] = np++;
+        }
+      }
+    }
+    for (int k = 1; k < n; ++k)
+      if (k != heir[d->parent[k]]) x_slot[k] = kids_x_slot[d->parent[k]];
+    lay.n_pool = std::max(lay.n_pool, np);
     if (d->n_pool > lay.n_pool) lay.n_pool = d->n_pool;      // the caller asks for more (padding experiments)
     if (lay.n_pool > FL_POOL_MASK) return "more than 4095 pool slots";
   }
-  // the slot a bus's correction travels down in: that of the child (among those behind pool slots) eliminated
-  // first - it holds its slot from its own row up to the parent's, which covers its siblings' rows
-  std::vector<int32_t> kids_x_slot(n, 0), x_slot(n, 0);
-  if (newton) {
-    for (int k = 0; k < n; ++k) {
-      int best = -1;
-      for (int q = d->child_ptr[k]; q < d->child_ptr[k + 1]; ++q) {
-        const int c = d->child_idx[q];
-        if (c != heir[k] && (best < 0 || sch.row[c] > sch.row[best])) best = c;
-      }
-      if (best >= 0) {
-        kids_x_slot[k] = pool_slot[best];
-        for (int q = d->child_ptr[k]; q < d->child_ptr[k + 1]; ++q)
-          if (d->child_idx[q] != heir[k]) x_slot[d->child_idx[q]] = pool_slot[best];
-      }
-    }
-  }
 
   ImageBuilder ib;
-  // ---- per-position records + child lists (the heir first, then the children handed over through the pool:
-  //      the order every pass sums them in)
-  std::vector<int32_t> sched(4 * (size_t)P, 0), child_ent, child_slot;
+  // ---- per-position records + tail lists (the slots of the chain tails a bus gathers, in the order every pass
+  //      sums them in: after the heir's hand-off)
+  std::vector<int32_t> sched(4 * (size_t)P, 0), child_slot;
   std::vector<int32_t> topo(4 * (size_t)n);
   for (int p = 0; p < P; ++p) {
     const int k = bus_at[p];
     if (k < 0) continue;
     const int kp = k > 0 ? d->parent[k] : 0;
-    const int begin = (int)child_ent.size();
-    int n_pool_kids = 0, n_all = 0;
-    if (newton) {
-      for (int pass = 0; pass < 2; ++pass)
-        for (int q = d->child_ptr[k]; q < d->child_ptr[k + 1]; ++q) {
-          const int c = d->child_idx[q];
-          if ((c == heir[k]) != (pass == 0)) continue;
-          child_ent.push_back((int32_t)((uint32_t)c | ((uint32_t)pos[c] << 16)));
-          child_slot.push_back(pool_slot[c]);
-          ++n_all;
-          if (pass == 1) ++n_pool_kids;
-        }
-      if (n_all > 65535) return "more than 65535 children on one bus";
-    }
+    const int begin = (int)child_slot.size();
+    for (int c : tails[k]) child_slot.push_back(pool_slot[c]);
+    const int n_tails = (int)tails[k].size();
+    if (n_tails > 65535) return "more than 65535 chain tails on one bus";
     sched[4 * p + 0] = (int32_t)((uint32_t)k | ((uint32_t)kp << 16));
     if (begin > REC_LIST_MASK) return "child lists too long";
-    sched[4 * p + 1] = (int32_t)((uint32_t)begin | ((uint32_t)kids_x_slot[k] << REC_KIDX_SHIFT));
+    sched[4 * p + 1] = (int32_t)((uint32_t)begin | ((uint32_t)(kids_x_slot[k] + 1) << REC_KIDX_SHIFT));
     sched[4 * p + 2] = (int32_t)((uint32_t)flags[k] | ((uint32_t)pool_slot[k] << FL_POOL_SHIFT) | ((uint32_t)x_slot[k] << FL_XSLOT_SHIFT));
-    sched[4 * p + 3] = (int32_t)((uint32_t)n_pool_kids | ((uint32_t)n_all << 16));
+    sched[4 * p + 3] = (int32_t)((uint32_t)n_tails | ((uint32_t)(absorb[k] >= 0 ? pool_slot[absorb[k]] + 1 : 0) << 16));
   }
   for (int k = 0; k < n; ++k) {
     topo[4 * k + 0] = k > 0 ? d->parent[k] : 0;
@@ -408,15 +458,15 @@ inline std::string build_feeder_image(const gfr_feeder_desc* d, int lanes, int s
   lay.o_kids = -1;
   lay.o_rowrec = -1; lay.sw_rows = 0;
   if (newton) {
-    lay.o_child_slot = ib.add_i(child_slot.data(), (int)child_slot.size());   // (child_ent: no kernel reads it any more)
+    lay.o_child_slot = ib.add_i(child_slot.data(), (int)child_slot.size());
     if (lanes >= GFR_WIDE_GROUP_MIN_LANES) {
-      // CTA-wide groups: the first 8 pool children's slots of every position, 16 bits each, in list order
+      // CTA-wide groups: the first 8 chain tails' slots of every position, 16 bits each, in list order
       std::vector<int32_t> kids(4 * (size_t)P, 0);
       for (int p = 0; p < P; ++p) {
         const uint32_t begin = (uint32_t)sched[4 * p + 1] & (uint32_t)REC_LIST_MASK;
-        const uint32_t npk = (uint32_t)sched[4 * p + 3] & 0xffffu, nall = (uint32_t)sched[4 * p + 3] >> 16;
-        for (uint32_t j = 0; j < npk && j < 8; ++j) {
-          const uint32_t slot = (uint32_t)child_slot[begin + nall - npk + j];
+        const uint32_t nt = (uint32_t)sched[4 * p + 3] & 0xffffu;
+        for (uint32_t j = 0; j < nt && j < 8; ++j) {
+          const uint32_t slot = (uint32_t)child_slot[begin + j];
           kids[4 * p + (j >> 1)] = (int32_t)((uint32_t)kids[4 * p + (j >> 1)] | (slot << (16 * (j & 1))));
         }
       }

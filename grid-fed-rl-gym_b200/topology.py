@@ -327,6 +327,9 @@ def _schedule(n: int, root: int, adj, width: Optional[int], alap: bool = True):
     return order, parent_ref, level_of
 
 
+CHAIN_MIN_LANES = 8        # groups of this many lanes and more sum pool hand-offs along sibling chains (gfr_device.cuh)
+
+
 def _schedule_paths(n: int, root: int, adj, width: int):
     """Order the buses for leaf -> root elimination on ``width`` lanes so that a lane FOLLOWS A PATH:
     list scheduling in elimination time where a lane whose last bus's parent has become ready takes
@@ -382,23 +385,38 @@ def _schedule_paths(n: int, root: int, adj, width: int):
         steps.append(assign)
     steps.reverse()                       # level 0 = last eliminated = root
     assert list(steps[0]) == [root]
-    # As-late-as-possible pass for the leaves that hand over through shared memory: a leaf eliminated long
-    # before its parent parks its contribution in a pool slot all that time; moved to a free lane of a row
-    # nearer the parent's, fewer slots are alive at once (IEEE-123 on 8 lanes: 17 -> fewer slots).
+    # Placement of the leaves that hand over through shared memory: a leaf eliminated long before its parent
+    # parks its contribution in a pool slot all that time, so it moves to a free lane of a row nearer the
+    # parent's.  From CHAIN_MIN_LANES lanes on, not into a row that already holds more of its siblings than
+    # another candidate row does: there siblings in different rows chain their hand-offs (each adds an earlier
+    # one's partial sum to its own, see csrc/gfr_image.hpp) and the parent reads one sum per chain; siblings in
+    # one row cannot chain.  Fewer lanes take the row nearest the parent's.
     row_of = {v: l for l, assign in enumerate(steps) for v in assign}
     has_kids = set(parent_ref[v][0] for v in bfs[1:])
+    kids_of = {}
+    for v in bfs[1:]:
+        kids_of.setdefault(parent_ref[v][0], []).append(v)
+
+    def is_heir(v):
+        u = parent_ref[v][0]
+        return row_of[v] == row_of[u] + 1 and steps[row_of[v]][v] == steps[row_of[u]].get(u)
+
     for v in sorted((v for v in bfs[1:] if v not in has_kids), key=lambda v: -(row_of[v] - row_of[parent_ref[v][0]])):
         u = parent_ref[v][0]
         cur = row_of[v]
-        if cur == row_of[u] + 1 and steps[cur][v] == steps[row_of[u]].get(u):
+        if is_heir(v):
             continue                      # the heir of its parent: nothing parked
-        for r in range(row_of[u] + 1, cur):
-            if len(steps[r]) < width:
-                lane = min(set(range(width)) - set(steps[r].values()))
-                del steps[cur][v]
-                steps[r][v] = lane
-                row_of[v] = r
-                break
+        rows = [r for r in range(row_of[u] + 1, cur + 1) if r == cur or len(steps[r]) < width]
+        if width >= CHAIN_MIN_LANES:
+            sibs = [row_of[w] for w in kids_of[u] if w != v and not is_heir(w)]
+            r = min(rows, key=lambda r: (sibs.count(r), r))
+        else:
+            r = rows[0]
+        if r != cur:
+            lane = min(set(range(width)) - set(steps[r].values()))
+            del steps[cur][v]
+            steps[r][v] = lane
+            row_of[v] = r
     order, level_of, lane_of = [], {}, {}
     for l, assign in enumerate(steps):
         for v in sorted(assign, key=lambda v: assign[v]):
