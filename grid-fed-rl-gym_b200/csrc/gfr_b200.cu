@@ -32,18 +32,8 @@ namespace {
 
 constexpr int kSmemHeader = 16;   // the mbarrier, keeps the image 16-byte aligned
 // threads per CTA the kernels are compiled for (sets their register budget: 65536 / threads).
-// 16-lane groups are the ones that want more than 512 threads (IEEE-123: 38 instances x 16 lanes).
-#ifndef GFR_MAX_THREADS_16
-#define GFR_MAX_THREADS_16 512
-#endif
-#ifndef GFR_MAX_THREADS
-#define GFR_MAX_THREADS 512
-#endif
-constexpr int kMaxThreads = GFR_MAX_THREADS;
-#ifndef GFR_WIDE_LANES
-#define GFR_WIDE_LANES 0      // groups up to this many lanes are compiled for 768 threads per CTA (80 registers): measured, no gain (IEEE-34 237M -> 230M)
-#endif
-constexpr int max_threads_for(int lanes) { return lanes == 16 ? GFR_MAX_THREADS_16 : (lanes <= GFR_WIDE_LANES ? 768 : kMaxThreads); }
+// Measured, no gain: 768 threads (80 registers) for small groups (IEEE-34 237 M -> 230 M env-steps/s).
+constexpr int kMaxThreads = 512;
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
   return (uint32_t)__cvta_generic_to_shared(p);
@@ -107,7 +97,7 @@ template <int LANES> __device__ __forceinline__ void use_local_injections(SGrp<L
 // IMG_SMEM: the feeder image is staged into shared memory (small / medium feeders); otherwise it is
 // read through L1 / L2 from global memory and all of shared memory goes to the working sets.
 template <int LANES, int SOLVER, bool IMG_SMEM>
-__global__ void __launch_bounds__(max_threads_for(LANES))
+__global__ void __launch_bounds__(kMaxThreads)
 step_kernel(const Layout lay, const EnvCfg cfg, const void* __restrict__ img, const int slot_bytes,
             D2* __restrict__ mscratch, double* __restrict__ state, void* __restrict__ obs,
             const void* obs_prev, const int obs_f32,
@@ -127,7 +117,7 @@ step_kernel(const Layout lay, const EnvCfg cfg, const void* __restrict__ img, co
 }
 
 template <int LANES, int SOLVER, bool IMG_SMEM>
-__global__ void __launch_bounds__(max_threads_for(LANES))
+__global__ void __launch_bounds__(kMaxThreads)
 solve_kernel(const Layout lay, const EnvCfg cfg, const void* __restrict__ img, const int slot_bytes,
              D2* __restrict__ mscratch, const double* __restrict__ p_inj, const SolOut o, const long long B) {
   extern __shared__ __align__(16) unsigned char smem[];
@@ -431,7 +421,7 @@ PlanTry plan_mode(const gfr_feeder* f, const Layout& lay, const void* fn, int la
       if (share < fixed + per_env + 1024) break;
       long long E = (long long)((share - 1024 - fixed) / per_env);
       if (lanes > 32) E = 1;                              // one CTA per instance
-      if (E * lanes > max_threads_for(lanes)) E = max_threads_for(lanes) / lanes;
+      if (E * lanes > kMaxThreads) E = kMaxThreads / lanes;
       if (pass == 0) E -= E % gran;                        // (a partial last warp was measured: no gain)
       if (E < 1) continue;
       const int threads = (int)(E * lanes);

@@ -133,7 +133,7 @@ struct SolveStat {
 // Loads are plain (weak) loads without L1 allocation: __ldcg would be a STRONG.GPU load here, ordered against
 // every earlier store of the thread (measured: 3 x slower kernel).
 GFR_HD uint64_t scratch_policy() {
-#if defined(__CUDA_ARCH__) && !defined(GFR_NO_L2_POLICY)
+#if defined(__CUDA_ARCH__)
   uint64_t pol;
   asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
   return pol;
@@ -142,13 +142,9 @@ GFR_HD uint64_t scratch_policy() {
 #endif
 }
 GFR_HD D2 ld_scratch(const D2* p, uint64_t pol) {
-#if defined(__CUDA_ARCH__) && !defined(GFR_NO_L2_POLICY)
+#if defined(__CUDA_ARCH__)
   D2 r;
   asm volatile("ld.global.L1::no_allocate.L2::cache_hint.v2.f64 {%0, %1}, [%2], %3;" : "=d"(r.x), "=d"(r.y) : "l"(p), "l"(pol) : "memory");
-  return r;
-#elif defined(__CUDA_ARCH__)
-  D2 r;
-  asm volatile("ld.global.L1::no_allocate.v2.f64 {%0, %1}, [%2];" : "=d"(r.x), "=d"(r.y) : "l"(p) : "memory");
   return r;
 #else
   (void)pol;
@@ -156,7 +152,7 @@ GFR_HD D2 ld_scratch(const D2* p, uint64_t pol) {
 #endif
 }
 GFR_HD void st_scratch(D2* p, const D2 v, uint64_t pol) {
-#if defined(__CUDA_ARCH__) && !defined(GFR_NO_L2_POLICY)
+#if defined(__CUDA_ARCH__)
   asm volatile("st.global.L2::cache_hint.v2.f64 [%0], {%1, %2}, %3;" ::"l"(p), "d"(v.x), "d"(v.y), "l"(pol) : "memory");
 #else
   (void)pol;
@@ -164,7 +160,7 @@ GFR_HD void st_scratch(D2* p, const D2 v, uint64_t pol) {
 #endif
 }
 GFR_HD double ld_scratch1(const double* p, uint64_t pol) {
-#if defined(__CUDA_ARCH__) && !defined(GFR_NO_L2_POLICY)
+#if defined(__CUDA_ARCH__)
   double r;
   asm volatile("ld.global.L1::no_allocate.L2::cache_hint.f64 %0, [%1], %2;" : "=d"(r) : "l"(p), "l"(pol) : "memory");
   return r;
@@ -174,7 +170,7 @@ GFR_HD double ld_scratch1(const double* p, uint64_t pol) {
 #endif
 }
 GFR_HD void st_scratch1(double* p, double v, uint64_t pol) {
-#if defined(__CUDA_ARCH__) && !defined(GFR_NO_L2_POLICY)
+#if defined(__CUDA_ARCH__)
   asm volatile("st.global.L2::cache_hint.f64 [%0], %1, %2;" ::"l"(p), "d"(v), "l"(pol) : "memory");
 #else
   (void)pol;
@@ -532,33 +528,17 @@ GFR_HD double noise_slot(uint64_t seed, uint64_t draw, int s) {
 
 // ----------------------------------------------------------------------------- solvers
 
-// Row passes of CTA-wide groups fetch what the NEXT row needs (its record, its branch / diagonal admittances) while
-// the present row computes: their feeder image is in global memory, an L2 round trip per row otherwise
-// (synthetic-1000: +8 %).  Measured and left off: the same for warp-sized groups, whose image is in shared memory
-// (GFR_PIPE_SMEM: IEEE-123 99.0 M -> 94.3 M, IEEE-34 306 M -> 284 M env-steps/s - the registers and moves cost more
-// than the shared-memory latency they hide), and fetching the branch's two voltages ahead as well (GFR_PIPE_EF:
-// synthetic-1000 5.91 M -> 5.64 M).
-#ifndef GFR_PIPE_SMEM
-#define GFR_PIPE_SMEM 0
-#endif
-// After a solve the Newton scratch of the slot is dead, but L2 cannot know: its dirty lines were written back to HBM
-// whenever the observation stream pushed them out (IEEE-123, 131 072 instances: 1.02 GB written per launch for 0.59 GB
-// of observation + state + outputs; the evict-last hint alone changed nothing).  2 = drop the D^-1 U / D^-1 r lines
-// with discard.global.L2 when the solve ends (581 MB written, 98.1 M env-steps/s), 1 = the injections' lines too
-// (565 MB, 97.8 M), 0 = keep them (1.02 GB, 99.2 M).
-#ifndef GFR_SCRATCH_DISCARD
-#define GFR_SCRATCH_DISCARD 2
-#endif
-#ifndef GFR_PIPE_EF
-#define GFR_PIPE_EF 0
-#endif
-// Groups this wide read the feeder image from global memory (one CTA per instance): they take the variants that
-// fetch index chains several positions at a time and the packed pool-child records.
+// Groups this wide read the feeder image from global memory (one CTA per instance).  Their row passes fetch what the
+// NEXT row needs (its record, its branch / diagonal admittances, its packed pool-child record) while the present row
+// computes - an L2 round trip per row otherwise (synthetic-1000: +8 %) - and they fetch index chains several
+// positions at a time.  Measured and left off: the same row pipeline for warp-sized groups, whose image is in shared
+// memory (IEEE-123 99.0 M -> 94.3 M, IEEE-34 306 M -> 284 M env-steps/s - the registers and moves cost more than the
+// shared-memory latency they hide), and fetching the branch's two voltages one row ahead as well (synthetic-1000
+// 5.91 M -> 5.64 M).
 #ifndef GFR_WIDE_GROUP_MIN_LANES
-#define GFR_WIDE_GROUP_MIN_LANES 64      // (the host emulation builds with 8 to walk this path on its 8- and 16-lane teams)
+#define GFR_WIDE_GROUP_MIN_LANES 64      // (the host emulation builds with 8 to walk these paths on its 8- and 16-lane teams)
 #endif
 template <int LANES> GFR_HD constexpr bool wide_group() { return LANES >= GFR_WIDE_GROUP_MIN_LANES; }
-template <int LANES> GFR_HD constexpr bool pipe_rows() { return LANES > 32 || GFR_PIPE_SMEM; }
 
 // Flat start (power_flow.py:103, :131): 1.0 at 0 rad, slack / PV buses at their set magnitude.
 template <class G, int LANES>
@@ -655,32 +635,27 @@ GFR_HD unsigned shr16_pair(unsigned lo, unsigned hi) { return (lo >> 16) | (hi <
   } while (0)
 
 // What a leaf -> root row pass (mismatch, elimination) needs of a row besides the children's hand-offs: its record,
-// branch / diagonal admittances and the voltages at both ends of its branch (fixed during the pass).  With the
-// pipe on they are fetched one row ahead into registers.
+// branch / diagonal admittances and the voltages at both ends of its branch (fixed during the pass).  CTA-wide
+// groups fetch the record, the admittances and the packed pool-child record one row ahead into registers.
 #define GFR_ROW_PIPE_DECL                                                                                          \
-  I4 t_next, kq_next; D2 y_next, yd_next, vk_next, vp_next;                                                        \
+  I4 t_next, kq_next; D2 y_next, yd_next;                                                                          \
   t_next.x = t_next.y = t_next.z = t_next.w = 0;                                                                   \
   kq_next = t_next;                                                                                                \
-  y_next.x = y_next.y = yd_next.x = yd_next.y = vk_next.x = vk_next.y = vp_next.x = vp_next.y = 0.0
+  y_next.x = y_next.y = yd_next.x = yd_next.y = 0.0
 #define GFR_ROW_PIPE_LOAD(pos_)                                                                                    \
-  do {                                                                                                             \
-    t_next = sched[(pos_)]; y_next = gb[(pos_)]; yd_next = gbd[(pos_)];                                            \
-    if (wide_group<LANES>()) kq_next = kids[(pos_)];                                                              \
-    if (GFR_PIPE_EF) { vk_next = g.ef(rec_bus(t_next)); vp_next = g.ef(rec_parent(t_next)); }                      \
-  } while (0)
+  do { t_next = sched[(pos_)]; y_next = gb[(pos_)]; yd_next = gbd[(pos_)]; kq_next = kids[(pos_)]; } while (0)
 #define GFR_ROW_PIPE_FIRST(pos_)                                                                                   \
-  do { if (pipe_rows<LANES>()) GFR_ROW_PIPE_LOAD(pos_); } while (0)
+  do { if (wide_group<LANES>()) GFR_ROW_PIPE_LOAD(pos_); } while (0)
 // defines t, yb, yd, vk, vp of position p_ (idle positions: record 0 -> bus 0, harmless) and starts the next row's fetch
 #define GFR_ROW_PIPE_TAKE(p_, more_, next_)                                                                        \
   I4 t, kq; D2 yb, yd, vk, vp;                                                                                     \
   kq.x = kq.y = kq.z = kq.w = 0;                                                                                   \
-  if (pipe_rows<LANES>()) {                                                                                        \
+  if (wide_group<LANES>()) {                                                                                       \
     t = t_next; yb = y_next; yd = yd_next; kq = kq_next;                                                           \
-    if (GFR_PIPE_EF) { vk = vk_next; vp = vp_next; } else { vk = g.ef(rec_bus(t)); vp = g.ef(rec_parent(t)); }     \
+    vk = g.ef(rec_bus(t)); vp = g.ef(rec_parent(t));                                                               \
     if (more_) GFR_ROW_PIPE_LOAD(next_);                                                                           \
   } else {                                                                                                         \
     t = sched[(p_)]; yb = gb[(p_)]; yd = gbd[(p_)]; vk = g.ef(rec_bus(t)); vp = g.ef(rec_parent(t));               \
-    if (wide_group<LANES>()) kq = kids[(p_)];                                                                     \
   }
 
 // max |mismatch| of the present voltages (power_flow.py:150-166), as a leaf -> root row pass on the elimination
@@ -761,15 +736,14 @@ GFR_HD void newton_back_update(const NGrp<LANES>& g, const Layout& lay, const in
   do {                                                                     \
     const int p = (row_) * LANES + g.lane;                                 \
     I4 t;                                                                  \
-    D2 e_now;                                                              \
-    if (pipe_rows<LANES>()) {                                              \
-      t = t_next; e_now = e_next;                                          \
-      if ((row_) + 1 < nrows) { t_next = sched[p + LANES]; if (GFR_PIPE_EF) e_next = g.efp[rec_bus(t_next)]; } \
-      if (!GFR_PIPE_EF) e_now = g.efp[rec_bus(t)];                         \
-    } else { t = sched[p]; e_now = g.efp[rec_bus(t)]; }                    \
+    if (wide_group<LANES>()) {                                             \
+      t = t_next;                                                          \
+      if ((row_) + 1 < nrows) t_next = sched[p + LANES];                   \
+    } else t = sched[p];                                                   \
+    const D2 e_now = g.efp[rec_bus(t)];                                    \
     D2 m0 = m0_, m1 = m1_, v = v_;                                         \
     if (f0) {                                                              \
-      if (LANES > 32) {                                                    \
+      if (wide_group<LANES>()) {                                           \
         m0 = f0m0_next; m1 = f0m1_next;                                    \
         if ((row_) + 1 < nrows) { f0m0_next = f0[2 * P + p + LANES]; f0m1_next = f0[3 * P + p + LANES]; } \
       } else { m0 = f0[2 * P + p]; m1 = f0[3 * P + p]; }                   \
@@ -800,9 +774,8 @@ GFR_HD void newton_back_update(const NGrp<LANES>& g, const Layout& lay, const in
   t_next.x = t_next.y = t_next.z = t_next.w = 0;
   D2 f0m0_next, f0m1_next;                             // ... and the flat-start D^-1 U rows in the first iteration
   f0m0_next.x = f0m0_next.y = f0m1_next.x = f0m1_next.y = 0.0;
-  D2 e_next; e_next.x = e_next.y = 0.0;                // ... and the voltage of its bus (only its own lane ever rewrites it)
-  if (pipe_rows<LANES>()) { t_next = sched[g.lane]; if (GFR_PIPE_EF) e_next = g.efp[rec_bus(t_next)]; }
-  if (LANES > 32 && f0) { f0m0_next = f0[2 * P + g.lane]; f0m1_next = f0[3 * P + g.lane]; }
+  if (wide_group<LANES>()) t_next = sched[g.lane];
+  if (wide_group<LANES>() && f0) { f0m0_next = f0[2 * P + g.lane]; f0m1_next = f0[3 * P + g.lane]; }
   for (int row = 0; row < nrows; row += 2) {
     GFR_BU_ROW(row, a0, a1, av);
     if (row + 1 < nrows) GFR_BU_ROW(row + 1, b0, b1, bv);
@@ -858,25 +831,24 @@ GFR_HD void newton_solve(const NGrp<LANES>& g, const Layout& lay, const int* sim
       t_next.x = t_next.y = t_next.z = t_next.w = 0;
       kq_next = t_next;
       pc_next.x = pc_next.y = i0_next.x = i0_next.y = i1_next.x = i1_next.y = lp_next.x = lp_next.y = 0.0;
-      if (pipe_rows<LANES>()) {
+      if (wide_group<LANES>()) {
         const int p0 = (nrows - 1) * LANES + g.lane;
         t_next = sched[p0]; pc_next = f0[5 * P + p0]; i0_next = f0[p0]; i1_next = f0[P + p0]; lp_next = f0[4 * P + p0];
-        if (wide_group<LANES>()) kq_next = kids[p0];
+        kq_next = kids[p0];
       }
       for (int row = nrows - 1; row >= 0; --row) {
         const int p = row * LANES + g.lane;
         I4 t, kq; D2 pc, i0, i1, lp;                    // record, flat-profile (P, Q), D^-1 rows, (ll, gl)
         kq.x = kq.y = kq.z = kq.w = 0;
-        if (pipe_rows<LANES>()) {
+        if (wide_group<LANES>()) {
           t = t_next; pc = pc_next; i0 = i0_next; i1 = i1_next; lp = lp_next; kq = kq_next;
           if (row > 0) {
-            if (wide_group<LANES>()) kq_next = kids[p - LANES];
+            kq_next = kids[p - LANES];
             t_next = sched[p - LANES]; pc_next = f0[5 * P + p - LANES];
             i0_next = f0[p - LANES]; i1_next = f0[P + p - LANES]; lp_next = f0[4 * P + p - LANES];
           }
         } else {
           t = sched[p]; pc = f0[5 * P + p]; i0 = f0[p]; i1 = f0[P + p]; lp = f0[4 * P + p];
-          if (wide_group<LANES>()) kq = kids[p];
         }
         const double ps = ps_next;
         if (row > 0) ps_next = g.pspec(p - LANES);
@@ -1023,17 +995,16 @@ GFR_HD void newton_solve(const NGrp<LANES>& g, const Layout& lay, const int* sim
       mm_prev = mm;
     }
   }
-#if defined(__CUDA_ARCH__) && GFR_SCRATCH_DISCARD
+#if defined(__CUDA_ARCH__)
   // The scratch of this solve is dead (the next instance of the slot rewrites it before reading): tell L2, so that
   // the dirty lines need not be written back to HBM when the observation stream pushes them out.  Every exit of the
-  // loop above comes after a group-wide reduction, and every scratch read before that.
+  // loop above comes after a group-wide reduction, and every scratch read before that.  Measured on IEEE-123, 131 072
+  // instances (0.59 GB of observation + state + outputs per launch; the evict-last hint alone changed nothing):
+  // discarding the D^-1 U / D^-1 r lines writes 581 MB per launch at 98.1 M env-steps/s, discarding the injections'
+  // lines too 565 MB at 97.8 M, keeping everything 1.02 GB at 99.2 M.
   {
     char* const base = reinterpret_cast<char*>(g.mg);
-#if GFR_SCRATCH_DISCARD == 2
     const size_t bytes = ((size_t)P * 48) & ~(size_t)127;         // D^-1 U, D^-1 r only (whole lines), not the injections
-#else
-    const size_t bytes = newton_scratch_doubles(P) * 8;
-#endif
     for (size_t off = (size_t)g.lane * 128; off < bytes; off += (size_t)LANES * 128)
       asm volatile("discard.global.L2 [%0], 128;" ::"l"(base + off) : "memory");
   }

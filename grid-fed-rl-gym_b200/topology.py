@@ -24,7 +24,6 @@ from __future__ import annotations
 from dataclasses import dataclass, field
 from typing import Any, Dict, List, Optional, Sequence, Tuple
 
-import os
 import numpy as np
 
 # zero-length IEEE-13 entries keep their configured impedance, un-scaled, as pu
@@ -249,15 +248,10 @@ def _series_admittance(r: float, x: float) -> complex:
     return 1.0 / z if abs(z) > OPEN_Z else 0.0
 
 
-def _schedule(n: int, root: int, adj, width: Optional[int], alap: bool = True):
-    """Order the buses for leaf -> root elimination on ``width`` lanes.
-
-    Returns (order, parent_ref, level_of): ``order`` lists ref bus indices level by level,
-    level 0 = {root}; every bus sits in a later level than its parent, and each level holds at
-    most ``width`` buses when a width is given.  Levels are the time steps (reversed) of Hu's
-    highest-level-first list schedule, which is optimal for unit tasks on an in-tree: with
-    unbounded width it is the plain height-from-the-leaves layering.
-    """
+def _rooted_tree(n: int, root: int, adj):
+    """Breadth-first walk of the tree from ``root``.  Returns (bfs, parent_ref, depth, pending):
+    ``bfs`` lists ref bus indices root first, ``parent_ref[v]`` = (parent, line index) ((-1, -1) for the
+    root), ``pending[v]`` = number of children of v (what must be eliminated before v)."""
     parent_ref = {root: (-1, -1)}
     depth = {root: 0}
     bfs = [root]
@@ -272,6 +266,19 @@ def _schedule(n: int, root: int, adj, width: Optional[int], alap: bool = True):
     pending = [0] * n
     for v in bfs[1:]:
         pending[parent_ref[v][0]] += 1
+    return bfs, parent_ref, depth, pending
+
+
+def _schedule(n: int, root: int, adj, width: Optional[int]):
+    """Order the buses for leaf -> root elimination on ``width`` lanes.
+
+    Returns (order, parent_ref, level_of): ``order`` lists ref bus indices level by level,
+    level 0 = {root}; every bus sits in a later level than its parent, and each level holds at
+    most ``width`` buses when a width is given.  Levels are the time steps (reversed) of Hu's
+    highest-level-first list schedule, which is optimal for unit tasks on an in-tree: with
+    unbounded width it is the plain height-from-the-leaves layering.
+    """
+    bfs, parent_ref, depth, pending = _rooted_tree(n, root, adj)
     ready = [v for v in bfs if pending[v] == 0]
     steps = []
     while ready:
@@ -295,12 +302,8 @@ def _schedule(n: int, root: int, adj, width: Optional[int], alap: bool = True):
     for l, members in enumerate(steps):
         for v in members:
             level[v] = l
-    if not alap:
-        bfs_moves = []
-    else:
-        bfs_moves = bfs[1:]
     room = [None if width is None else width - len(members) for members in steps]
-    for v in bfs_moves:                  # breadth-first from the root: parents first
+    for v in bfs[1:]:                    # breadth-first from the root: parents first
         target = level[parent_ref[v][0]] + 1
         cur = level[v]
         while target < cur:
@@ -341,20 +344,7 @@ def _schedule_paths(n: int, root: int, adj, width: int):
 
     Returns (order, parent_ref, level_of, lane_of): ``order`` lists ref bus indices level by level,
     level 0 = {root}; a level is one elimination step (reversed), at most ``width`` buses."""
-    parent_ref = {root: (-1, -1)}
-    depth = {root: 0}
-    bfs = [root]
-    for u in bfs:
-        for v, k in adj[u]:
-            if v not in parent_ref:
-                parent_ref[v] = (u, k)
-                depth[v] = depth[u] + 1
-                bfs.append(v)
-    if len(bfs) != n:
-        raise TopologyError("feeder is not connected (run repair_topology first)")
-    pending = [0] * n
-    for v in bfs[1:]:
-        pending[parent_ref[v][0]] += 1
+    bfs, parent_ref, depth, pending = _rooted_tree(n, root, adj)
     ready = set(v for v in bfs if pending[v] == 0)
     last = [None] * width                 # the bus each lane eliminated in the previous step
     steps = []                            # per step: {bus: lane}
@@ -525,50 +515,41 @@ def compile_feeder(feeder, renewable_sources: Optional[Sequence[str]] = None,
     if width is not None and int(width) < 1:
         raise TopologyError("width must be >= 1")
     root_ref = slack if root == "slack" else tree_center(n, adj, slack)
-    def layout(alap: bool):
-        lane_map = None
-        if paths and width is not None:
-            order, parent_ref, level_of, lane_map = _schedule_paths(n, root_ref, adj, int(width))
-        else:
-            order, parent_ref, level_of = _schedule(n, root_ref, adj, None if width is None else int(width), alap)
-        rank = np.empty(n, dtype=np.int32)
-        rank[np.array(order)] = np.arange(n, dtype=np.int32)
+    lane_map = None
+    if paths and width is not None:
+        order, parent_ref, level_of, lane_map = _schedule_paths(n, root_ref, adj, int(width))
+    else:
+        order, parent_ref, level_of = _schedule(n, root_ref, adj, None if width is None else int(width))
+    rank = np.empty(n, dtype=np.int32)
+    rank[np.array(order)] = np.arange(n, dtype=np.int32)
 
-        parent = np.full(n, -1, dtype=np.int32)
-        line_of = np.full(n, -1, dtype=np.int32)
-        from_is_parent = np.zeros(n, dtype=np.int32)
-        g = np.zeros(n); b = np.zeros(n); r = np.zeros(n); x = np.zeros(n); rating = np.zeros(n)
-        for k in range(1, n):
-            u, li = parent_ref[order[k]]
-            parent[k] = rank[u]
-            line_of[k] = li
-            ln = lines[li]
-            from_is_parent[k] = 1 if index[ln.from_bus] == u else 0
-            g[k], b[k] = ys[li].real, ys[li].imag
-            r[k], x[k] = ln.resistance, ln.reactance
-            rating[k] = ln.rating
-        levels = np.array([level_of[v] for v in order])
-        n_levels = int(levels.max()) + 1
-        level_ptr = np.searchsorted(levels, np.arange(n_levels + 1)).astype(np.int32)
-        child_cnt = np.bincount(parent[1:], minlength=n) if n > 1 else np.zeros(n, dtype=np.int64)
-        child_ptr = np.zeros(n + 1, dtype=np.int32)
-        child_ptr[1:] = np.cumsum(child_cnt)
-        child_idx = np.zeros(max(n - 1, 0), dtype=np.int32)
-        fill = child_ptr[:-1].copy()
-        for k in range(1, n):
-            child_idx[fill[parent[k]]] = k
-            fill[parent[k]] += 1
-        for k in range(1, n):
-            assert parent[k] < k and levels[parent[k]] < levels[k]
-        lane_arr = None if lane_map is None else np.array([lane_map[v] for v in order], dtype=np.int32)
-        return dict(lane_of=lane_arr, order=order, rank=rank, parent=parent, line_of=line_of, from_is_parent=from_is_parent,
-                    g=g, b=b, r=r, x=x, rating=rating, levels=levels, n_levels=n_levels, level_ptr=level_ptr,
-                    child_ptr=child_ptr, child_idx=child_idx)
-
-    lay = layout(True)
-    order, rank, parent, line_of, from_is_parent = (lay[k] for k in ("order", "rank", "parent", "line_of", "from_is_parent"))
-    g, b, r, x, rating = (lay[k] for k in ("g", "b", "r", "x", "rating"))
-    level_ptr, child_ptr, child_idx = (lay[k] for k in ("level_ptr", "child_ptr", "child_idx"))
+    parent = np.full(n, -1, dtype=np.int32)
+    line_of = np.full(n, -1, dtype=np.int32)
+    from_is_parent = np.zeros(n, dtype=np.int32)
+    g = np.zeros(n); b = np.zeros(n); r = np.zeros(n); x = np.zeros(n); rating = np.zeros(n)
+    for k in range(1, n):
+        u, li = parent_ref[order[k]]
+        parent[k] = rank[u]
+        line_of[k] = li
+        ln = lines[li]
+        from_is_parent[k] = 1 if index[ln.from_bus] == u else 0
+        g[k], b[k] = ys[li].real, ys[li].imag
+        r[k], x[k] = ln.resistance, ln.reactance
+        rating[k] = ln.rating
+    levels = np.array([level_of[v] for v in order])
+    n_levels = int(levels.max()) + 1
+    level_ptr = np.searchsorted(levels, np.arange(n_levels + 1)).astype(np.int32)
+    child_cnt = np.bincount(parent[1:], minlength=n) if n > 1 else np.zeros(n, dtype=np.int64)
+    child_ptr = np.zeros(n + 1, dtype=np.int32)
+    child_ptr[1:] = np.cumsum(child_cnt)
+    child_idx = np.zeros(max(n - 1, 0), dtype=np.int32)
+    fill = child_ptr[:-1].copy()
+    for k in range(1, n):
+        child_idx[fill[parent[k]]] = k
+        fill[parent[k]] += 1
+    for k in range(1, n):
+        assert parent[k] < k and levels[parent[k]] < levels[k]
+    lane_of = None if lane_map is None else np.array([lane_map[v] for v in order], dtype=np.int32)
 
     # ---- ties: end points in level order and the inverse of the loop-impedance matrix
     #      Z_loop[i][j] = sum over tree branches e of z_e s_i(e) s_j(e) + [i == j] z_tie_i, where
@@ -604,7 +585,7 @@ def compile_feeder(feeder, renewable_sources: Optional[Sequence[str]] = None,
         s_base=float(feeder.parameters.base_power) * 1e6,
         bus_ids=[b_.id for b_ in buses], line_ids=[l_.id for l_ in lines],
         order=np.array(order, dtype=np.int32), rank=rank, parent=parent, level_ptr=level_ptr,
-        child_ptr=child_ptr, child_idx=child_idx, n_pool=0, lane_of=lay["lane_of"],
+        child_ptr=child_ptr, child_idx=child_idx, n_pool=0, lane_of=lane_of,
         bus_type=bus_type, vm_set=vm_set, g=g, b=b,
         gdiag=ydiag.real[order].copy(), bdiag=ydiag.imag[order].copy(), r=r, x=x,
         line_of=line_of, from_is_parent=from_is_parent, rating=rating, **tie_soa)

@@ -28,8 +28,8 @@ def _compile(out: str, extra) -> str:
            # the header-only builder is also compiled into libgfr_b200.so, which loads with RTLD_GLOBAL: without these
            # the emulation would bind to THAT copy of the inline functions (stale whenever the two are built apart)
            "-fvisibility-inlines-hidden", "-Wl,-Bsymbolic",
-           # packed pool-child records (the kernels use them for CTA-wide groups) on the 8- and 16-lane teams, the
-           # child lists on the 2- and 4-lane ones
+           # the CTA-wide groups' paths (row pipeline, packed pool-child records) on the 8- and 16-lane teams, the
+           # warp-sized groups' ones on the 2- and 4-lane teams
            "-DGFR_WIDE_GROUP_MIN_LANES=8", *[f"-D{d}" for d in extra], "-o", out,
            os.path.join(HERE, "gfr_emu.cpp"), "-lm"]
     res = subprocess.run(cmd, capture_output=True, text=True)
