@@ -180,8 +180,11 @@ GFR_HD void st_scratch1(double* p, double v, uint64_t pol) {
 
 // ----------------------------------------------------------------------------- group ops
 
-struct OpMaxNan { GFR_HD double operator()(double v, double w) const { return (w > v || w != w) ? w : v; } };
-struct OpMinNan { GFR_HD double operator()(double v, double w) const { return (w < v || w != w) ? w : v; } };
+// numpy's maximum / minimum: a NaN in either argument is the result
+GFR_HD double max_nan(double v, double w) { return (w > v || w != w) ? w : v; }
+GFR_HD double min_nan(double v, double w) { return (w < v || w != w) ? w : v; }
+struct OpMaxNan { GFR_HD double operator()(double v, double w) const { return max_nan(v, w); } };
+struct OpMinNan { GFR_HD double operator()(double v, double w) const { return min_nan(v, w); } };
 struct OpMax { GFR_HD double operator()(double v, double w) const { return fmax(v, w); } };
 struct OpMin { GFR_HD double operator()(double v, double w) const { return fmin(v, w); } };
 struct OpSum { GFR_HD double operator()(double v, double w) const { return v + w; } };
@@ -541,9 +544,8 @@ GFR_HD double noise_slot(uint64_t seed, uint64_t draw, int s) {
 template <int LANES> GFR_HD constexpr bool wide_group() { return LANES >= GFR_WIDE_GROUP_MIN_LANES; }
 
 // Flat start (power_flow.py:103, :131): 1.0 at 0 rad, slack / PV buses at their set magnitude.
-template <class G, int LANES>
-GFR_HD void flat_start_t(const G& g, const Lanes<LANES>&, const Layout& lay, const int* simg,
-                         const double* dimg) {
+template <template <int> class G, int LANES>
+GFR_HD void flat_start(const G<LANES>& g, const Layout& lay, const int* simg, const double* dimg) {
   const I4* sched = reinterpret_cast<const I4*>(simg + lay.o_sched);
   if (wide_group<LANES>()) {
     // image in global memory: four positions' records (and set points) per L2 round trip
@@ -565,6 +567,8 @@ GFR_HD void flat_start_t(const G& g, const Lanes<LANES>&, const Layout& lay, con
       }
     }
   } else
+  // warp-sized groups read a set point only where a position has one (the wide loop's form with one position per
+  // round, which reads every set point, is unrolled differently by the compiler: 3 - 10 % more or fewer instructions)
   for (int p = g.lane; p < lay.P; p += LANES) {
     const I4 t = sched[p];
     if (!(t.z & FL_VALID)) continue;
@@ -574,10 +578,6 @@ GFR_HD void flat_start_t(const G& g, const Lanes<LANES>&, const Layout& lay, con
     g.ef(rec_bus(t)) = v;
   }
   g.sync();
-}
-template <class G>
-GFR_HD void flat_start(const G& g, const Layout& lay, const int* simg, const double* dimg) {
-  flat_start_t(g, g, lay, simg, dimg);
 }
 
 // Polar Newton-Raphson on a radial feeder.  Same iterates as the reference's dense solve:
@@ -596,9 +596,6 @@ GFR_HD void flat_start(const G& g, const Layout& lay, const int* simg, const dou
 // Elimination of bus k (all its children done): D_k = J[k,k] - sum_c C_c, r_k = mismatch_k - sum_c cc_c,
 //   M_k = D_k^-1 J[k,p], v_k = D_k^-1 r_k, and its contribution to the parent p:
 //   C_k = J[p,k] M_k, cc_k = J[p,k] v_k.   Back-substitution: x_k = v_k - M_k x_p.
-#ifdef GFR_EMU_STATS
-static long long gfr_emu_stats[4];   // host debugging: mismatch-only passes, elimination passes, of those converged
-#endif
 struct BranchT { double ga, al, gl, ll; };
 // vk: the bus below the branch, vp: its parent, y: series g + jb
 GFR_HD BranchT branch_terms(const D2 vk, const D2 vp, const D2 y) {
@@ -609,54 +606,58 @@ GFR_HD BranchT branch_terms(const D2 vk, const D2 vp, const D2 y) {
   return t;
 }
 
-// The pool slots of a position's chain tails, one after the other in `slot` for the body given last.  CTA-wide groups
-// read their image from global memory: there the first 8 slots come packed in a record (kq_) that travels one row
-// ahead with the position's own record, which takes the list's L2 round trip off every row's critical path.
+// Calls f(slot) with the pool slot of each of a position's chain tails in turn.  CTA-wide groups read their image
+// from global memory: there the first 8 slots come packed in a record (kq) that travels one row ahead with the
+// position's own record, which takes the list's L2 round trip off every row's critical path.
 GFR_HD unsigned shr16_pair(unsigned lo, unsigned hi) { return (lo >> 16) | (hi << 16); }
-#define GFR_POOL_GATHER(t_, kq_, ...)                                                                              \
-  do {                                                                                                             \
-    const int npk_ = rec_tails(t_);                                                                                \
-    if (wide_group<LANES>() && npk_ <= 8) {                                                                       \
-      unsigned w0_ = (unsigned)(kq_).x, w1_ = (unsigned)(kq_).y, w2_ = (unsigned)(kq_).z, w3_ = (unsigned)(kq_).w; \
-      _Pragma("unroll 1")                                                                                          \
-      for (int j_ = 0; j_ < npk_; ++j_) {                                                                          \
-        const int slot = (int)(w0_ & 0xffffu);                                                                     \
-        w0_ = shr16_pair(w0_, w1_); w1_ = shr16_pair(w1_, w2_); w2_ = shr16_pair(w2_, w3_); w3_ >>= 16;            \
-        __VA_ARGS__                                                                                                \
-      }                                                                                                            \
-    } else {                                                                                                       \
-      const int q0_ = rec_list(t_);                                                                                \
-      _Pragma("unroll 1")                                                                                          \
-      for (int q_ = q0_; q_ < q0_ + npk_; ++q_) {                                                                  \
-        const int slot = child_slot[q_];                                                                           \
-        __VA_ARGS__                                                                                                \
-      }                                                                                                            \
-    }                                                                                                              \
-  } while (0)
-
-// What a leaf -> root row pass (mismatch, elimination) needs of a row besides the children's hand-offs: its record,
-// branch / diagonal admittances and the voltages at both ends of its branch (fixed during the pass).  CTA-wide
-// groups fetch the record, the admittances and the packed pool-child record one row ahead into registers.
-#define GFR_ROW_PIPE_DECL                                                                                          \
-  I4 t_next, kq_next; D2 y_next, yd_next;                                                                          \
-  t_next.x = t_next.y = t_next.z = t_next.w = 0;                                                                   \
-  kq_next = t_next;                                                                                                \
-  y_next.x = y_next.y = yd_next.x = yd_next.y = 0.0
-#define GFR_ROW_PIPE_LOAD(pos_)                                                                                    \
-  do { t_next = sched[(pos_)]; y_next = gb[(pos_)]; yd_next = gbd[(pos_)]; kq_next = kids[(pos_)]; } while (0)
-#define GFR_ROW_PIPE_FIRST(pos_)                                                                                   \
-  do { if (wide_group<LANES>()) GFR_ROW_PIPE_LOAD(pos_); } while (0)
-// defines t, yb, yd, vk, vp of position p_ (idle positions: record 0 -> bus 0, harmless) and starts the next row's fetch
-#define GFR_ROW_PIPE_TAKE(p_, more_, next_)                                                                        \
-  I4 t, kq; D2 yb, yd, vk, vp;                                                                                     \
-  kq.x = kq.y = kq.z = kq.w = 0;                                                                                   \
-  if (wide_group<LANES>()) {                                                                                       \
-    t = t_next; yb = y_next; yd = yd_next; kq = kq_next;                                                           \
-    vk = g.ef(rec_bus(t)); vp = g.ef(rec_parent(t));                                                               \
-    if (more_) GFR_ROW_PIPE_LOAD(next_);                                                                           \
-  } else {                                                                                                         \
-    t = sched[(p_)]; yb = gb[(p_)]; yd = gbd[(p_)]; vk = g.ef(rec_bus(t)); vp = g.ef(rec_parent(t));               \
+template <int LANES, class F>
+GFR_HD void for_each_tail(const I4& t, const I4& kq, const int* child_slot, F&& f) {
+  const int npk = rec_tails(t);
+  if (wide_group<LANES>() && npk <= 8) {
+    unsigned w0 = (unsigned)kq.x, w1 = (unsigned)kq.y, w2 = (unsigned)kq.z, w3 = (unsigned)kq.w;
+#pragma unroll 1
+    for (int j = 0; j < npk; ++j) {
+      const int slot = (int)(w0 & 0xffffu);
+      w0 = shr16_pair(w0, w1); w1 = shr16_pair(w1, w2); w2 = shr16_pair(w2, w3); w3 >>= 16;
+      f(slot);
+    }
+  } else {
+    const int q0 = rec_list(t);
+#pragma unroll 1
+    for (int q = q0; q < q0 + npk; ++q) f(child_slot[q]);
   }
+}
+
+// What a row pass reads of each of its positions (`load(p)`: record, admittances, factors ...).  CTA-wide groups take
+// it from registers filled while the previous row computed; warp-sized groups, whose image is in shared memory,
+// load it when they need it.
+template <int LANES, class T>
+struct Ahead {
+  T next = T();
+  template <class Load> GFR_HD void first(const Load& load, int p) {
+    if (wide_group<LANES>()) next = load(p);
+  }
+  // the data of position p; with more, the fetch of position p_next starts
+  template <class Load> GFR_HD T take(const Load& load, int p, bool more, int p_next) {
+    if (!wide_group<LANES>()) return load(p);
+    const T now = next;
+    if (more) next = load(p_next);
+    return now;
+  }
+};
+// a leaf -> root row pass (mismatch, elimination): the position's record, packed tail record (CTA-wide groups), and
+// its branch's and diagonal admittances
+struct RowIn { I4 t, kq; D2 y, yd; };
+
+// A pool slot's hand-off to a parent, four fields: L D^-1 U (two rows), L D^-1 r, the branch's share of P, Q
+GFR_HD void add_hand_off(const D2* e, int np, D2& h0, D2& h1, D2& hc, D2& hf) {
+  const D2 c0 = e[0], c1 = e[np], cc = e[2 * np], fl = e[3 * np];
+  h0.x += c0.x; h0.y += c0.y; h1.x += c1.x; h1.y += c1.y; hc.x += cc.x; hc.y += cc.y;
+  hf.x += fl.x; hf.y += fl.y;
+}
+GFR_HD void put_hand_off(D2* e, int np, const D2 h0, const D2 h1, const D2 hc, const D2 hf) {
+  e[0] = h0; e[np] = h1; e[2 * np] = hc; e[3 * np] = hf;
+}
 
 // max |mismatch| of the present voltages (power_flow.py:150-166), as a leaf -> root row pass on the elimination
 // schedule: every branch is evaluated ONCE, by the bus below it, which keeps its own share (ga, al) and hands the
@@ -673,29 +674,35 @@ GFR_HD double newton_mismatch(const NGrp<LANES>& g, const Layout& lay, const int
   double mm = 0.0;
   D2 hf; hf.x = hf.y = 0.0;                             // (gl, ll) of the bus this lane handled in the previous row
   double ps_next = g.pspec((nrows - 1) * LANES + g.lane);
-  GFR_ROW_PIPE_DECL;
-  GFR_ROW_PIPE_FIRST((nrows - 1) * LANES + g.lane);
+  const auto row_in = [&](int p) {
+    RowIn r = {sched[p], I4(), gb[p], gbd[p]};
+    if (wide_group<LANES>()) r.kq = kids[p];
+    return r;
+  };
+  Ahead<LANES, RowIn> ahead;
+  ahead.first(row_in, (nrows - 1) * LANES + g.lane);
   for (int row = nrows - 1; row >= 0; --row) {
     const int p = row * LANES + g.lane;
-    GFR_ROW_PIPE_TAKE(p, row > 0, p - LANES);
+    const RowIn in = ahead.take(row_in, p, row > 0, p - LANES);
+    const I4 t = in.t;                                  // idle positions: record 0 -> bus 0, harmless
+    const D2 vk = g.ef(rec_bus(t)), vp = g.ef(rec_parent(t));
     const double ps = ps_next;
     if (row > 0) ps_next = g.pspec(p - LANES);
     if (t.z & FL_VALID) {
       const double v2 = fma(vk.x, vk.x, vk.y * vk.y);
-      const BranchT bt = branch_terms(vk, vp, yb);
+      const BranchT bt = branch_terms(vk, vp, in.y);
       if (!(t.z & FL_C_REG)) { hf.x = hf.y = 0.0; }
-      GFR_POOL_GATHER(t, kq, {
+      for_each_tail<LANES>(t, in.kq, child_slot, [&](int slot) {
         const D2 fl = g.poolp[3 * np + slot];
         hf.x += fl.x; hf.y += fl.y;
       });
-      const double P = fma(yd.x, v2, bt.ga) + hf.x, Q = fma(-yd.y, v2, bt.al) + hf.y;
+      const double P = fma(in.yd.x, v2, bt.ga) + hf.x, Q = fma(-in.yd.y, v2, bt.al) + hf.y;
       double aP = fabs(ps - P), aQ = fabs(Q);
       if ((t.z & (FL_PQ | FL_THETA)) != (FL_PQ | FL_THETA)) {   // slack: no equations; PV: no Q equation
         if (!(t.z & FL_THETA)) aP = 0.0;
         if (!(t.z & FL_PQ)) aQ = 0.0;
       }
-      const double loc = (aQ > aP || aQ != aQ) ? aQ : aP;
-      mm = (loc > mm || loc != loc) ? loc : mm;
+      mm = max_nan(mm, max_nan(aP, aQ));
       hf.x = bt.gl; hf.y = bt.ll;
       if (sibling_chains<LANES>() && rec_absorb(t) >= 0) {                         // the partial of an earlier sibling's chain
         const D2 fl = g.poolp[3 * np + rec_absorb(t)];
@@ -717,6 +724,43 @@ GFR_HD double newton_mismatch(const NGrp<LANES>& g, const Layout& lay, const int
 // each lane reads back what it wrote itself.  Their L2 round trip is taken off the critical path by
 // loading them TWO rows ahead into registers (the row loop is unrolled by two: even rows use the A set,
 // odd rows the B set).
+// D^-1 U (not in the first iteration: f0 holds it) and D^-1 r of a row into a register set.  Idle positions are
+// loaded too (their scratch entries exist): no record is needed this early.
+template <int LANES>
+GFR_HD void load_mv(const NGrp<LANES>& g, int P, const D2* f0, int row, D2& m0, D2& m1, D2& v) {
+  const int p = row * LANES + g.lane;
+  if (!f0) { m0 = ld_scratch(g.mg + p, g.pol); m1 = ld_scratch(g.mg + P + p, g.pol); }
+  v = ld_scratch(g.mg + 2 * P + p, g.pol);
+}
+struct BackIn { I4 t; D2 m0, m1; };                    // a position's record and, in the first iteration, D^-1 U
+// One row: `in` is its position's record (and first-iteration D^-1 U), m0s / m1s / vs the register set loaded two
+// rows earlier, refilled here for the row two ahead; hx is the correction of the bus this lane handled in the
+// previous row.
+template <int LANES>
+GFR_HD void back_update_row(const NGrp<LANES>& g, int nrows, int P, const D2* f0, double accel, int row,
+                            const BackIn& in, D2& hx, D2& m0s, D2& m1s, D2& vs) {
+  const I4 t = in.t;
+  const D2 e = g.efp[rec_bus(t)];
+  D2 m0 = m0s, m1 = m1s, v = vs;
+  if (f0) { m0 = in.m0; m1 = in.m1; }
+  if (row + 2 < nrows) load_mv(g, P, f0, row + 2, m0s, m1s, vs);
+  if (t.z & FL_VALID) {
+    D2 x = hx;
+    if (!(t.z & FL_P_REG)) x = g.poolp[x_slot_of(t.z)];
+    v.x = fma(-m0.x, x.x, fma(-m0.y, x.y, v.x));
+    v.y = fma(-m1.x, x.x, fma(-m1.y, x.y, v.y));
+    if (rec_kids_x_slot(t) >= 0) g.poolp[rec_kids_x_slot(t)] = v;
+    hx = v;
+    double sn, cs;
+    sincos_small(accel * v.x, &sn, &cs);
+    const double sc = fma(accel, v.y, 1.0);
+    D2 w;
+    w.x = sc * fma(e.x, cs, -e.y * sn);
+    w.y = sc * fma(e.x, sn, e.y * cs);
+    g.efp[rec_bus(t)] = w;
+  }
+  g.sync();
+}
 template <int LANES>
 GFR_HD void newton_back_update(const NGrp<LANES>& g, const Layout& lay, const int* simg, const D2* f0,
                                double accel) {
@@ -724,64 +768,23 @@ GFR_HD void newton_back_update(const NGrp<LANES>& g, const Layout& lay, const in
   const I4* sched = reinterpret_cast<const I4*>(simg + lay.o_sched);
   D2 a0, a1, av, b0, b1, bv;
   a0.x = a0.y = a1.x = a1.y = b0.x = b0.y = b1.x = b1.y = bv.x = bv.y = 0.0;
-  // idle positions are loaded too (their scratch entries exist): no record is needed this early
-#define GFR_LOAD_MV(row_, m0_, m1_, v_)                                    \
-  do {                                                                     \
-    const int ps_ = (row_) * LANES + g.lane;                               \
-    if (!f0) { m0_ = ld_scratch(g.mg + ps_, g.pol); m1_ = ld_scratch(g.mg + P + ps_, g.pol); } \
-    v_ = ld_scratch(g.mg + 2 * P + ps_, g.pol);                                   \
-  } while (0)
-  D2 hx; hx.x = hx.y = 0.0;                            // the correction of the bus this lane handled in the previous row
-#define GFR_BU_ROW(row_, m0_, m1_, v_)                                     \
-  do {                                                                     \
-    const int p = (row_) * LANES + g.lane;                                 \
-    I4 t;                                                                  \
-    if (wide_group<LANES>()) {                                             \
-      t = t_next;                                                          \
-      if ((row_) + 1 < nrows) t_next = sched[p + LANES];                   \
-    } else t = sched[p];                                                   \
-    const D2 e_now = g.efp[rec_bus(t)];                                    \
-    D2 m0 = m0_, m1 = m1_, v = v_;                                         \
-    if (f0) {                                                              \
-      if (wide_group<LANES>()) {                                           \
-        m0 = f0m0_next; m1 = f0m1_next;                                    \
-        if ((row_) + 1 < nrows) { f0m0_next = f0[2 * P + p + LANES]; f0m1_next = f0[3 * P + p + LANES]; } \
-      } else { m0 = f0[2 * P + p]; m1 = f0[3 * P + p]; }                   \
-    }                                                                      \
-    if ((row_) + 2 < nrows) GFR_LOAD_MV((row_) + 2, m0_, m1_, v_);         \
-    if (t.z & FL_VALID) {                                                  \
-      D2 x = hx;                                                           \
-      if (!(t.z & FL_P_REG)) x = g.poolp[x_slot_of(t.z)];                  \
-      v.x = fma(-m0.x, x.x, fma(-m0.y, x.y, v.x));                         \
-      v.y = fma(-m1.x, x.x, fma(-m1.y, x.y, v.y));                         \
-      if (rec_kids_x_slot(t) >= 0) g.poolp[rec_kids_x_slot(t)] = v;        \
-      hx = v;                                                              \
-      double sn, cs;                                                       \
-      sincos_small(accel * v.x, &sn, &cs);                                 \
-      const double sc = fma(accel, v.y, 1.0);                              \
-      D2* const ep = g.efp + rec_bus(t);                                   \
-      const D2 e = e_now;                                                  \
-      D2 w;                                                                \
-      w.x = sc * fma(e.x, cs, -e.y * sn);                                  \
-      w.y = sc * fma(e.x, sn, e.y * cs);                                   \
-      *ep = w;                                                             \
-    }                                                                      \
-    g.sync();                                                              \
-  } while (0)
-  GFR_LOAD_MV(0, a0, a1, av);
-  if (nrows > 1) GFR_LOAD_MV(1, b0, b1, bv);
-  I4 t_next;                                           // CTA-wide groups (image in global memory): the record one row ahead
-  t_next.x = t_next.y = t_next.z = t_next.w = 0;
-  D2 f0m0_next, f0m1_next;                             // ... and the flat-start D^-1 U rows in the first iteration
-  f0m0_next.x = f0m0_next.y = f0m1_next.x = f0m1_next.y = 0.0;
-  if (wide_group<LANES>()) t_next = sched[g.lane];
-  if (wide_group<LANES>() && f0) { f0m0_next = f0[2 * P + g.lane]; f0m1_next = f0[3 * P + g.lane]; }
+  D2 hx; hx.x = hx.y = 0.0;
+  load_mv(g, P, f0, 0, a0, a1, av);
+  if (nrows > 1) load_mv(g, P, f0, 1, b0, b1, bv);
+  const auto back_in = [&](int p) {
+    BackIn r = {sched[p], D2(), D2()};
+    if (f0) { r.m0 = f0[2 * P + p]; r.m1 = f0[3 * P + p]; }
+    return r;
+  };
+  Ahead<LANES, BackIn> ahead;
+  ahead.first(back_in, g.lane);
   for (int row = 0; row < nrows; row += 2) {
-    GFR_BU_ROW(row, a0, a1, av);
-    if (row + 1 < nrows) GFR_BU_ROW(row + 1, b0, b1, bv);
+    const int p = row * LANES + g.lane;
+    back_update_row(g, nrows, P, f0, accel, row, ahead.take(back_in, p, row + 1 < nrows, p + LANES), hx, a0, a1, av);
+    if (row + 1 < nrows)
+      back_update_row(g, nrows, P, f0, accel, row + 1, ahead.take(back_in, p + LANES, row + 2 < nrows, p + 2 * LANES),
+                      hx, b0, b1, bv);
   }
-#undef GFR_BU_ROW
-#undef GFR_LOAD_MV
 }
 
 template <int LANES>
@@ -815,8 +818,8 @@ GFR_HD void newton_solve(const NGrp<LANES>& g, const Layout& lay, const int* sim
         double aP = fabs(g.pspec(p) - pc.x), aQ = fabs(pc.y);
         if (!(fl & FL_THETA)) aP = 0.0;
         if (!(fl & FL_PQ)) aQ = 0.0;
-        const double loc = (aQ > aP || aQ != aQ) ? aQ : aP;
-        if (fl & FL_VALID) mm = (loc > mm || loc != loc) ? loc : mm;
+        const double loc = max_nan(aP, aQ);
+        if (fl & FL_VALID) mm = max_nan(mm, loc);
       }
       mm = g.gmax_nan(mm);
       out->max_mismatch = mm;
@@ -827,46 +830,35 @@ GFR_HD void newton_solve(const NGrp<LANES>& g, const Layout& lay, const int* sim
       }
       D2 hc; hc.x = hc.y = 0.0;                         // L v of the bus this lane eliminated in the previous row
       double ps_next = g.pspec((nrows - 1) * LANES + g.lane);     // the specified injection, one row ahead (an L2 round trip)
-      I4 t_next, kq_next; D2 pc_next, i0_next, i1_next, lp_next;   // CTA-wide groups: records and flat-start factors one row ahead
-      t_next.x = t_next.y = t_next.z = t_next.w = 0;
-      kq_next = t_next;
-      pc_next.x = pc_next.y = i0_next.x = i0_next.y = i1_next.x = i1_next.y = lp_next.x = lp_next.y = 0.0;
-      if (wide_group<LANES>()) {
-        const int p0 = (nrows - 1) * LANES + g.lane;
-        t_next = sched[p0]; pc_next = f0[5 * P + p0]; i0_next = f0[p0]; i1_next = f0[P + p0]; lp_next = f0[4 * P + p0];
-        kq_next = kids[p0];
-      }
+      struct F0In { I4 t, kq; D2 pc, i0, i1, lp; };   // record, packed tails, flat-profile (P, Q), D^-1 rows, (ll, gl)
+      const auto f0_in = [&](int p) {
+        F0In r = {sched[p], I4(), f0[5 * P + p], f0[p], f0[P + p], f0[4 * P + p]};
+        if (wide_group<LANES>()) r.kq = kids[p];
+        return r;
+      };
+      Ahead<LANES, F0In> ahead;
+      ahead.first(f0_in, (nrows - 1) * LANES + g.lane);
       for (int row = nrows - 1; row >= 0; --row) {
         const int p = row * LANES + g.lane;
-        I4 t, kq; D2 pc, i0, i1, lp;                    // record, flat-profile (P, Q), D^-1 rows, (ll, gl)
-        kq.x = kq.y = kq.z = kq.w = 0;
-        if (wide_group<LANES>()) {
-          t = t_next; pc = pc_next; i0 = i0_next; i1 = i1_next; lp = lp_next; kq = kq_next;
-          if (row > 0) {
-            kq_next = kids[p - LANES];
-            t_next = sched[p - LANES]; pc_next = f0[5 * P + p - LANES];
-            i0_next = f0[p - LANES]; i1_next = f0[P + p - LANES]; lp_next = f0[4 * P + p - LANES];
-          }
-        } else {
-          t = sched[p]; pc = f0[5 * P + p]; i0 = f0[p]; i1 = f0[P + p]; lp = f0[4 * P + p];
-        }
+        const F0In in = ahead.take(f0_in, p, row > 0, p - LANES);
+        const I4 t = in.t;
         const double ps = ps_next;
         if (row > 0) ps_next = g.pspec(p - LANES);
         if (t.z & FL_VALID) {
           if (!(t.z & FL_C_REG)) { hc.x = hc.y = 0.0; }
-          GFR_POOL_GATHER(t, kq, {
+          for_each_tail<LANES>(t, in.kq, child_slot, [&](int slot) {
             const D2 cc = g.poolp[2 * np + slot];
             hc.x += cc.x; hc.y += cc.y;
           });
           const D2 sc = hc;
-          double r0 = ps - pc.x - sc.x, r1 = 0.0 - pc.y - sc.y;
+          double r0 = ps - in.pc.x - sc.x, r1 = 0.0 - in.pc.y - sc.y;
           if (!(t.z & FL_THETA)) r0 = 0.0;
           if (!(t.z & FL_PQ)) r1 = 0.0;
           D2 v;
-          v.x = fma(i0.x, r0, i0.y * r1);
-          v.y = fma(i1.x, r0, i1.y * r1);
-          hc.x = fma(lp.x, v.x, lp.y * v.y);
-          hc.y = fma(-lp.y, v.x, lp.x * v.y);
+          v.x = fma(in.i0.x, r0, in.i0.y * r1);
+          v.y = fma(in.i1.x, r0, in.i1.y * r1);
+          hc.x = fma(in.lp.x, v.x, in.lp.y * v.y);
+          hc.y = fma(-in.lp.y, v.x, in.lp.x * v.y);
           if (sibling_chains<LANES>() && rec_absorb(t) >= 0) {
             const D2 cc = g.poolp[2 * np + rec_absorb(t)];
             hc.x += cc.x; hc.y += cc.y;
@@ -881,9 +873,6 @@ GFR_HD void newton_solve(const NGrp<LANES>& g, const Layout& lay, const int* sim
       // ---- the iterate is expected to have converged (quadratic rate seen so far): a mismatch-only
       //      pass settles it without the elimination
       if (rate * mm_prev * mm_prev < 0.25 * tol) {
-#ifdef GFR_EMU_STATS
-        ++gfr_emu_stats[0];
-#endif
         mm = newton_mismatch(g, lay, simg, dimg);
         if (mm < tol) {
           out->max_mismatch = mm;
@@ -899,24 +888,26 @@ GFR_HD void newton_solve(const NGrp<LANES>& g, const Layout& lay, const int* sim
       D2 h0, h1, hc, hf;                               // what the bus this lane eliminated in the previous row hands up
       h0.x = h0.y = h1.x = h1.y = hc.x = hc.y = hf.x = hf.y = 0.0;
       double ps_next = g.pspec((nrows - 1) * LANES + g.lane);     // the specified injection, one row ahead (an L2 round trip)
-      GFR_ROW_PIPE_DECL;
-      GFR_ROW_PIPE_FIRST((nrows - 1) * LANES + g.lane);
+      const auto row_in = [&](int p) {
+        RowIn r = {sched[p], I4(), gb[p], gbd[p]};
+        if (wide_group<LANES>()) r.kq = kids[p];
+        return r;
+      };
+      Ahead<LANES, RowIn> ahead;
+      ahead.first(row_in, (nrows - 1) * LANES + g.lane);
       for (int row = nrows - 1; row >= 0; --row) {
         const int p = row * LANES + g.lane;
-        GFR_ROW_PIPE_TAKE(p, row > 0, p - LANES);
+        const RowIn in = ahead.take(row_in, p, row > 0, p - LANES);
+        const I4 t = in.t;
+        const D2 vk = g.ef(rec_bus(t)), vp = g.ef(rec_parent(t)), yd = in.yd;
         const double ps = ps_next;
         if (row > 0) ps_next = g.pspec(p - LANES);
         if (t.z & FL_VALID) {
           const double v2 = fma(vk.x, vk.x, vk.y * vk.y);
-          const BranchT bt = branch_terms(vk, vp, yb);
+          const BranchT bt = branch_terms(vk, vp, in.y);
           // children's contributions: plain sums, the heir first - it is what the lane still holds in h*
           if (!(t.z & FL_C_REG)) { h0.x = h0.y = h1.x = h1.y = hc.x = hc.y = hf.x = hf.y = 0.0; }
-          GFR_POOL_GATHER(t, kq, {
-            const D2* e = g.poolp + slot;
-            const D2 c0 = e[0], c1 = e[np], cc = e[2 * np], fl = e[3 * np];
-            h0.x += c0.x; h0.y += c0.y; h1.x += c1.x; h1.y += c1.y; hc.x += cc.x; hc.y += cc.y;
-            hf.x += fl.x; hf.y += fl.y;
-          });
+          for_each_tail<LANES>(t, in.kq, child_slot, [&](int slot) { add_hand_off(g.poolp + slot, np, h0, h1, hc, hf); });
           const D2 s0 = h0, s1 = h1, sc = hc, sf = hf;
           const double Pk = fma(yd.x, v2, bt.ga) + sf.x, Q = fma(-yd.y, v2, bt.al) + sf.y;
           D2 d0, d1, r;
@@ -935,8 +926,7 @@ GFR_HD void newton_solve(const NGrp<LANES>& g, const Layout& lay, const int* sim
             if (!(t.z & FL_THETA)) { aP = 0.0; d0.x = 1.0; d0.y = 0.0; r.x = 0.0; u00 = 0.0; u01 = 0.0; }
             if (!(t.z & FL_PQ)) { aQ = 0.0; d1.x = 0.0; d1.y = 1.0; r.y = 0.0; u10 = 0.0; u11 = 0.0; }
           }
-          const double loc = (aQ > aP || aQ != aQ) ? aQ : aP;
-          mm = (loc > mm || loc != loc) ? loc : mm;
+          mm = max_nan(mm, max_nan(aP, aQ));
           const double det = fma(d0.x, d1.y, -d0.y * d1.x);
           if (det == 0.0) singular = 1;                 // dgesv's exact-zero pivot (:188-190)
           const double inv = rcp_fast(det);
@@ -956,27 +946,16 @@ GFR_HD void newton_solve(const NGrp<LANES>& g, const Layout& lay, const int* sim
           hc.x = fma(bt.ll, v.x, bt.gl * v.y);
           hc.y = fma(-bt.gl, v.x, bt.ll * v.y);
           hf.x = bt.gl; hf.y = bt.ll;
-          if (sibling_chains<LANES>() && rec_absorb(t) >= 0) {                     // the partial of an earlier sibling's chain
-            const D2* e = g.poolp + rec_absorb(t);
-            const D2 c0 = e[0], c1 = e[np], cc = e[2 * np], fl = e[3 * np];
-            h0.x += c0.x; h0.y += c0.y; h1.x += c1.x; h1.y += c1.y; hc.x += cc.x; hc.y += cc.y;
-            hf.x += fl.x; hf.y += fl.y;
-          }
+          if (sibling_chains<LANES>() && rec_absorb(t) >= 0)                       // the partial of an earlier sibling's chain
+            add_hand_off(g.poolp + rec_absorb(t), np, h0, h1, hc, hf);
           st_scratch(g.mg + p, m0, g.pol);               // needed again in the back-substitution only
           st_scratch(g.mg + P + p, m1, g.pol);
           st_scratch(g.mg + 2 * P + p, v, g.pol);
-          if (!(t.z & FL_P_REG)) {
-            D2* const own = g.poolp + pool_slot_of(t.z);
-            own[0] = h0; own[np] = h1; own[2 * np] = hc; own[3 * np] = hf;
-          }
+          if (!(t.z & FL_P_REG)) put_hand_off(g.poolp + pool_slot_of(t.z), np, h0, h1, hc, hf);
         }
         g.sync();
       }
       mm = g.gmax_nan(mm);
-#ifdef GFR_EMU_STATS
-      ++gfr_emu_stats[1];
-      if (mm < tol) ++gfr_emu_stats[2];
-#endif
       out->max_mismatch = mm;
       if (mm < tol) {                                   // checked before the update (:168-171)
         out->converged = 1;
@@ -1029,6 +1008,16 @@ GFR_HD void newton_solve(const NGrp<LANES>& g, const Layout& lay, const int* sim
 // by the host.  Convergence then needs max |dV| AND max |e| below the tolerance.
 // TIES is a compile-time switch: the radial kernels do not carry the compensation code (4 more registers cost the
 // IEEE-34 sweep its second CTA per SM: 270 M -> 238 M env-steps/s).
+// adds to a the current the ties feed into bus k: + J at a to-end, - J at a from-end (nt = 0: nothing, no code)
+GFR_HD void add_tie_current(const int* tie_ptr, const int* tie_inc, const D2* jt, int nt, int k, D2& a) {
+  if (!nt) return;
+  for (int q = tie_ptr[k]; q < tie_ptr[k + 1]; ++q) {
+    const int e = tie_inc[q];
+    const D2 j = jt[e >> 1];
+    if (e & 1) { a.x += j.x; a.y += j.y; }
+    else { a.x -= j.x; a.y -= j.y; }
+  }
+}
 template <int LANES, bool TIES>
 GFR_HD void sweep_solve(const SGrp<LANES>& g, const Layout& lay, const int* simg,
                         const double* dimg, double tol, int max_it, SolveStat* out) {
@@ -1048,18 +1037,6 @@ GFR_HD void sweep_solve(const SGrp<LANES>& g, const Layout& lay, const int* simg
     for (int i = g.lane; i < nt; i += LANES) g.jt[i] = z0;
     g.sync();
   }
-  // current the ties feed into bus k: + J at a to-end, - J at a from-end
-#define GFR_TIE_CURRENT(k_, a_)                                            \
-  do {                                                                     \
-    if (nt) {                                                              \
-      for (int q_ = tie_ptr[(k_)]; q_ < tie_ptr[(k_) + 1]; ++q_) {         \
-        const int e_ = tie_inc[q_];                                        \
-        const D2 j_ = g.jt[e_ >> 1];                                       \
-        if (e_ & 1) { (a_).x += j_.x; (a_).y += j_.y; }                    \
-        else { (a_).x -= j_.x; (a_).y -= j_.y; }                           \
-      }                                                                    \
-    }                                                                      \
-  } while (0)
   for (int it = 0; it < max_it; ++it) {
     if (LANES == 1) {
       // one thread per instance: buses are numbered parent before child, so a plain descending loop that
@@ -1075,7 +1052,7 @@ GFR_HD void sweep_solve(const SGrp<LANES>& g, const Layout& lay, const int* simg
         const double w = (t.w & FL_THETA) ? p_k * rcp_fast(fma(v.x, v.x, v.y * v.y)) : 0.0;
         D2 a = g.at2(S_JR, k);
         a.x = fma(w, v.x, a.x); a.y = fma(w, v.y, a.y);
-        GFR_TIE_CURRENT(k, a);
+        add_tie_current(tie_ptr, tie_inc, g.jt, nt, k, a);
         g.at2(S_JR, k) = a;
         if (k > 0) { D2& ap = g.at2(S_JR, t.x); ap.x += a.x; ap.y += a.y; }
       }
@@ -1092,7 +1069,7 @@ GFR_HD void sweep_solve(const SGrp<LANES>& g, const Layout& lay, const int* simg
           const double w = (t.w & FL_THETA) ? g.at(S_P, k) * rcp_fast(fma(v.x, v.x, v.y * v.y)) : 0.0;   // conj(S / V) = P V / |V|^2
           D2 a;
           a.x = w * v.x; a.y = w * v.y;
-          GFR_TIE_CURRENT(k, a);
+          add_tie_current(tie_ptr, tie_inc, g.jt, nt, k, a);
 #pragma unroll 1
           for (int q = t.y; q < t.z; ++q) {
             const D2 ac = g.at2(S_JR, child_idx[q]);
@@ -1127,8 +1104,8 @@ GFR_HD void sweep_solve(const SGrp<LANES>& g, const Layout& lay, const int* simg
           D2 vn;
           vn.x = vslack + w.x; vn.y = w.y;
           const double de = fabs(vn.x - vo.x), df = fabs(vn.y - vo.y);
-          const double loc = (df > de || df != df) ? df : de;
-          mm = (loc > mm || loc != loc) ? loc : mm;
+          const double loc = max_nan(de, df);
+          mm = max_nan(mm, loc);
           g.at2(F_E, k) = vn;
         }
       }
@@ -1153,8 +1130,8 @@ GFR_HD void sweep_solve(const SGrp<LANES>& g, const Layout& lay, const int* simg
             D2 vn;
             vn.x = vslack + w.x; vn.y = w.y;
             const double de = fabs(vn.x - vo.x), df = fabs(vn.y - vo.y);
-            const double loc = (df > de || df != df) ? df : de;
-            mm = (loc > mm || loc != loc) ? loc : mm;
+            const double loc = max_nan(de, df);
+            mm = max_nan(mm, loc);
             g.at2(F_E, k) = vn;
           }
         }
@@ -1172,8 +1149,8 @@ GFR_HD void sweep_solve(const SGrp<LANES>& g, const Layout& lay, const int* simg
       vn.y = (0.0 - ws.y) + w.y;
       if (k == ks) { vn.x = vslack; vn.y = 0.0; }
       const double de = fabs(vn.x - vo.x), df = fabs(vn.y - vo.y);
-      const double loc = (df > de || df != df) ? df : de;
-      mm = (loc > mm || loc != loc) ? loc : mm;
+      const double loc = max_nan(de, df);
+      mm = max_nan(mm, loc);
       g.at2(F_E, k) = vn;
     }
     if (nt) {
@@ -1190,8 +1167,8 @@ GFR_HD void sweep_solve(const SGrp<LANES>& g, const Layout& lay, const int* simg
         e.y = (va.y - vb.y) - fma(z.x, j.y, z.y * j.x);
         et[i] = e;
         const double de = fabs(e.x), df = fabs(e.y);
-        const double loc = (df > de || df != df) ? df : de;
-        mm = (loc > mm || loc != loc) ? loc : mm;
+        const double loc = max_nan(de, df);
+        mm = max_nan(mm, loc);
       }
       g.sync();
       for (int i = g.lane; i < nt; i += LANES) {
@@ -1215,7 +1192,6 @@ GFR_HD void sweep_solve(const SGrp<LANES>& g, const Layout& lay, const int* simg
       break;
     }
   }
-#undef GFR_TIE_CURRENT
 }
 
 // From -> to flow of the branch above the bus at position p (power_flow.py:329-358): P (pu), |S| (pu), series loss (pu)
@@ -1618,8 +1594,8 @@ GFR_HD void step_instance(const typename GroupOf<LANES, SOLVER>::type& g, const 
         double vm = sqrt(e * e + f * f);
         ob.put2(2 * i, vm, atan2_bus(f, e));
         dev += fabs(vm - 1.0);
-        vmax = (vm > vmax || vm != vm) ? vm : vmax;
-        vmin = (vm < vmin || vm != vm) ? vm : vmin;
+        vmax = max_nan(vmax, vm);
+        vmin = min_nan(vmin, vm);
         v_hi |= vm > cfg.v_max;
         v_lo |= vm < cfg.v_min;
       }

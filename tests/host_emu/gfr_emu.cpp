@@ -203,7 +203,3 @@ void emu_noise_fill(long long B, int n_slots, const uint64_t* seeds, const uint6
 }
 
 }  // extern "C"
-
-#ifdef GFR_EMU_STATS
-extern "C" long long* emu_stats(void) { return gfr::gfr_emu_stats; }
-#endif
