@@ -16,8 +16,7 @@ import numpy as np
 from .topology import FeederSoA
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-# GFR_B200_LIB: a tuning aid (tools/: kernels built with other compile-time settings under build_variants/)
-LIB_PATH = os.environ.get("GFR_B200_LIB") or os.path.join(HERE, "libgfr_b200.so")
+LIB_PATH = os.path.join(HERE, "libgfr_b200.so")
 
 GFR_OK, GFR_E_ARG, GFR_E_CUDA, GFR_E_LIMIT = 0, -1, -2, -3
 SOLVER_SWEEP, SOLVER_NEWTON = 0, 1

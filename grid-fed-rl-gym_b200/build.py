@@ -59,5 +59,4 @@ def build(force: bool = False, verbose: bool = False, defines=(), out: str = OUT
 
 
 if __name__ == "__main__":
-    print(build(force="--force" in sys.argv, verbose="-v" in sys.argv,
-                defines=[a[2:] for a in sys.argv[1:] if a.startswith("-D")]))
+    print(build(force="--force" in sys.argv, verbose="-v" in sys.argv))

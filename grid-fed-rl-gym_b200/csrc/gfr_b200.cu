@@ -13,7 +13,6 @@
 #include <atomic>
 #include <cmath>
 #include <cstdio>
-#include <cstdlib>
 #include <cstring>
 #include <map>
 #include <string>
@@ -73,7 +72,7 @@ constexpr int kRedBytes = 128;    // cross-warp reduction scratch of a CTA-wide 
 // Shared memory of a CTA: [mbarrier 16 B][feeder image, if staged][reduction scratch, if LANES > 32][slots]
 template <int LANES, int SOLVER>
 __device__ __forceinline__ typename GroupOf<LANES, SOLVER>::type
-make_group(const Layout& lay, unsigned char* work, int slot_bytes, D2* mscratch) {
+make_group(const Layout& lay, unsigned char* work, int slot_bytes, D2* mscratch, double* p_local) {
   typename GroupOf<LANES, SOLVER>::type g;
   g.lane = threadIdx.x % LANES;
   g.mask = (LANES >= 32) ? 0xffffffffu
@@ -83,15 +82,8 @@ make_group(const Layout& lay, unsigned char* work, int slot_bytes, D2* mscratch)
   const int slot = threadIdx.x / LANES;
   const int E = blockDim.x / LANES;
   D2* mg = mscratch ? mscratch + ((size_t)blockIdx.x * E + slot) * (newton_scratch_doubles(lay.P) / 2) : nullptr;
-  bind_slot(g, work + (size_t)slot * slot_bytes, lay, mg);
+  bind_slot(g, work + (size_t)slot * slot_bytes, lay, mg, p_local);
   return g;
-}
-
-// One thread per instance, small feeder, sweep: the specified injections live in the thread's local array
-// (the host sized the shared-memory slot without them, sweep_p_local)
-template <int LANES> __device__ __forceinline__ void use_local_injections(NGrp<LANES>&, const Layout&, double*) {}
-template <int LANES> __device__ __forceinline__ void use_local_injections(SGrp<LANES>& g, const Layout& lay, double* p_local) {
-  if (sweep_p_local(LANES, lay.n)) g.pp = p_local;
 }
 
 // IMG_SMEM: the feeder image is staged into shared memory (small / medium feeders); otherwise it is
@@ -107,10 +99,9 @@ step_kernel(const Layout lay, const EnvCfg cfg, const void* __restrict__ img, co
   if (IMG_SMEM) stage_image(smem, img, lay.img_bytes);
   const int* simg = IMG_SMEM ? (const int*)(smem + kSmemHeader) : (const int*)img;
   const double* dimg = IMG_SMEM ? (const double*)(smem + kSmemHeader) : (const double*)img;
-  auto g = make_group<LANES, SOLVER>(lay, smem + kSmemHeader + (IMG_SMEM ? lay.img_bytes : 0),
-                                     slot_bytes, mscratch);
   double p_local[LANES == 1 && SOLVER != SOLVER_NEWTON ? SWEEP_P_LOCAL_MAX : 1];
-  use_local_injections(g, lay, p_local);
+  auto g = make_group<LANES, SOLVER>(lay, smem + kSmemHeader + (IMG_SMEM ? lay.img_bytes : 0),
+                                     slot_bytes, mscratch, p_local);
   const int E = blockDim.x / LANES;
   for (long long env = (long long)blockIdx.x * E + threadIdx.x / LANES; env < B; env += (long long)gridDim.x * E)
     step_instance<LANES, SOLVER>(g, lay, simg, dimg, cfg, env, state, obs, obs_prev, obs_f32, actions, noise, o);
@@ -124,10 +115,9 @@ solve_kernel(const Layout lay, const EnvCfg cfg, const void* __restrict__ img, c
   if (IMG_SMEM) stage_image(smem, img, lay.img_bytes);
   const int* simg = IMG_SMEM ? (const int*)(smem + kSmemHeader) : (const int*)img;
   const double* dimg = IMG_SMEM ? (const double*)(smem + kSmemHeader) : (const double*)img;
-  auto g = make_group<LANES, SOLVER>(lay, smem + kSmemHeader + (IMG_SMEM ? lay.img_bytes : 0),
-                                     slot_bytes, mscratch);
   double p_local[LANES == 1 && SOLVER != SOLVER_NEWTON ? SWEEP_P_LOCAL_MAX : 1];
-  use_local_injections(g, lay, p_local);
+  auto g = make_group<LANES, SOLVER>(lay, smem + kSmemHeader + (IMG_SMEM ? lay.img_bytes : 0),
+                                     slot_bytes, mscratch, p_local);
   const int E = blockDim.x / LANES;
   for (long long env = (long long)blockIdx.x * E + threadIdx.x / LANES; env < B; env += (long long)gridDim.x * E)
     solve_instance<LANES, SOLVER>(g, lay, simg, dimg, cfg, env, p_inj, o);
@@ -247,6 +237,8 @@ struct DeviceGuard {
   ~DeviceGuard() { if (ok && prev >= 0 && prev != cur) cudaSetDevice(prev); }
   int cur = -1;
 };
+// what an entry point that needs the device returns when DeviceGuard could not switch to it
+int no_device() { return fail(GFR_E_CUDA, "no usable CUDA device (this library has no CPU fallback)"); }
 
 }  // namespace
 
@@ -353,52 +345,23 @@ int auto_lanes_rule(int n, int solver, int depth) {
   return 128;                      // one CTA per instance
 }
 
-template <int SOLVER>
-const void* step_fn(int lanes, bool img_smem) {
-  if (img_smem) {
-    switch (lanes) {
-      case 1: return (const void*)step_kernel<1, SOLVER, true>;
-      case 2: return (const void*)step_kernel<2, SOLVER, true>;
-      case 4: return (const void*)step_kernel<4, SOLVER, true>;
-      case 8: return (const void*)step_kernel<8, SOLVER, true>;
-      case 16: return (const void*)step_kernel<16, SOLVER, true>;
-      case 32: return (const void*)step_kernel<32, SOLVER, true>;
-    }
-  } else {
-    switch (lanes) {
-      case 32: return (const void*)step_kernel<32, SOLVER, false>;
-      case 64: return (const void*)step_kernel<64, SOLVER, false>;
-      case 128: return (const void*)step_kernel<128, SOLVER, false>;
-      case 256: return (const void*)step_kernel<256, SOLVER, false>;
-    }
-  }
-  return nullptr;
+// The step or solve kernel of one (lanes, image placement) out of the lane list L it is compiled for: 1 - 32 lanes
+// with the image in shared memory, 32 - 256 without it; nullptr for any other lane count
+template <int SOLVER, bool IMG_SMEM, int... L>
+const void* kernel_in(bool step, int lanes) {
+  const void* fn = nullptr;
+  auto pick = [&](int l, const void* step_k, const void* solve_k) { if (lanes == l) fn = step ? step_k : solve_k; };
+  (pick(L, (const void*)step_kernel<L, SOLVER, IMG_SMEM>, (const void*)solve_kernel<L, SOLVER, IMG_SMEM>), ...);
+  return fn;
 }
 template <int SOLVER>
-const void* solve_fn(int lanes, bool img_smem) {
-  if (img_smem) {
-    switch (lanes) {
-      case 1: return (const void*)solve_kernel<1, SOLVER, true>;
-      case 2: return (const void*)solve_kernel<2, SOLVER, true>;
-      case 4: return (const void*)solve_kernel<4, SOLVER, true>;
-      case 8: return (const void*)solve_kernel<8, SOLVER, true>;
-      case 16: return (const void*)solve_kernel<16, SOLVER, true>;
-      case 32: return (const void*)solve_kernel<32, SOLVER, true>;
-    }
-  } else {
-    switch (lanes) {
-      case 32: return (const void*)solve_kernel<32, SOLVER, false>;
-      case 64: return (const void*)solve_kernel<64, SOLVER, false>;
-      case 128: return (const void*)solve_kernel<128, SOLVER, false>;
-      case 256: return (const void*)solve_kernel<256, SOLVER, false>;
-    }
-  }
-  return nullptr;
+const void* kernel_of(bool step, int lanes, bool img_smem) {
+  return img_smem ? kernel_in<SOLVER, true, 1, 2, 4, 8, 16, 32>(step, lanes)
+                  : kernel_in<SOLVER, false, 32, 64, 128, 256>(step, lanes);
 }
 const void* kernel_fn(bool step, int solver, int lanes, bool img_smem, bool ties) {
-  if (solver == GFR_SOLVER_NEWTON) return step ? step_fn<SOLVER_NEWTON>(lanes, img_smem) : solve_fn<SOLVER_NEWTON>(lanes, img_smem);
-  if (ties) return step ? step_fn<SOLVER_SWEEP_TIES>(lanes, img_smem) : solve_fn<SOLVER_SWEEP_TIES>(lanes, img_smem);
-  return step ? step_fn<SOLVER_SWEEP>(lanes, img_smem) : solve_fn<SOLVER_SWEEP>(lanes, img_smem);
+  if (solver == GFR_SOLVER_NEWTON) return kernel_of<SOLVER_NEWTON>(step, lanes, img_smem);
+  return ties ? kernel_of<SOLVER_SWEEP_TIES>(step, lanes, img_smem) : kernel_of<SOLVER_SWEEP>(step, lanes, img_smem);
 }
 
 // One candidate split of an SM: `c` CTAs of E instance slots each.
@@ -547,11 +510,17 @@ int launch_solve(const ImageDev* im, const LaunchPlan& p, const void* fn, const 
   return GFR_OK;
 }
 
+// the stopping rule of every solve
+int check_stopping(const gfr_solver_cfg* c) {
+  if (c->max_iterations < 1) return fail(GFR_E_ARG, "max_iterations must be >= 1");
+  if (!(c->tolerance > 0.0)) return fail(GFR_E_ARG, "tolerance must be > 0");
+  return GFR_OK;
+}
+
 int check_solver_cfg(const gfr_feeder* f, const gfr_solver_cfg* c) {
   if (c->solver != GFR_SOLVER_SWEEP && c->solver != GFR_SOLVER_NEWTON)
     return fail(GFR_E_ARG, "solver must be GFR_SOLVER_SWEEP or GFR_SOLVER_NEWTON");
-  if (c->max_iterations < 1) return fail(GFR_E_ARG, "max_iterations must be >= 1");
-  if (!(c->tolerance > 0.0)) return fail(GFR_E_ARG, "tolerance must be > 0");
+  if (int rc = check_stopping(c)) return rc;
   if (c->solver == GFR_SOLVER_SWEEP && f->has_pv)
     return fail(GFR_E_ARG, "the sweep solver handles slack + PQ buses only; use GFR_SOLVER_NEWTON for PV buses");
   return GFR_OK;
@@ -578,7 +547,7 @@ int gfr_feeder_create(const gfr_feeder_desc* d, int device, gfr_feeder** out) {
     if (!complaint.empty()) return fail(GFR_E_ARG, complaint);
   }
   DeviceGuard guard(device);
-  if (!guard.ok) return fail(GFR_E_CUDA, "no usable CUDA device (this library has no CPU fallback)");
+  if (!guard.ok) return no_device();
   cudaDeviceProp prop;
   GFR_CUDA(cudaGetDeviceProperties(&prop, device));
   auto* f = new gfr_feeder();
@@ -623,12 +592,7 @@ static int fill_env_cfg(const gfr_feeder* f, const gfr_env_cfg* c, EnvCfg* out) 
   if (int rc = check_solver_cfg(f, &c->solver)) return rc;
   if (!(c->timestep > 0.0)) return fail(GFR_E_ARG, "timestep must be > 0");
   if (c->episode_length < 1) return fail(GFR_E_ARG, "episode_length must be >= 1");
-  out->dt = c->timestep; out->v_min = c->v_min; out->v_max = c->v_max; out->f_min = c->f_min;
-  out->f_max = c->f_max; out->penalty = c->safety_penalty; out->load_noise = c->load_noise;
-  out->tol = c->solver.tolerance;
-  out->accel = c->solver.solver == GFR_SOLVER_NEWTON ? (c->solver.acceleration != 0.0 ? c->solver.acceleration : 1.0) : 1.0;
-  out->episode_length = c->episode_length; out->stochastic_loads = c->stochastic_loads != 0;
-  out->weather_variation = c->weather_variation != 0; out->max_it = c->solver.max_iterations;
+  *out = env_cfg_of(c);
   return GFR_OK;
 }
 
@@ -653,7 +617,7 @@ int gfr_env_create(const gfr_feeder* f, int64_t n_envs, const gfr_env_cfg* cfg, 
   EnvCfg ec;
   if (int rc = fill_env_cfg(f, cfg, &ec)) return rc;
   DeviceGuard guard(f->device);
-  if (!guard.ok) return fail(GFR_E_CUDA, "no usable CUDA device (this library has no CPU fallback)");
+  if (!guard.ok) return no_device();
   LaunchPlan plan;
   const void* fn = nullptr;
   const ImageDev* im = nullptr;
@@ -774,36 +738,22 @@ int gfr_env_reset(gfr_env* e, const uint64_t* seeds, const uint8_t* mask, const 
   return launch_reset(e, seeds, mask, noise, start_time, 0, (cudaStream_t)stream);
 }
 
-static StepOut step_out_of(const gfr_step_out* out) {
-  StepOut o{};
-  if (out) {
-    o.reward = out->reward; o.terminated = out->terminated; o.truncated = out->truncated;
-    o.error = out->error; o.converged = out->converged; o.iterations = out->iterations;
-    o.max_voltage = out->max_voltage; o.min_voltage = out->min_voltage; o.losses = out->losses;
-    o.max_mismatch = out->max_mismatch; o.violations = out->violations;
-    o.violation_count = out->violation_count; o.current_step = out->current_step;
-    o.episode_reward = out->episode_reward; o.noise_used = out->noise_used;
-  }
-  return o;
-}
-
 int gfr_env_step(gfr_env* e, const double* actions, const double* noise, const gfr_step_out* out,
                  void* stream) {
   if (!e || !actions) return fail(GFR_E_ARG, "null argument");
-  const StepOut o = step_out_of(out);
+  const StepOut o = out ? *out : StepOut{};
   DeviceGuard guard(e->f->device);
   return launch_step(e, actions, noise, o, (cudaStream_t)stream);
 }
 
 int gfr_env_reset_outputs(gfr_env* e, const uint8_t* mask, const gfr_step_out* out, void* stream) {
   if (!e || !out) return fail(GFR_E_ARG, "null argument");
-  const StepOut o = step_out_of(out);
   DeviceGuard guard(e->f->device);
   const long long B = e->B;
   const int threads = 256;
   long long blocks = (B + threads - 1) / threads;
   if (blocks > 4LL * e->f->sm_count) blocks = 4LL * e->f->sm_count;
-  reset_outputs_kernel<<<(unsigned)blocks, threads, 0, (cudaStream_t)stream>>>(o, mask, B);
+  reset_outputs_kernel<<<(unsigned)blocks, threads, 0, (cudaStream_t)stream>>>(*out, mask, B);
   GFR_CUDA(cudaGetLastError());
   g_launches.fetch_add(1);
   return GFR_OK;
@@ -815,19 +765,12 @@ int gfr_solve(const gfr_feeder* f, int64_t B, const double* p_inj, const gfr_sol
   if (B < 1) return fail(GFR_E_ARG, "B must be >= 1");
   if (int rc = check_solver_cfg(f, cfg)) return rc;
   DeviceGuard guard(f->device);
-  if (!guard.ok) return fail(GFR_E_CUDA, "no usable CUDA device (this library has no CPU fallback)");
+  if (!guard.ok) return no_device();
   LaunchPlan plan;
   const void* fn = nullptr;
   const ImageDev* im = nullptr;
   if (int rc = plan_launch(f, false, cfg->solver, cfg->lanes, B, &plan, &fn, &im)) return rc;
-  EnvCfg ec{};
-  ec.tol = cfg->tolerance; ec.max_it = cfg->max_iterations;
-  ec.accel = cfg->acceleration != 0.0 ? cfg->acceleration : 1.0;
-  SolOut o{};
-  o.converged = out->converged; o.iterations = out->iterations; o.bus_voltages = out->bus_voltages;
-  o.bus_angles = out->bus_angles; o.line_flows = out->line_flows; o.line_loadings = out->line_loadings;
-  o.losses = out->losses; o.max_mismatch = out->max_mismatch;
-  return launch_solve(im, plan, fn, ec, p_inj, o, B, (cudaStream_t)stream);
+  return launch_solve(im, plan, fn, env_cfg_of(cfg), p_inj, *out, B, (cudaStream_t)stream);
 }
 
 int gfr_network_create(const gfr_network_desc* d, int device, gfr_network** out) {
@@ -873,7 +816,7 @@ int gfr_network_create(const gfr_network_desc* d, int device, gfr_network** out)
     adj_ptr[i + 1] = (int32_t)adj_idx.size();
   }
   DeviceGuard guard(device);
-  if (!guard.ok) return fail(GFR_E_CUDA, "no usable CUDA device (this library has no CPU fallback)");
+  if (!guard.ok) return no_device();
   cudaDeviceProp prop;
   GFR_CUDA(cudaGetDeviceProperties(&prop, device));
   if ((N <= 127 ? dense_reg_smem_bytes(n, N) : dense_smem_bytes(n, N)) > (size_t)prop.sharedMemPerBlockOptin)
@@ -922,10 +865,9 @@ int gfr_network_solve(const gfr_network* net, int64_t B, const double* p_inj, co
                       const gfr_sol_out* out, void* stream) {
   if (!net || !p_inj || !cfg || !out) return fail(GFR_E_ARG, "null argument");
   if (B < 1) return fail(GFR_E_ARG, "B must be >= 1");
-  if (cfg->max_iterations < 1) return fail(GFR_E_ARG, "max_iterations must be >= 1");
-  if (!(cfg->tolerance > 0.0)) return fail(GFR_E_ARG, "tolerance must be > 0");
+  if (int rc = check_stopping(cfg)) return rc;
   DeviceGuard guard(net->device);
-  if (!guard.ok) return fail(GFR_E_CUDA, "no usable CUDA device (this library has no CPU fallback)");
+  if (!guard.ok) return no_device();
   // kernel choice: [J | mismatch] in registers up to 127 unknowns (cfg->lanes: 0 = this choice, 1 = always the
   // shared-memory kernel, 2 = the register kernel or GFR_E_LIMIT)
   typedef void (*dense_fn)(const NetDev, const double, const int, const double, const double*, const SolOut, const long long);
@@ -939,35 +881,14 @@ int gfr_network_solve(const gfr_network* net, int64_t B, const double* p_inj, co
   if (in_regs) {
     smem = dense_reg_smem_bytes(net->nd.n, N);
     // 8 x TX threads, R = ceil(N / 8) register rows each: TX = 8 up to 56 unknowns, 16 up to 96, 32 above (measured
-    // sweep, profiles/r01_tune_dense.txt)
-    // (GFR_DENSE_TX overrides the choice where the tile fits, for tuning)
-    // (the tuning sweep, tools/tune_dense.py, needs a build with -DGFR_DENSE_ALL_SHAPES: every thread grid at every
-    // R it can hold, selected with GFR_DENSE_TX; the default build carries the 16 shapes the rule above uses)
-#ifdef GFR_DENSE_ALL_SHAPES
-#define GFR_ALT(...) __VA_ARGS__
-#else
-#define GFR_ALT(...) nullptr
-#endif
+    // sweep, profiles/r01_tune_dense.txt).  R alone sets TX: 8 for R 1 - 7, 16 for R 8 - 12, 32 for R 13 - 16
 #define K dense_solve_reg_kernel
-    static const dense_fn by_tx8[] = { nullptr, K<8, 1>, K<8, 2>, K<8, 3>, K<8, 4>, K<8, 5>, K<8, 6>, K<8, 7>,
-                                       GFR_ALT(K<8, 8>), GFR_ALT(K<8, 9>) };
-    static const dense_fn by_tx16[] = { nullptr, nullptr, GFR_ALT(K<16, 2>), GFR_ALT(K<16, 3>), GFR_ALT(K<16, 4>),
-                                        GFR_ALT(K<16, 5>), GFR_ALT(K<16, 6>), GFR_ALT(K<16, 7>), K<16, 8>, K<16, 9>,
-                                        K<16, 10>, K<16, 11>, K<16, 12> };
-    static const dense_fn by_tx32[] = { nullptr, nullptr, nullptr, nullptr, GFR_ALT(K<32, 4>), GFR_ALT(K<32, 5>),
-                                        GFR_ALT(K<32, 6>), GFR_ALT(K<32, 7>), GFR_ALT(K<32, 8>), GFR_ALT(K<32, 9>),
-                                        GFR_ALT(K<32, 10>), GFR_ALT(K<32, 11>), GFR_ALT(K<32, 12>), K<32, 13>, K<32, 14>,
-                                        K<32, 15>, K<32, 16> };
+    static const dense_fn by_r[] = { nullptr, K<8, 1>, K<8, 2>, K<8, 3>, K<8, 4>, K<8, 5>, K<8, 6>, K<8, 7>,
+                                     K<16, 8>, K<16, 9>, K<16, 10>, K<16, 11>, K<16, 12>,
+                                     K<32, 13>, K<32, 14>, K<32, 15>, K<32, 16> };
 #undef K
-#undef GFR_ALT
-    const int R = (N + 7) / 8;
-    int tx = N <= 56 ? 8 : N <= 96 ? 16 : 32;
-    if (const char* e = std::getenv("GFR_DENSE_TX")) {
-      const int want = std::atoi(e);
-      const dense_fn alt = want == 8 && R <= 9 ? by_tx8[R] : want == 16 && R <= 12 ? by_tx16[R] : want == 32 ? by_tx32[R] : nullptr;
-      if (alt) tx = want;
-    }
-    fn = tx == 8 ? by_tx8[R] : tx == 16 ? by_tx16[R] : by_tx32[R];
+    const int tx = N <= 56 ? 8 : N <= 96 ? 16 : 32;
+    fn = by_r[(N + 7) / 8];
     threads = 8 * tx;
   }
   GFR_CUDA(cudaFuncSetAttribute((const void*)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, net->smem_optin));
@@ -976,13 +897,8 @@ int gfr_network_solve(const gfr_network* net, int64_t B, const double* p_inj, co
   if (per_sm < 1) return fail(GFR_E_LIMIT, "the dense Jacobian of this network exceeds the shared memory of an SM");
   long long grid = (long long)net->sm_count * per_sm;
   if (grid > B) grid = B;
-  SolOut o{};
-  o.converged = out->converged; o.iterations = out->iterations; o.bus_voltages = out->bus_voltages;
-  o.bus_angles = out->bus_angles; o.line_flows = out->line_flows; o.line_loadings = out->line_loadings;
-  o.losses = out->losses; o.max_mismatch = out->max_mismatch;
-  const double accel = cfg->acceleration != 0.0 ? cfg->acceleration : 1.0;
-  fn<<<(int)grid, threads, smem, (cudaStream_t)stream>>>(net->nd, cfg->tolerance, cfg->max_iterations,
-                                                         accel, p_inj, o, (long long)B);
+  const EnvCfg k = env_cfg_of(cfg);
+  fn<<<(int)grid, threads, smem, (cudaStream_t)stream>>>(net->nd, k.tol, k.max_it, k.accel, p_inj, *out, (long long)B);
   g_launches.fetch_add(1);
   GFR_CUDA(cudaGetLastError());
   return GFR_OK;
@@ -992,7 +908,7 @@ int gfr_noise_fill(int device, int64_t B, int32_t n_slots, const uint64_t* seeds
                    double* out, void* stream) {
   if (B < 1 || n_slots < 1 || !seeds || !draws || !out) return fail(GFR_E_ARG, "bad argument");
   DeviceGuard guard(device);
-  if (!guard.ok) return fail(GFR_E_CUDA, "no usable CUDA device (this library has no CPU fallback)");
+  if (!guard.ok) return no_device();
   long long total = B * (long long)n_slots;
   long long grid = (total + 255) / 256;
   int sms = 148;
@@ -1007,7 +923,7 @@ int gfr_noise_fill(int device, int64_t B, int32_t n_slots, const uint64_t* seeds
 int gfr_fp64_peak(int device, double* tflops) {
   if (!tflops) return fail(GFR_E_ARG, "null argument");
   DeviceGuard guard(device);
-  if (!guard.ok) return fail(GFR_E_CUDA, "no usable CUDA device (this library has no CPU fallback)");
+  if (!guard.ok) return no_device();
   cudaDeviceProp prop;
   GFR_CUDA(cudaGetDeviceProperties(&prop, device));
   const int threads = 256, blocks = prop.multiProcessorCount * 8, iters = 1 << 15;

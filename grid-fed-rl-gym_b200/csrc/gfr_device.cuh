@@ -26,6 +26,8 @@
 #include <math.h>
 #include <stdint.h>
 
+#include "../../include/gfr_b200.h"
+
 #if defined(__CUDACC__)
 #define GFR_HD __host__ __device__ __forceinline__
 #else
@@ -335,8 +337,10 @@ GFR_HD size_t sweep_slot_bytes(int n, int n_src, bool p_local = false, int n_tie
   const size_t units = ((size_t)n * (p_local ? 32 : 40) + 15) / 16 + 2 * (size_t)n_tie;   // 16-byte units, made odd: neighbouring instances'
   return (units | 1) * 16;                                // slots then start 4 banks apart (conflict-free 128-bit accesses)
 }
+// Points a group at its instance slot: `slot` in shared memory, `mg` its global scratch (Newton), `p_local` the
+// thread's own array of SWEEP_P_LOCAL_MAX doubles (sweep, one lane; a caller that passes none points g.pp at its own)
 template <int LANES>
-GFR_HD void bind_slot(NGrp<LANES>& g, unsigned char* slot, const Layout& lay, D2* mg) {
+GFR_HD void bind_slot(NGrp<LANES>& g, unsigned char* slot, const Layout& lay, D2* mg, double* = nullptr) {
   g.np = lay.n_pool;
   g.efp = reinterpret_cast<D2*>(slot);
   g.poolp = g.efp + lay.n;
@@ -345,13 +349,16 @@ GFR_HD void bind_slot(NGrp<LANES>& g, unsigned char* slot, const Layout& lay, D2
   g.pol = scratch_policy();
 }
 template <int LANES>
-GFR_HD void bind_slot(SGrp<LANES>& g, unsigned char* slot, const Layout& lay, D2*) {
+GFR_HD void bind_slot(SGrp<LANES>& g, unsigned char* slot, const Layout& lay, D2*, double* p_local = nullptr) {
   const int n = lay.n;
   g.efp = reinterpret_cast<D2*>(slot);
   g.jrp = g.efp + n;
   g.pp = reinterpret_cast<double*>(g.jrp + n);
   g.jt = g.jrp + n + (sweep_p_local(LANES, n) ? 0 : (n + 1) / 2);      // after the injections, when they live here
   g.n = n;
+  // one thread per instance on a small feeder: the specified injections live in the thread's local array (the host
+  // sized the shared-memory slot without them)
+  if (sweep_p_local(LANES, n)) g.pp = p_local;
 }
 
 
@@ -1245,10 +1252,7 @@ GFR_HD void line_flow(const G& g, const Layout& lay, const int* simg, const doub
 
 // ----------------------------------------------------------------------------- solver entry (gfr_solve)
 
-struct SolOut {
-  uint8_t* converged; int32_t* iterations; double* bus_voltages; double* bus_angles;
-  double* line_flows; double* line_loadings; double* losses; double* max_mismatch;
-};
+typedef gfr_sol_out SolOut;      // the caller's output table, as the C ABI declares it
 
 template <int SOLVER, int LANES>
 GFR_HD void run_solver(const NGrp<LANES>& g, const Layout& lay, const int* simg, const double* dimg,
@@ -1301,12 +1305,7 @@ GFR_HD void solve_instance(const typename GroupOf<LANES, SOLVER>::type& g, const
 
 // ----------------------------------------------------------------------------- environment
 
-struct StepOut {
-  double* reward; uint8_t* terminated; uint8_t* truncated; uint8_t* error; uint8_t* converged;
-  int32_t* iterations; double* max_voltage; double* min_voltage; double* losses;
-  double* max_mismatch; uint8_t* violations; int32_t* violation_count; int32_t* current_step;
-  double* episode_reward; double* noise_used;
-};
+typedef gfr_step_out StepOut;    // the caller's output table, as the C ABI declares it
 
 GFR_HD bool finite_d(double x) { return fabs(x) <= 1.7976931348623157e308; }   // false for NaN / Inf
 

@@ -158,6 +158,24 @@ inline std::string check_feeder_desc(const gfr_feeder_desc* d) {
   return std::string();
 }
 
+// The kernels' settings of a solve: tolerance, iteration cap, Newton's acceleration factor (0 = the reference's 1.0)
+inline EnvCfg env_cfg_of(const gfr_solver_cfg* c) {
+  EnvCfg k{};
+  k.tol = c->tolerance; k.max_it = c->max_iterations;
+  k.accel = c->acceleration != 0.0 ? c->acceleration : 1.0;
+  return k;
+}
+// ... and of an environment step; the sweep leaves the acceleration factor at 1
+inline EnvCfg env_cfg_of(const gfr_env_cfg* c) {
+  EnvCfg k = env_cfg_of(&c->solver);
+  if (c->solver.solver != GFR_SOLVER_NEWTON) k.accel = 1.0;
+  k.dt = c->timestep; k.v_min = c->v_min; k.v_max = c->v_max; k.f_min = c->f_min; k.f_max = c->f_max;
+  k.penalty = c->safety_penalty; k.load_noise = c->load_noise;
+  k.episode_length = c->episode_length; k.stochastic_loads = c->stochastic_loads != 0;
+  k.weather_variation = c->weather_variation != 0;
+  return k;
+}
+
 // The elimination schedule on `lanes` lanes: row and lane of every bus.  The description's levels are
 // the rows and its lane_of the lanes whenever they fit (every level at most `lanes` wide, lanes
 // distinct inside a level); otherwise levels are cut into rows of `lanes` buses in index order.
@@ -204,9 +222,7 @@ inline Schedule make_schedule(const gfr_feeder_desc* d, int lanes) {
 }
 
 // returns an empty string on success, the complaint otherwise
-// flat_start_factors: include the factorisation of the flat-start Jacobian (96 B per position)
-inline std::string build_feeder_image(const gfr_feeder_desc* d, int lanes, int solver, FeederImage* out,
-                                      bool flat_start_factors = true) {
+inline std::string build_feeder_image(const gfr_feeder_desc* d, int lanes, int solver, FeederImage* out) {
   {
     std::string complaint = check_feeder_desc(d);
     if (!complaint.empty()) return complaint;
@@ -523,7 +539,7 @@ inline std::string build_feeder_image(const gfr_feeder_desc* d, int lanes, int s
   // the same leaf -> root block elimination the kernel runs, done once here.
   if (newton) {
     std::vector<double> f0(12 * (size_t)P, 0.0), C(4 * (size_t)n, 0.0);
-    bool ok = flat_start_factors;
+    bool ok = true;
     for (int k = n - 1; k >= 0 && ok; --k) {           // children have larger indices: done before their parent
       const bool th = d->bus_type[k] != GFR_BUS_SLACK, pq = d->bus_type[k] == GFR_BUS_PQ;
       const double vk = pq ? 1.0 : d->vm_set[k];

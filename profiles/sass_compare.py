@@ -2,7 +2,9 @@
 """Compares the machine code of two builds of libgfr_b200.so (no GPU needed): the SASS of every kernel, with addresses
 and encodings stripped, and `cuobjdump -res-usage` (registers, stack, shared / local memory) per kernel.  For each
 kernel whose SASS differs it prints the differing lines and whether the two instruction lists hold the same
-instructions in another order.  usage: python profiles/sass_compare.py OLD.so NEW.so"""
+instructions in another order.  Kernels are matched by their short name with template arguments
+(`step_kernel<8,1,1>`), so a renamed parameter type, which changes every mangled name, still compares kernel by
+kernel.  usage: python profiles/sass_compare.py OLD.so NEW.so"""
 import collections
 import difflib
 import re
@@ -19,13 +21,18 @@ def short(name):
     return m.group(1) + ("<" + ",".join(re.findall(r"L[ib](\d+)E", m.group(2))) + ">" if m.group(2) else "")
 
 
+def key(mangled):
+    return short(ANON.sub("_GLOBAL__N_", mangled))
+
+
 def sass(lib):
     text = subprocess.run(["cuobjdump", "-sass", lib], capture_output=True, text=True, check=True).stdout
     out, cur = {}, None
     for line in text.splitlines():
         m = re.search(r"Function : (\S+)", line)
         if m:
-            cur = ANON.sub("_GLOBAL__N_", m.group(1))
+            cur = key(m.group(1))
+            assert cur not in out, f"two kernels of {lib} share the short name {cur}"
             out[cur] = []
             continue
         m = re.match(r"\s+/\*[0-9a-f]+\*/\s+(.*?)\s*;", line)
@@ -40,7 +47,8 @@ def resources(lib):
     for line in text.splitlines():
         m = re.search(r"Function (\S+):", line)
         if m:
-            cur = ANON.sub("_GLOBAL__N_", m.group(1))
+            cur = key(m.group(1))
+            assert cur not in out, f"two kernels of {lib} share the short name {cur}"
         elif cur and "REG:" in line:
             out[cur] = " ".join(line.split()[:4])
             cur = None
@@ -58,13 +66,13 @@ def main():
           f"{sum(ra[f] != rb.get(f) for f in ra)}")
     for f in differ:
         same = collections.Counter(a[f]) == collections.Counter(b.get(f, []))
-        print(f"\n{short(f)}: {len(a[f])} / {len(b.get(f, []))} instructions, same instructions reordered: {same}")
+        print(f"\n{f}: {len(a[f])} / {len(b.get(f, []))} instructions, same instructions reordered: {same}")
         for line in difflib.unified_diff(a[f], b.get(f, []), lineterm="", n=3):
             if not line.startswith(("---", "+++")):
                 print("   ", line)
     print("\n# resource usage per kernel (old | new)")
-    for f in sorted(ra, key=short):
-        print(f"{short(f):36s} {ra[f]:44s} | {rb.get(f)}")
+    for f in sorted(ra):
+        print(f"{f:36s} {ra[f]:44s} | {rb.get(f)}")
 
 
 if __name__ == "__main__":

@@ -39,15 +39,10 @@ struct EmuSlot {
   explicit EmuSlot(const Layout& lay)
       : work(8 + (newton_slot_bytes(lay.n, lay.n_pool, 0) + sweep_slot_bytes(lay.n, 0, false, lay.n_tie)) / 8, 0.0),
         mg(newton_scratch_doubles(lay.P) / 2 + 1), plocal(SWEEP_P_LOCAL_MAX + 1, 0.0) {}
-  template <int LANES> void local_injections(NGrp<LANES>&, const Layout&) {}
-  template <int LANES> void local_injections(SGrp<LANES>& g, const Layout& lay) {
-    if (sweep_p_local(LANES, lay.n)) g.pp = plocal.data();          // as use_local_injections in gfr_b200.cu
-  }
   template <class G> G group(const Layout& lay, int lane, EmuTeam* team) {
     G g;
     g.lane = lane; g.mask = 1u; g.red = nullptr; g.team = team;
-    bind_slot(g, reinterpret_cast<unsigned char*>(work.data()), lay, mg.data());
-    local_injections(g, lay);
+    bind_slot(g, reinterpret_cast<unsigned char*>(work.data()), lay, mg.data(), plocal.data());
     return g;
   }
 };
@@ -119,18 +114,13 @@ emu_env* emu_create(const gfr_feeder_desc* d, long long B, const gfr_env_cfg* c)
   const Layout& lay = e->fi.lay;
   e->B = B;
   e->solver = c->solver.solver == GFR_SOLVER_NEWTON ? SOLVER_NEWTON : SOLVER_SWEEP;
-  EnvCfg& k = e->cfg;
-  k.dt = c->timestep; k.v_min = c->v_min; k.v_max = c->v_max; k.f_min = c->f_min; k.f_max = c->f_max;
-  k.penalty = c->safety_penalty; k.load_noise = c->load_noise; k.tol = c->solver.tolerance;
-  k.accel = c->solver.acceleration != 0.0 ? c->solver.acceleration : 1.0;
-  k.episode_length = c->episode_length; k.stochastic_loads = c->stochastic_loads != 0;
-  k.weather_variation = c->weather_variation != 0; k.max_it = c->solver.max_iterations;
+  e->cfg = env_cfg_of(c);
   e->state.assign((size_t)B * lay.R, 0.0);
   e->obs.assign((size_t)B * lay.D, 0.0);
   e->bat_soc0.assign(d->bat_soc0, d->bat_soc0 + lay.Bt);
   Lanes<1> g; g.lane = 0; g.mask = 1u;
   for (long long i = 0; i < B; ++i)
-    reset_instance<1>(g, lay, (const int*)e->fi.img.data(), (const double*)e->fi.img.data(), k, i,
+    reset_instance<1>(g, lay, (const int*)e->fi.img.data(), (const double*)e->fi.img.data(), e->cfg, i,
                       e->state.data(), e->obs.data(), 0, e->fi.load_pq.data(), e->bat_soc0.data(),
                       nullptr, nullptr, 0.0, true, (long long)c->env_id_offset);
   return e;
@@ -157,19 +147,12 @@ void emu_reset(emu_env* e, const uint64_t* seeds, const uint8_t* mask, const dou
 }
 
 void emu_step(emu_env* e, const double* actions, const double* noise, const gfr_step_out* out) {
-  StepOut o{};
-  o.reward = out->reward; o.terminated = out->terminated; o.truncated = out->truncated;
-  o.error = out->error; o.converged = out->converged; o.iterations = out->iterations;
-  o.max_voltage = out->max_voltage; o.min_voltage = out->min_voltage; o.losses = out->losses;
-  o.max_mismatch = out->max_mismatch; o.violations = out->violations;
-  o.violation_count = out->violation_count; o.current_step = out->current_step;
-  o.episode_reward = out->episode_reward; o.noise_used = out->noise_used;
   switch (e->lanes) {
-    case 1: step_all<1>(e, actions, noise, o); break;
-    case 2: step_all<2>(e, actions, noise, o); break;
-    case 4: step_all<4>(e, actions, noise, o); break;
-    case 8: step_all<8>(e, actions, noise, o); break;
-    case 16: step_all<16>(e, actions, noise, o); break;
+    case 1: step_all<1>(e, actions, noise, *out); break;
+    case 2: step_all<2>(e, actions, noise, *out); break;
+    case 4: step_all<4>(e, actions, noise, *out); break;
+    case 8: step_all<8>(e, actions, noise, *out); break;
+    case 16: step_all<16>(e, actions, noise, *out); break;
   }
 }
 
@@ -181,18 +164,13 @@ int emu_solve(const gfr_feeder_desc* d, long long B, const double* p_inj, const 
   std::string err = build_feeder_image(d, lanes, c->solver, &fi);
   if (!err.empty()) return -1;
   const int solver = c->solver == GFR_SOLVER_NEWTON ? SOLVER_NEWTON : SOLVER_SWEEP;
-  EnvCfg k{};
-  k.tol = c->tolerance; k.max_it = c->max_iterations; k.accel = c->acceleration != 0.0 ? c->acceleration : 1.0;
-  SolOut o{};
-  o.converged = out->converged; o.iterations = out->iterations; o.bus_voltages = out->bus_voltages;
-  o.bus_angles = out->bus_angles; o.line_flows = out->line_flows; o.line_loadings = out->line_loadings;
-  o.losses = out->losses; o.max_mismatch = out->max_mismatch;
+  const EnvCfg k = env_cfg_of(c);
   switch (lanes) {
-    case 1: solve_all<1>(fi, solver, k, B, p_inj, o); break;
-    case 2: solve_all<2>(fi, solver, k, B, p_inj, o); break;
-    case 4: solve_all<4>(fi, solver, k, B, p_inj, o); break;
-    case 8: solve_all<8>(fi, solver, k, B, p_inj, o); break;
-    case 16: solve_all<16>(fi, solver, k, B, p_inj, o); break;
+    case 1: solve_all<1>(fi, solver, k, B, p_inj, *out); break;
+    case 2: solve_all<2>(fi, solver, k, B, p_inj, *out); break;
+    case 4: solve_all<4>(fi, solver, k, B, p_inj, *out); break;
+    case 8: solve_all<8>(fi, solver, k, B, p_inj, *out); break;
+    case 16: solve_all<16>(fi, solver, k, B, p_inj, *out); break;
   }
   return 0;
 }

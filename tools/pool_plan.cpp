@@ -14,7 +14,7 @@ extern "C" {
 int pool_plan(const gfr_feeder_desc* d, int lanes, int* info, int32_t* sched, int sched_cap, int32_t* tails,
               int tails_cap, char* err, int err_cap) {
   gfr::FeederImage fi;
-  const std::string complaint = gfr::build_feeder_image(d, lanes, GFR_SOLVER_NEWTON, &fi, false);
+  const std::string complaint = gfr::build_feeder_image(d, lanes, GFR_SOLVER_NEWTON, &fi);
   if (!complaint.empty()) {
     if (err && err_cap > 0) std::snprintf(err, (size_t)err_cap, "%s", complaint.c_str());
     return -1;
