@@ -246,7 +246,6 @@ int no_device() { return fail(GFR_E_CUDA, "no usable CUDA device (this library h
 struct ImageDev {
   Layout lay{};
   void* d_img = nullptr;
-  int n_reg_edges = 0;
 };
 
 struct gfr_feeder {
@@ -256,7 +255,6 @@ struct gfr_feeder {
   int smem_per_sm = 0;
   Layout lay{};                  // sizes only (n, L, G, Bt, A, D, R, ...): offsets belong to an image
   bool has_pv = false;
-  bool root_is_slack = true;
   int lanes_hint = 0;            // lane count the level schedule was capped for (0: not said)
   int center_depth = 0;          // levels of the tree rooted at its center, uncapped
   DescCopy desc;                 // the description, kept to build further images
@@ -307,7 +305,6 @@ int image_for(const gfr_feeder* f, int solver, int lanes, const ImageDev** out) 
   if (!complaint.empty()) return fail(GFR_E_ARG, complaint);
   ImageDev dev;
   dev.lay = fi.lay;
-  dev.n_reg_edges = fi.n_reg_edges;
   GFR_CUDA(cudaMalloc(&dev.d_img, fi.img.size()));
   cudaError_t ce = cudaMemcpy(dev.d_img, fi.img.data(), fi.img.size(), cudaMemcpyHostToDevice);
   if (ce != cudaSuccess) { cudaFree(dev.d_img); return cuda_fail(ce, "cudaMemcpy(image)"); }
@@ -557,7 +554,6 @@ int gfr_feeder_create(const gfr_feeder_desc* d, int device, gfr_feeder** out) {
   f->smem_per_sm = (int)prop.sharedMemPerMultiprocessor;
   f->lay = fi.lay;
   f->has_pv = fi.has_pv;
-  f->root_is_slack = fi.root_is_slack;
   f->lanes_hint = d->lanes_hint;
   f->center_depth = fi.center_depth;
   f->desc.assign(d);

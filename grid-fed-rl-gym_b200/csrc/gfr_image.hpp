@@ -7,6 +7,10 @@
 // and diagonal admittances, the flat-start factors.  A lane therefore reads consecutive 16-byte units
 // next to its neighbours', with no index chain (the position is known before anything is loaded).
 // The sweep keeps its compact per-bus arrays (position = bus index there).
+//
+// build_feeder_image runs, in order: the description check, the sizes, the schedule (make_schedule), the bus
+// flags, the Newton plan of the hand-offs (plan_newton), the int arrays, then the double arrays with the
+// flat-start factors (flat_start_factors).
 #pragma once
 #include <algorithm>
 #include <cstring>
@@ -38,9 +42,7 @@ struct ImageBuilder {
 struct FeederImage {
   Layout lay{};
   bool has_pv = false;
-  bool root_is_slack = false;
   int center_depth = 0;            // levels of the tree rooted at its center (ceil(diameter / 2) + 1), uncapped
-  int lanes = 0, solver = 0;
   int n_reg_edges = 0;             // branches whose hand-off stays in registers (Newton)
   std::vector<unsigned char> img;
   std::vector<double> load_pq;     // [2L] static active / reactive power (observation)
@@ -221,8 +223,200 @@ inline Schedule make_schedule(const gfr_feeder_desc* d, int lanes) {
   return s;
 }
 
+// Slots handed out lowest free first: a released slot is taken again before a new one is opened.
+struct SlotPool {
+  std::vector<int> free_slots;
+  int n = 0;                                       // slots opened
+  int take() {
+    if (free_slots.empty()) return n++;
+    auto it = std::min_element(free_slots.begin(), free_slots.end());
+    const int s = *it;
+    free_slots.erase(it);
+    return s;
+  }
+};
+
+// entries 0 .. keys.size() - 1 grouped by key, as ptr[n_keys + 1] / idx: a counting sort, so the entries of one key
+// keep their order
+inline void group_by_key(const std::vector<int32_t>& keys, int n_keys, std::vector<int32_t>& ptr, std::vector<int32_t>& idx) {
+  ptr.assign(n_keys + 1, 0);
+  for (int key : keys) ptr[key + 1]++;
+  for (int k = 0; k < n_keys; ++k) ptr[k + 1] += ptr[k];
+  std::vector<int32_t> fill(ptr.begin(), ptr.end() - 1);
+  idx.resize(keys.size());
+  for (size_t i = 0; i < keys.size(); ++i) idx[fill[keys[i]]++] = (int32_t)i;
+}
+
+// How every bus hands its Schur terms to its parent and gets its correction back (Newton).  The defaults (no heir,
+// no chain, slot 0, no correction slot) are what the sweep's records carry.
+struct NewtonPlan {
+  std::vector<int> heir, absorb;           // per bus: the child that hands over in registers; the sibling whose partial it absorbs
+  std::vector<std::vector<int>> tails;     // per bus: the chain tails it gathers, in summation order
+  std::vector<int32_t> pool_slot, x_slot;  // per bus: the slot of its hand-off; the slot its parent's correction arrives in
+  std::vector<int32_t> kids_x_slot;        // per bus: the slot it writes its correction into for its pool children (-1: none)
+  int n_pool = 1, n_reg_edges = 0;
+  std::string complaint;                   // not empty: the plan does not fit the record formats
+  explicit NewtonPlan(int n) : heir(n, -1), absorb(n, -1), tails(n), pool_slot(n, 0), x_slot(n, 0), kids_x_slot(n, -1) {}
+};
+
+// The Newton plan on schedule `sch`; marks the register hand-offs in `flags` (FL_C_REG, FL_P_REG)
+inline NewtonPlan plan_newton(const gfr_feeder_desc* d, const Schedule& sch, int lanes, std::vector<int32_t>& flags) {
+  const int n = d->n_bus;
+  NewtonPlan pl(n);
+  // ---- register hand-off: a bus eliminated right after one of its children on the same lane takes that child's
+  //      Schur terms from registers, and hands its correction back the same way
+  for (int k = 1; k < n; ++k) {
+    const int p = d->parent[k];
+    if (sch.row[k] == sch.row[p] + 1 && sch.lane[k] == sch.lane[p] && pl.heir[p] < 0) {
+      pl.heir[p] = k;
+      flags[p] |= FL_C_REG;
+      flags[k] |= FL_P_REG;
+      ++pl.n_reg_edges;
+    }
+  }
+  flags[0] |= FL_P_REG;               // the root has no parent: its "correction from above" is the zero its lane starts with
+  // ---- sibling chains: the children handed over through shared memory ("pool children") are summed along chains
+  //      instead of by their parent alone.  Taken in elimination order (rows nrows-1 .. 0), each pool child ABSORBS
+  //      the partial sum of one sibling eliminated in a strictly earlier row - it adds that sibling's slot to its own
+  //      hand-off and writes the sum into its own slot - and the heir absorbs one more into the hand-off it passes in
+  //      registers.  Siblings of one row run in parallel and cannot chain; each starts or continues its own chain.
+  //      The parent gathers only the chain TAILS nobody absorbed: at most as many as it has pool children in one
+  //      row, instead of all of them on one lane.
+  //      Groups of fewer than CHAIN_MIN_LANES lanes run without chains: every pool child is a tail of its own.
+  std::vector<int> reader_row(n, -1);                      // the row a bus's slot is read in
+  std::vector<int> kids;
+  for (int k = 0; k < n; ++k) {
+    kids.clear();
+    for (int q = d->child_ptr[k]; q < d->child_ptr[k + 1]; ++q)
+      if (d->child_idx[q] != pl.heir[k]) kids.push_back(d->child_idx[q]);
+    std::vector<int>& open = pl.tails[k];                  // chain tails so far, oldest first
+    if (lanes < CHAIN_MIN_LANES) {
+      open = kids;
+      for (int c : kids) reader_row[c] = sch.row[k];
+      continue;
+    }
+    std::stable_sort(kids.begin(), kids.end(), [&](int a, int b) { return sch.row[a] > sch.row[b]; });
+    for (size_t i = 0; i < kids.size();) {
+      const int r = sch.row[kids[i]];
+      size_t j = i;
+      size_t avail = open.size();                          // tails of earlier rows: the ones open before this row
+      std::vector<int> started;
+      for (; j < kids.size() && sch.row[kids[j]] == r; ++j) {
+        const int c = kids[j];
+        if (avail > 0) {
+          pl.absorb[c] = open.front();
+          reader_row[open.front()] = r;
+          open.erase(open.begin());
+          --avail;
+        }
+        started.push_back(c);
+      }
+      open.insert(open.end(), started.begin(), started.end());
+      i = j;
+    }
+    // the heir (row of k + 1, the last row before k's) absorbs the oldest tail unless that one shares its row
+    const int h = pl.heir[k];
+    if (h >= 0 && !open.empty() && sch.row[open.front()] > sch.row[h]) {
+      pl.absorb[h] = open.front();
+      reader_row[open.front()] = sch.row[h];
+      open.erase(open.begin());
+    }
+    for (int c : open) reader_row[c] = sch.row[k];
+  }
+  // ---- pool plan: a slot for every bus whose hand-off goes through shared memory, held from its own row up to the
+  //      row that reads it (the next link of its chain, or its parent).  Slots are handed out row by row; a slot read
+  //      (released) in one row is reused by LATER rows only, so the group barrier that ends a row orders every read
+  //      before the next write.
+  std::vector<std::vector<int>> by_row(sch.nrows), read_in(sch.nrows);
+  for (int k = 0; k < n; ++k) {
+    by_row[sch.row[k]].push_back(k);
+    if (reader_row[k] >= 0) read_in[reader_row[k]].push_back(k);
+  }
+  SlotPool pool;
+  for (int r = sch.nrows - 1; r >= 0; --r) {
+    for (int k : by_row[r])
+      if (!(flags[k] & FL_P_REG)) pl.pool_slot[k] = pool.take();   // (not handed over in registers, not the root)
+    for (int k : read_in[r]) pool.free_slots.push_back(pl.pool_slot[k]);
+  }
+  // ---- correction plan (back-substitution, root -> leaf): a bus with pool children writes its correction once, into
+  //      a slot every such child reads in its own row.  The slot is held from the parent's row to the last of those
+  //      children's rows, and reused from the row after that on.  This pass writes nothing else into the pool, and
+  //      group barriers separate it from the leaf -> root passes.
+  std::vector<int> last_read(n, -1);
+  for (int k = 1; k < n; ++k)
+    if (k != pl.heir[d->parent[k]]) last_read[d->parent[k]] = std::max(last_read[d->parent[k]], sch.row[k]);
+  std::vector<std::vector<int>> freed_after(sch.nrows);
+  for (int k = 0; k < n; ++k)
+    if (last_read[k] >= 0) freed_after[last_read[k]].push_back(k);
+  SlotPool xpool;
+  for (int r = 0; r < sch.nrows; ++r) {
+    if (r > 0)
+      for (int k : freed_after[r - 1]) xpool.free_slots.push_back(pl.kids_x_slot[k]);
+    for (int k : by_row[r])
+      if (last_read[k] >= 0) pl.kids_x_slot[k] = xpool.take();
+  }
+  for (int k = 1; k < n; ++k)
+    if (k != pl.heir[d->parent[k]]) pl.x_slot[k] = pl.kids_x_slot[d->parent[k]];
+  pl.n_pool = std::max({pool.n, 1, xpool.n, d->n_pool});    // d->n_pool: the caller asks for more (padding experiments)
+  if (pl.n_pool > FL_POOL_MASK) pl.complaint = "more than 4095 pool slots";
+  return pl;
+}
+
+// Factorisation of the flat-start Jacobian (the first Newton iteration of every instance): the same leaf -> root
+// block elimination the kernel runs, done once here.  12 * P doubles, or none when the matrix is singular at the
+// flat start.
+inline std::vector<double> flat_start_factors(const gfr_feeder_desc* d, const std::vector<int>& pos, int P) {
+  const int n = d->n_bus;
+  std::vector<double> f0(12 * (size_t)P, 0.0), C(4 * (size_t)n, 0.0);
+  auto vm = [&](int j) { return d->bus_type[j] == GFR_BUS_PQ ? 1.0 : d->vm_set[j]; };
+  for (int k = n - 1; k >= 0; --k) {                 // children have larger indices: done before their parent
+    const bool th = d->bus_type[k] != GFR_BUS_SLACK, pq = d->bus_type[k] == GFR_BUS_PQ;
+    const double vk = vm(k);
+    const double v2 = vk * vk;
+    double Pc = d->gdiag[k] * v2, Qc = -d->bdiag[k] * v2;
+    if (k > 0) { const double a = vk * vm(d->parent[k]); Pc += -d->g[k] * a; Qc += d->b[k] * a; }
+    for (int q = d->child_ptr[k]; q < d->child_ptr[k + 1]; ++q) {
+      const int c = d->child_idx[q];
+      const double a = vk * vm(c);
+      Pc += -d->g[c] * a; Qc += d->b[c] * a;
+    }
+    double d00 = -Qc - d->bdiag[k] * v2, d01 = Pc + d->gdiag[k] * v2, d10 = Pc - d->gdiag[k] * v2,
+           d11 = Qc - d->bdiag[k] * v2;
+    for (int q = d->child_ptr[k]; q < d->child_ptr[k + 1]; ++q) {
+      const double* cc = &C[4 * (size_t)d->child_idx[q]];
+      d00 -= cc[0]; d01 -= cc[1]; d10 -= cc[2]; d11 -= cc[3];
+    }
+    const double a = k > 0 ? vk * vm(d->parent[k]) : 0.0;
+    const double gk = k > 0 ? d->g[k] : 0.0, bk = k > 0 ? d->b[k] : 0.0;
+    const double ga = -gk * a, al = bk * a, gl = -gk * a, ll = bk * a;      // sin = 0 at a flat start
+    double u00 = al, u01 = ga, u10 = -ga, u11 = al;
+    if (!th) { d00 = 1.0; d01 = 0.0; u00 = u01 = 0.0; }
+    if (!pq) { d10 = 0.0; d11 = 1.0; u10 = u11 = 0.0; }
+    const double det = d00 * d11 - d01 * d10;
+    if (det == 0.0 || !(det == det)) return {};
+    const double inv = 1.0 / det;
+    const double i00 = d11 * inv, i01 = -d01 * inv, i10 = -d10 * inv, i11 = d00 * inv;
+    const double m00 = i00 * u00 + i01 * u10, m01 = i00 * u01 + i01 * u11,
+                 m10 = i10 * u00 + i11 * u10, m11 = i10 * u01 + i11 * u11;
+    // six 16-byte fields per position, field-major (field f of position p at f0[2 * (f * P + p)]): the lanes
+    // of a row read consecutive 16-byte units
+    const int p = pos[k];
+    auto put = [&](int fld, double a0, double a1) {
+      f0[2 * ((size_t)fld * P + p)] = a0; f0[2 * ((size_t)fld * P + p) + 1] = a1;
+    };
+    put(0, i00, i01); put(1, i10, i11);
+    put(2, m00, m01); put(3, m10, m11);
+    put(4, ll, gl);
+    put(5, Pc, Qc);                                  // calculated injections of the flat profile
+    double* cc = &C[4 * (size_t)k];
+    cc[0] = ll * m00 + gl * m10; cc[1] = ll * m01 + gl * m11;
+    cc[2] = -gl * m00 + ll * m10; cc[3] = -gl * m01 + ll * m11;
+  }
+  return f0;
+}
+
 // returns an empty string on success, the complaint otherwise
-inline std::string build_feeder_image(const gfr_feeder_desc* d, int lanes, int solver, FeederImage* out) {
+inline std::string build_feeder_image(const gfr_feeder_desc* d, int lanes, int solver, FeederImage* f) {
   {
     std::string complaint = check_feeder_desc(d);
     if (!complaint.empty()) return complaint;
@@ -233,8 +427,7 @@ inline std::string build_feeder_image(const gfr_feeder_desc* d, int lanes, int s
   if (newton && nt)
     return "the feeder has loop-closing lines: the tree-ordered Newton-Raphson takes radial feeders "
            "(GFR_SOLVER_SWEEP restores the loops by compensation)";
-  FeederImage* f = out;
-  f->lanes = lanes; f->solver = solver; f->n_reg_edges = 0; f->has_pv = false;
+  f->has_pv = false;
   {
     // depth of the tree rooted at its center: the longest path (in edges) is found leaf -> root from the two
     // deepest subtrees of every bus (children come after their parent in level order)
@@ -258,20 +451,13 @@ inline std::string build_feeder_image(const gfr_feeder_desc* d, int lanes, int s
   for (int l = 0; l < L; ++l) lp = lp + d->load_p[l];   // sequential, as grid_env.py:744
   lay.load_p_sum = lp;
 
-  // ---- schedule positions: Newton = (row, lane); sweep = the bus index itself
-  Schedule sch;
+  // ---- schedule positions: Newton = (row, lane); sweep = the bus index itself (its multi-lane records use the rows)
+  const Schedule sch = make_schedule(d, lanes);
   std::vector<int> pos(n);
-  if (newton) {
-    sch = make_schedule(d, lanes);
-    for (int k = 0; k < n; ++k) pos[k] = sch.row[k] * lanes + sch.lane[k];
-    lay.nrows = sch.nrows;
-    lay.P = sch.nrows * lanes;
-    if (lay.P > 65535) return "more than 65535 schedule positions";
-  } else {
-    for (int k = 0; k < n; ++k) pos[k] = k;
-    lay.nrows = nl;
-    lay.P = n;
-  }
+  for (int k = 0; k < n; ++k) pos[k] = newton ? sch.row[k] * lanes + sch.lane[k] : k;
+  lay.nrows = newton ? sch.nrows : nl;
+  lay.P = newton ? sch.nrows * lanes : n;
+  if (lay.P > 65535) return "more than 65535 schedule positions";
   const int P = lay.P;
   std::vector<int> bus_at(P, -1);
   for (int k = 0; k < n; ++k) bus_at[pos[k]] = k;
@@ -297,173 +483,41 @@ inline std::string build_feeder_image(const gfr_feeder_desc* d, int lanes, int s
     lay.k_slack = ks;
     for (int k = ks; k > 0; k = d->parent[k]) flags[k] |= FL_SLACK_PATH;
   }
-  // ---- register hand-off (Newton): a bus eliminated right after one of its children on the same lane
-  //      takes that child's Schur terms from registers, and hands its correction back the same way
-  std::vector<int> heir(n, -1);
-  if (newton) {
-    for (int k = 1; k < n; ++k) {
-      const int p = d->parent[k];
-      if (sch.row[k] == sch.row[p] + 1 && sch.lane[k] == sch.lane[p] && heir[p] < 0) {
-        heir[p] = k;
-        flags[p] |= FL_C_REG;
-        flags[k] |= FL_P_REG;
-        ++f->n_reg_edges;
-      }
-    }
-    flags[0] |= FL_P_REG;               // the root has no parent: its "correction from above" is the zero its lane starts with
-  }
-  // ---- sibling chains (Newton): the children handed over through shared memory ("pool children") are summed
-  //      along chains instead of by their parent alone.  Taken in elimination order (rows nrows-1 .. 0), each
-  //      pool child ABSORBS the partial sum of one sibling eliminated in a strictly earlier row - it adds that
-  //      sibling's slot to its own hand-off and writes the sum into its own slot - and the heir absorbs one more
-  //      into the hand-off it passes in registers.  Siblings of one row run in parallel and cannot chain; each
-  //      starts or continues its own chain.  The parent gathers only the chain TAILS nobody absorbed: at most as
-  //      many as it has pool children in one row, instead of all of them on one lane.
-  //      Groups of fewer than CHAIN_MIN_LANES lanes run without chains: every pool child is a tail of its own.
-  std::vector<int> absorb(n, -1), reader_row(n, -1);       // the sibling whose partial a bus absorbs; row its slot is read in
-  std::vector<std::vector<int>> tails(n);                  // per bus: the chain tails it gathers, in summation order
-  if (newton) {
-    std::vector<int> kids;
-    for (int k = 0; k < n; ++k) {
-      kids.clear();
-      for (int q = d->child_ptr[k]; q < d->child_ptr[k + 1]; ++q)
-        if (d->child_idx[q] != heir[k]) kids.push_back(d->child_idx[q]);
-      if (lanes < CHAIN_MIN_LANES) {
-        tails[k] = kids;
-        for (int c : kids) reader_row[c] = sch.row[k];
-        continue;
-      }
-      std::stable_sort(kids.begin(), kids.end(), [&](int a, int b) { return sch.row[a] > sch.row[b]; });
-      std::vector<int>& open = tails[k];                   // chain tails so far, oldest first
-      for (size_t i = 0; i < kids.size();) {
-        const int r = sch.row[kids[i]];
-        size_t j = i;
-        size_t avail = open.size();                        // tails of earlier rows: the ones open before this row
-        std::vector<int> started;
-        for (; j < kids.size() && sch.row[kids[j]] == r; ++j) {
-          const int c = kids[j];
-          if (avail > 0) {
-            absorb[c] = open.front();
-            reader_row[open.front()] = r;
-            open.erase(open.begin());
-            --avail;
-          }
-          started.push_back(c);
-        }
-        open.insert(open.end(), started.begin(), started.end());
-        i = j;
-      }
-      // the heir (row of k + 1, the last row before k's) absorbs the oldest tail unless that one shares its row
-      if (heir[k] >= 0 && !open.empty() && sch.row[open.front()] > sch.row[heir[k]]) {
-        absorb[heir[k]] = open.front();
-        reader_row[open.front()] = sch.row[heir[k]];
-        open.erase(open.begin());
-      }
-      for (int c : open) reader_row[c] = sch.row[k];
-    }
-  }
-  // ---- pool plan (Newton): a slot for every bus whose hand-off goes through shared memory, held from its own
-  //      row up to the row that reads it (the next link of its chain, or its parent).  Slots are handed out row by
-  //      row; a slot read (released) in one row is reused by LATER rows only, so the group barrier that ends a row
-  //      orders every read before the next write.
-  std::vector<int32_t> pool_slot(n, 0);
-  lay.n_pool = 1;
-  if (newton) {
-    std::vector<std::vector<int>> by_row(sch.nrows), read_in(sch.nrows);
-    for (int k = 0; k < n; ++k) {
-      by_row[sch.row[k]].push_back(k);
-      if (reader_row[k] >= 0) read_in[reader_row[k]].push_back(k);
-    }
-    std::vector<int> free_slots;
-    int np = 0;
-    for (int r = sch.nrows - 1; r >= 0; --r) {
-      for (int k : by_row[r]) {
-        if (flags[k] & FL_P_REG) continue;            // handed over in registers (or the root)
-        if (!free_slots.empty()) {
-          auto it = std::min_element(free_slots.begin(), free_slots.end());
-          pool_slot[k] = *it;
-          free_slots.erase(it);
-        } else {
-          pool_slot[k] = np++;
-        }
-      }
-      for (int k : read_in[r]) free_slots.push_back(pool_slot[k]);
-    }
-    lay.n_pool = std::max(np, 1);
-  }
-  // ---- correction plan (Newton, back-substitution, root -> leaf): a bus with pool children writes its correction
-  //      once, into a slot every such child reads in its own row.  The slot is held from the parent's row to the
-  //      last of those children's rows, and reused from the row after that on.  This pass writes nothing else
-  //      into the pool, and group barriers separate it from the leaf -> root passes.
-  std::vector<int32_t> kids_x_slot(n, -1), x_slot(n, 0);
-  if (newton) {
-    std::vector<int> last_read(n, -1);
-    for (int k = 1; k < n; ++k)
-      if (k != heir[d->parent[k]]) last_read[d->parent[k]] = std::max(last_read[d->parent[k]], sch.row[k]);
-    std::vector<std::vector<int>> by_row(sch.nrows), freed_after(sch.nrows);
-    for (int k = 0; k < n; ++k)
-      if (last_read[k] >= 0) { by_row[sch.row[k]].push_back(k); freed_after[last_read[k]].push_back(k); }
-    std::vector<int> free_slots;
-    int np = 0;
-    for (int r = 0; r < sch.nrows; ++r) {
-      if (r > 0)
-        for (int k : freed_after[r - 1]) free_slots.push_back(kids_x_slot[k]);
-      for (int k : by_row[r]) {
-        if (!free_slots.empty()) {
-          auto it = std::min_element(free_slots.begin(), free_slots.end());
-          kids_x_slot[k] = *it;
-          free_slots.erase(it);
-        } else {
-          kids_x_slot[k] = np++;
-        }
-      }
-    }
-    for (int k = 1; k < n; ++k)
-      if (k != heir[d->parent[k]]) x_slot[k] = kids_x_slot[d->parent[k]];
-    lay.n_pool = std::max(lay.n_pool, np);
-    if (d->n_pool > lay.n_pool) lay.n_pool = d->n_pool;      // the caller asks for more (padding experiments)
-    if (lay.n_pool > FL_POOL_MASK) return "more than 4095 pool slots";
-  }
+  const NewtonPlan pl = newton ? plan_newton(d, sch, lanes, flags) : NewtonPlan(n);
+  if (!pl.complaint.empty()) return pl.complaint;
+  lay.n_pool = pl.n_pool;
+  f->n_reg_edges = pl.n_reg_edges;
 
   ImageBuilder ib;
   // ---- per-position records + tail lists (the slots of the chain tails a bus gathers, in the order every pass
-  //      sums them in: after the heir's hand-off)
-  std::vector<int32_t> sched(4 * (size_t)P, 0), child_slot;
-  std::vector<int32_t> topo(4 * (size_t)n);
+  //      sums them in: after the heir's hand-off); CTA-wide groups read the first 8 of every position's tail slots
+  //      from `kids` instead, 16 bits each, in list order
+  std::vector<int32_t> sched(4 * (size_t)P, 0), kids(4 * (size_t)P, 0), child_slot;
   for (int p = 0; p < P; ++p) {
     const int k = bus_at[p];
     if (k < 0) continue;
     const int kp = k > 0 ? d->parent[k] : 0;
     const int begin = (int)child_slot.size();
-    for (int c : tails[k]) child_slot.push_back(pool_slot[c]);
-    const int n_tails = (int)tails[k].size();
+    const std::vector<int>& tails = pl.tails[k];
+    for (size_t j = 0; j < tails.size(); ++j) {
+      child_slot.push_back(pl.pool_slot[tails[j]]);
+      if (j < 8) kids[4 * p + j / 2] |= pl.pool_slot[tails[j]] << (16 * (j & 1));
+    }
+    const int n_tails = (int)tails.size();
     if (n_tails > 65535) return "more than 65535 chain tails on one bus";
     sched[4 * p + 0] = (int32_t)((uint32_t)k | ((uint32_t)kp << 16));
     if (begin > REC_LIST_MASK) return "child lists too long";
-    sched[4 * p + 1] = (int32_t)((uint32_t)begin | ((uint32_t)(kids_x_slot[k] + 1) << REC_KIDX_SHIFT));
-    sched[4 * p + 2] = (int32_t)((uint32_t)flags[k] | ((uint32_t)pool_slot[k] << FL_POOL_SHIFT) | ((uint32_t)x_slot[k] << FL_XSLOT_SHIFT));
-    sched[4 * p + 3] = (int32_t)((uint32_t)n_tails | ((uint32_t)(absorb[k] >= 0 ? pool_slot[absorb[k]] + 1 : 0) << 16));
-  }
-  for (int k = 0; k < n; ++k) {
-    topo[4 * k + 0] = k > 0 ? d->parent[k] : 0;
-    topo[4 * k + 1] = d->child_ptr[k];
-    topo[4 * k + 2] = d->child_ptr[k + 1];
-    topo[4 * k + 3] = flags[k];
+    sched[4 * p + 1] = (int32_t)((uint32_t)begin | ((uint32_t)(pl.kids_x_slot[k] + 1) << REC_KIDX_SHIFT));
+    sched[4 * p + 2] = (int32_t)((uint32_t)flags[k] | ((uint32_t)pl.pool_slot[k] << FL_POOL_SHIFT) | ((uint32_t)pl.x_slot[k] << FL_XSLOT_SHIFT));
+    sched[4 * p + 3] = (int32_t)((uint32_t)n_tails | ((uint32_t)(pl.absorb[k] >= 0 ? pl.pool_slot[pl.absorb[k]] + 1 : 0) << 16));
   }
   lay.o_sched = ib.add_i(sched.data(), 4 * P);
   // injection sources per POSITION: loads, then generators, then batteries (reference accumulation order)
-  std::vector<int32_t> inj_ptr(P + 1, 0), inj_idx(lay.n_src);
-  {
-    std::vector<int> cnt(P, 0);
-    for (int l = 0; l < L; ++l) cnt[pos[d->load_bus[l]]]++;
-    for (int g = 0; g < G; ++g) cnt[pos[d->gen_bus[g]]]++;
-    for (int b = 0; b < Bt; ++b) cnt[pos[d->bat_bus[b]]]++;
-    for (int p = 0; p < P; ++p) inj_ptr[p + 1] = inj_ptr[p] + cnt[p];
-    std::vector<int> fill(inj_ptr.begin(), inj_ptr.end() - 1);
-    for (int l = 0; l < L; ++l) inj_idx[fill[pos[d->load_bus[l]]]++] = l;
-    for (int g = 0; g < G; ++g) inj_idx[fill[pos[d->gen_bus[g]]]++] = L + g;
-    for (int b = 0; b < Bt; ++b) inj_idx[fill[pos[d->bat_bus[b]]]++] = L + G + b;
-  }
+  std::vector<int32_t> src_pos, inj_ptr, inj_idx;
+  for (int l = 0; l < L; ++l) src_pos.push_back(pos[d->load_bus[l]]);
+  for (int g = 0; g < G; ++g) src_pos.push_back(pos[d->gen_bus[g]]);
+  for (int b = 0; b < Bt; ++b) src_pos.push_back(pos[d->bat_bus[b]]);
+  group_by_key(src_pos, P, inj_ptr, inj_idx);
   lay.o_rank = ib.add_i(rank.data(), n);
   lay.o_rankp = newton ? ib.add_i(rankp.data(), n) : lay.o_rank;
   lay.o_branch_of_line = ib.add_i(bol.data(), lay.m);
@@ -475,46 +529,37 @@ inline std::string build_feeder_image(const gfr_feeder_desc* d, int lanes, int s
   lay.o_rowrec = -1; lay.sw_rows = 0;
   if (newton) {
     lay.o_child_slot = ib.add_i(child_slot.data(), (int)child_slot.size());
-    if (lanes >= GFR_WIDE_GROUP_MIN_LANES) {
-      // CTA-wide groups: the first 8 chain tails' slots of every position, 16 bits each, in list order
-      std::vector<int32_t> kids(4 * (size_t)P, 0);
-      for (int p = 0; p < P; ++p) {
-        const uint32_t begin = (uint32_t)sched[4 * p + 1] & (uint32_t)REC_LIST_MASK;
-        const uint32_t nt = (uint32_t)sched[4 * p + 3] & 0xffffu;
-        for (uint32_t j = 0; j < nt && j < 8; ++j) {
-          const uint32_t slot = (uint32_t)child_slot[begin + j];
-          kids[4 * p + (j >> 1)] = (int32_t)((uint32_t)kids[4 * p + (j >> 1)] | (slot << (16 * (j & 1))));
-        }
-      }
-      lay.o_kids = ib.add_i(kids.data(), 4 * P);
-    }
+    if (lanes >= GFR_WIDE_GROUP_MIN_LANES) lay.o_kids = ib.add_i(kids.data(), 4 * P);
   } else {
+    std::vector<int32_t> topo(4 * (size_t)n);
+    for (int k = 0; k < n; ++k) {
+      topo[4 * k + 0] = k > 0 ? d->parent[k] : 0;
+      topo[4 * k + 1] = d->child_ptr[k];
+      topo[4 * k + 2] = d->child_ptr[k + 1];
+      topo[4 * k + 3] = flags[k];
+    }
     lay.o_topo = ib.add_i(topo.data(), 4 * n);
     lay.o_child_idx = ib.add_i(d->child_idx, n - 1);
     if (lanes > 1) {
       // several lanes: the levels cut into rows of at most `lanes` buses, one record per (row, lane)
-      const Schedule sw = make_schedule(d, lanes);
-      std::vector<int32_t> rowrec(4 * (size_t)sw.nrows * lanes, 0);
+      std::vector<int32_t> rowrec(4 * (size_t)sch.nrows * lanes, 0);
       for (int k = 0; k < n; ++k) {
-        int32_t* r = &rowrec[4 * ((size_t)sw.row[k] * lanes + sw.lane[k])];
+        int32_t* r = &rowrec[4 * ((size_t)sch.row[k] * lanes + sch.lane[k])];
         r[0] = (int32_t)((uint32_t)k | ((uint32_t)(k > 0 ? d->parent[k] : 0) << 16));
         r[1] = d->child_ptr[k];
         r[2] = d->child_ptr[k + 1];
         r[3] = flags[k];
       }
-      lay.sw_rows = sw.nrows;
+      lay.sw_rows = sch.nrows;
       lay.o_rowrec = ib.add_i(rowrec.data(), (int)rowrec.size());
     }
   }
   lay.o_tie_ends = lay.o_tie_ptr = lay.o_tie_inc = lay.o_tie_y = lay.o_tie_z = lay.o_tie_rating = lay.o_tie_zinv = -1;
   if (nt) {
     // tie ends (from, to) as ef indices, and per bus the ties that meet it: entry = tie << 1 | (1 if the bus is the to-end)
-    std::vector<int32_t> ends(2 * (size_t)nt), tptr(n + 1, 0), tinc(2 * (size_t)nt);
-    std::vector<int> cnt(n, 0);
-    for (int i = 0; i < nt; ++i) { ends[2 * i] = d->tie_from[i]; ends[2 * i + 1] = d->tie_to[i]; cnt[d->tie_from[i]]++; cnt[d->tie_to[i]]++; }
-    for (int k = 0; k < n; ++k) tptr[k + 1] = tptr[k] + cnt[k];
-    std::vector<int> fill(tptr.begin(), tptr.end() - 1);
-    for (int i = 0; i < nt; ++i) { tinc[fill[d->tie_from[i]]++] = i << 1; tinc[fill[d->tie_to[i]]++] = (i << 1) | 1; }
+    std::vector<int32_t> ends(2 * (size_t)nt), tptr, tinc;
+    for (int i = 0; i < nt; ++i) { ends[2 * i] = d->tie_from[i]; ends[2 * i + 1] = d->tie_to[i]; }
+    group_by_key(ends, n, tptr, tinc);
     lay.o_tie_ends = ib.add_i(ends.data(), 2 * nt);
     lay.o_tie_ptr = ib.add_i(tptr.data(), n + 1);
     lay.o_tie_inc = ib.add_i(tinc.data(), 2 * nt);
@@ -535,56 +580,9 @@ inline std::string build_feeder_image(const gfr_feeder_desc* d, int lanes, int s
   lay.o_gbd = lay.o_rx = lay.o_f0 = -1;
   if (newton) lay.o_gbd = dbase + ib.add_d(gbd.data(), 2 * P);
   else lay.o_rx = dbase + ib.add_d(rx.data(), 2 * P);
-  // Factorisation of the flat-start Jacobian (the first Newton iteration of every instance):
-  // the same leaf -> root block elimination the kernel runs, done once here.
   if (newton) {
-    std::vector<double> f0(12 * (size_t)P, 0.0), C(4 * (size_t)n, 0.0);
-    bool ok = true;
-    for (int k = n - 1; k >= 0 && ok; --k) {           // children have larger indices: done before their parent
-      const bool th = d->bus_type[k] != GFR_BUS_SLACK, pq = d->bus_type[k] == GFR_BUS_PQ;
-      const double vk = pq ? 1.0 : d->vm_set[k];
-      auto vm = [&](int j) { return d->bus_type[j] == GFR_BUS_PQ ? 1.0 : d->vm_set[j]; };
-      const double v2 = vk * vk;
-      double Pc = d->gdiag[k] * v2, Qc = -d->bdiag[k] * v2;
-      if (k > 0) { const double a = vk * vm(d->parent[k]); Pc += -d->g[k] * a; Qc += d->b[k] * a; }
-      for (int q = d->child_ptr[k]; q < d->child_ptr[k + 1]; ++q) {
-        const int c = d->child_idx[q];
-        const double a = vk * vm(c);
-        Pc += -d->g[c] * a; Qc += d->b[c] * a;
-      }
-      double d00 = -Qc - d->bdiag[k] * v2, d01 = Pc + d->gdiag[k] * v2, d10 = Pc - d->gdiag[k] * v2,
-             d11 = Qc - d->bdiag[k] * v2;
-      for (int q = d->child_ptr[k]; q < d->child_ptr[k + 1]; ++q) {
-        const double* cc = &C[4 * (size_t)d->child_idx[q]];
-        d00 -= cc[0]; d01 -= cc[1]; d10 -= cc[2]; d11 -= cc[3];
-      }
-      const double a = k > 0 ? vk * vm(d->parent[k]) : 0.0;
-      const double gk = k > 0 ? d->g[k] : 0.0, bk = k > 0 ? d->b[k] : 0.0;
-      const double ga = -gk * a, al = bk * a, gl = -gk * a, ll = bk * a;      // sin = 0 at a flat start
-      double u00 = al, u01 = ga, u10 = -ga, u11 = al;
-      if (!th) { d00 = 1.0; d01 = 0.0; u00 = u01 = 0.0; }
-      if (!pq) { d10 = 0.0; d11 = 1.0; u10 = u11 = 0.0; }
-      const double det = d00 * d11 - d01 * d10;
-      if (det == 0.0 || !(det == det)) { ok = false; break; }
-      const double inv = 1.0 / det;
-      const double i00 = d11 * inv, i01 = -d01 * inv, i10 = -d10 * inv, i11 = d00 * inv;
-      const double m00 = i00 * u00 + i01 * u10, m01 = i00 * u01 + i01 * u11,
-                   m10 = i10 * u00 + i11 * u10, m11 = i10 * u01 + i11 * u11;
-      // six 16-byte fields per position, field-major (field f of position p at f0[2 * (f * P + p)]): the lanes
-      // of a row read consecutive 16-byte units
-      const int p = pos[k];
-      auto put = [&](int fld, double a0, double a1) {
-        f0[2 * ((size_t)fld * P + p)] = a0; f0[2 * ((size_t)fld * P + p) + 1] = a1;
-      };
-      put(0, i00, i01); put(1, i10, i11);
-      put(2, m00, m01); put(3, m10, m11);
-      put(4, ll, gl);
-      put(5, Pc, Qc);                                  // calculated injections of the flat profile
-      double* cc = &C[4 * (size_t)k];
-      cc[0] = ll * m00 + gl * m10; cc[1] = ll * m01 + gl * m11;
-      cc[2] = -gl * m00 + ll * m10; cc[3] = -gl * m01 + ll * m11;
-    }
-    lay.o_f0 = ok ? dbase + ib.add_d(f0.data(), 12 * P) : -1;     // singular at the flat start: no shortcut
+    const std::vector<double> f0 = flat_start_factors(d, pos, P);
+    if (!f0.empty()) lay.o_f0 = dbase + ib.add_d(f0.data(), 12 * P);     // singular at the flat start: no shortcut
   }
   if (nt) {
     std::vector<double> ty(2 * (size_t)nt), tz(2 * (size_t)nt);
@@ -618,7 +616,6 @@ inline std::string build_feeder_image(const gfr_feeder_desc* d, int lanes, int s
   std::vector<double> load_pq(2 * (size_t)L + 1, 0.0);
   for (int l = 0; l < L; ++l) { load_pq[2 * l] = d->load_p[l]; load_pq[2 * l + 1] = d->load_q[l]; }
 
-  f->root_is_slack = d->bus_type[0] == GFR_BUS_SLACK;
   f->img.swap(img);
   f->load_pq.swap(load_pq);
   return std::string();
