@@ -105,10 +105,14 @@ SIGNATURES: Dict[str, Tuple[object, List[object]]] = {
     "gfr_env_reset_outputs": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(StepOut), C.c_void_p]),
     "gfr_env_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(StepOut), C.c_void_p]),
     "gfr_solve": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.POINTER(SolverCfg), C.POINTER(SolOut), C.c_void_p]),
+    "gfr_solve_pq": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.POINTER(SolverCfg), C.POINTER(SolOut),
+                               C.c_void_p]),
     "gfr_network_create": (C.c_int, [C.POINTER(NetworkDesc), C.c_int, C.POINTER(C.c_void_p)]),
     "gfr_network_destroy": (None, [C.c_void_p]),
     "gfr_network_unknowns": (C.c_int, [C.c_void_p]),
     "gfr_network_solve": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.POINTER(SolverCfg), C.POINTER(SolOut), C.c_void_p]),
+    "gfr_network_solve_pq": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_void_p, C.POINTER(SolverCfg),
+                                       C.POINTER(SolOut), C.c_void_p]),
     "gfr_noise_fill": (C.c_int, [C.c_int, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "gfr_fp64_peak": (C.c_int, [C.c_int, C.POINTER(C.c_double)]),
     "gfr_launch_count": (C.c_int64, []),

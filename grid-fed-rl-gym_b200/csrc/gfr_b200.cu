@@ -70,7 +70,7 @@ __device__ __forceinline__ void stage_image(unsigned char* smem, const void* img
 constexpr int kRedBytes = 128;    // cross-warp reduction scratch of a CTA-wide group (16 doubles)
 
 // Shared memory of a CTA: [mbarrier 16 B][feeder image, if staged][reduction scratch, if LANES > 32][slots]
-template <int LANES, int SOLVER>
+template <int LANES, int SOLVER, bool SPEC_Q = false>
 __device__ __forceinline__ typename GroupOf<LANES, SOLVER>::type
 make_group(const Layout& lay, unsigned char* work, int slot_bytes, D2* mscratch, double* p_local) {
   typename GroupOf<LANES, SOLVER>::type g;
@@ -81,8 +81,8 @@ make_group(const Layout& lay, unsigned char* work, int slot_bytes, D2* mscratch,
   if (LANES > 32) work += kRedBytes;
   const int slot = threadIdx.x / LANES;
   const int E = blockDim.x / LANES;
-  D2* mg = mscratch ? mscratch + ((size_t)blockIdx.x * E + slot) * (newton_scratch_doubles(lay.P) / 2) : nullptr;
-  bind_slot(g, work + (size_t)slot * slot_bytes, lay, mg, p_local);
+  D2* mg = mscratch ? mscratch + ((size_t)blockIdx.x * E + slot) * (newton_scratch_doubles(lay.P, SPEC_Q) / 2) : nullptr;
+  bind_slot<LANES, SPEC_Q>(g, work + (size_t)slot * slot_bytes, lay, mg, p_local);
   return g;
 }
 
@@ -121,6 +121,24 @@ solve_kernel(const Layout lay, const EnvCfg cfg, const void* __restrict__ img, c
   const int E = blockDim.x / LANES;
   for (long long env = (long long)blockIdx.x * E + threadIdx.x / LANES; env < B; env += (long long)gridDim.x * E)
     solve_instance<LANES, SOLVER>(g, lay, simg, dimg, cfg, env, p_inj, o);
+}
+
+// solve_kernel with specified Q at the PQ buses (q_inj [B, n]).  A kernel of its own, so that solve_kernel, which
+// P-only callers run, keeps its machine code: the Newton scratch holds (P, Q) pairs, the sweep slot 48 B per bus
+template <int LANES, int SOLVER, bool IMG_SMEM>
+__global__ void __launch_bounds__(kMaxThreads)
+solve_pq_kernel(const Layout lay, const EnvCfg cfg, const void* __restrict__ img, const int slot_bytes,
+                D2* __restrict__ mscratch, const double* __restrict__ p_inj, const double* __restrict__ q_inj,
+                const SolOut o, const long long B) {
+  extern __shared__ __align__(16) unsigned char smem[];
+  if (IMG_SMEM) stage_image(smem, img, lay.img_bytes);
+  const int* simg = IMG_SMEM ? (const int*)(smem + kSmemHeader) : (const int*)img;
+  const double* dimg = IMG_SMEM ? (const double*)(smem + kSmemHeader) : (const double*)img;
+  auto g = make_group<LANES, SOLVER, true>(lay, smem + kSmemHeader + (IMG_SMEM ? lay.img_bytes : 0),
+                                           slot_bytes, mscratch, nullptr);
+  const int E = blockDim.x / LANES;
+  for (long long env = (long long)blockIdx.x * E + threadIdx.x / LANES; env < B; env += (long long)gridDim.x * E)
+    solve_instance<LANES, SOLVER, true>(g, lay, simg, dimg, cfg, env, p_inj, o, q_inj);
 }
 
 // reset: 4 lanes per instance, image read through L2 (touched once per instance)
@@ -295,6 +313,9 @@ namespace {
 
 struct LaunchPlan { int lanes, threads, grid; size_t smem; int ctas_per_sm; int slot_bytes; size_t mscratch_bytes; bool img_smem; };
 
+// which kernel a launch plan is for: the environment step, the solve, the solve with specified Q
+enum KernelKind { K_STEP, K_SOLVE, K_SOLVE_PQ };
+
 // the image of a feeder for one (solver, lanes): built and uploaded on first use
 int image_for(const gfr_feeder* f, int solver, int lanes, const ImageDev** out) {
   const int key = solver * 1024 + lanes;
@@ -314,9 +335,10 @@ int image_for(const gfr_feeder* f, int solver, int lanes, const ImageDev** out) 
 }
 
 // shared memory of one instance slot; 0 if the scratch it doubles as cannot hold the sources
-size_t slot_bytes(const Layout& lay, int solver, int lanes) {
+size_t slot_bytes(const Layout& lay, int solver, int lanes, int kind) {
+  const bool spec_q = kind == K_SOLVE_PQ;
   return solver == GFR_SOLVER_NEWTON ? newton_slot_bytes(lay.n, lay.n_pool, lay.n_src)
-                                     : sweep_slot_bytes(lay.n, lay.n_src, sweep_p_local(lanes, lay.n), lay.n_tie);
+                                     : sweep_slot_bytes(lay.n, lay.n_src, !spec_q && sweep_p_local(lanes, lay.n), lay.n_tie, spec_q);
 }
 
 // Threads cooperating on one instance when the caller does not say: THE rule (exported as gfr_auto_lanes; the
@@ -342,23 +364,26 @@ int auto_lanes_rule(int n, int solver, int depth) {
   return 128;                      // one CTA per instance
 }
 
-// The step or solve kernel of one (lanes, image placement) out of the lane list L it is compiled for: 1 - 32 lanes
-// with the image in shared memory, 32 - 256 without it; nullptr for any other lane count
+// The step, solve or Q solve kernel of one (lanes, image placement) out of the lane list L it is compiled for: 1 - 32
+// lanes with the image in shared memory, 32 - 256 without it; nullptr for any other lane count
 template <int SOLVER, bool IMG_SMEM, int... L>
-const void* kernel_in(bool step, int lanes) {
+const void* kernel_in(int kind, int lanes) {
   const void* fn = nullptr;
-  auto pick = [&](int l, const void* step_k, const void* solve_k) { if (lanes == l) fn = step ? step_k : solve_k; };
-  (pick(L, (const void*)step_kernel<L, SOLVER, IMG_SMEM>, (const void*)solve_kernel<L, SOLVER, IMG_SMEM>), ...);
+  auto pick = [&](int l, const void* step_k, const void* solve_k, const void* solve_pq_k) {
+    if (lanes == l) fn = kind == K_STEP ? step_k : kind == K_SOLVE ? solve_k : solve_pq_k;
+  };
+  (pick(L, (const void*)step_kernel<L, SOLVER, IMG_SMEM>, (const void*)solve_kernel<L, SOLVER, IMG_SMEM>,
+        (const void*)solve_pq_kernel<L, SOLVER, IMG_SMEM>), ...);
   return fn;
 }
 template <int SOLVER>
-const void* kernel_of(bool step, int lanes, bool img_smem) {
-  return img_smem ? kernel_in<SOLVER, true, 1, 2, 4, 8, 16, 32>(step, lanes)
-                  : kernel_in<SOLVER, false, 32, 64, 128, 256>(step, lanes);
+const void* kernel_of(int kind, int lanes, bool img_smem) {
+  return img_smem ? kernel_in<SOLVER, true, 1, 2, 4, 8, 16, 32>(kind, lanes)
+                  : kernel_in<SOLVER, false, 32, 64, 128, 256>(kind, lanes);
 }
-const void* kernel_fn(bool step, int solver, int lanes, bool img_smem, bool ties) {
-  if (solver == GFR_SOLVER_NEWTON) return kernel_of<SOLVER_NEWTON>(step, lanes, img_smem);
-  return ties ? kernel_of<SOLVER_SWEEP_TIES>(step, lanes, img_smem) : kernel_of<SOLVER_SWEEP>(step, lanes, img_smem);
+const void* kernel_fn(int kind, int solver, int lanes, bool img_smem, bool ties) {
+  if (solver == GFR_SOLVER_NEWTON) return kernel_of<SOLVER_NEWTON>(kind, lanes, img_smem);
+  return ties ? kernel_of<SOLVER_SWEEP_TIES>(kind, lanes, img_smem) : kernel_of<SOLVER_SWEEP>(kind, lanes, img_smem);
 }
 
 // One candidate split of an SM: `c` CTAs of E instance slots each.
@@ -411,7 +436,7 @@ PlanTry plan_mode(const gfr_feeder* f, const Layout& lay, const void* fn, int la
 // instances resident, checked against the kernel's real register use through the occupancy API.
 // Small and medium feeders stage one copy of the feeder image per CTA; when that leaves fewer than
 // four instances resident (or the group is CTA-wide) the image is read from global memory instead.
-int plan_launch(const gfr_feeder* f, bool step, int solver, int lanes, long long B, LaunchPlan* out,
+int plan_launch(const gfr_feeder* f, int kind, int solver, int lanes, long long B, LaunchPlan* out,
                 const void** fn_out, const ImageDev** img_out) {
   // the lane count the description's level schedule was capped for, else the rule
   if (lanes == 0) lanes = f->lanes_hint > 0 ? f->lanes_hint : auto_lanes_rule(f->lay.n, solver, f->center_depth);
@@ -422,14 +447,14 @@ int plan_launch(const gfr_feeder* f, bool step, int solver, int lanes, long long
   if (int rc = image_for(f, solver, lanes, &im)) return rc;
   const Layout& lay = im->lay;
   *img_out = im;
-  const size_t per_env = slot_bytes(lay, solver, lanes);
+  const size_t per_env = slot_bytes(lay, solver, lanes, kind);
   if (!per_env)
     return fail(GFR_E_LIMIT, "more loads + generators + batteries than the solver's working set can stage "
                              "(sweep: 2 per bus on average)");
   PlanTry best;
-  if (lanes <= 32) best = plan_mode(f, lay, kernel_fn(step, solver, lanes, true, lay.n_tie > 0), lanes, true, per_env, B);
+  if (lanes <= 32) best = plan_mode(f, lay, kernel_fn(kind, solver, lanes, true, lay.n_tie > 0), lanes, true, per_env, B);
   if (lanes > 32 || (lanes == 32 && best.resident < 4)) {
-    PlanTry alt = plan_mode(f, lay, kernel_fn(step, solver, lanes, false, lay.n_tie > 0), lanes, false, per_env, B);
+    PlanTry alt = plan_mode(f, lay, kernel_fn(kind, solver, lanes, false, lay.n_tie > 0), lanes, false, per_env, B);
     if (alt.resident > best.resident) best = alt;
   }
   if (!best.resident)
@@ -467,9 +492,9 @@ int plan_launch(const gfr_feeder* f, bool step, int solver, int lanes, long long
   plan.grid = (int)grid;
   plan.slot_bytes = (int)per_env;
   // Newton spills D^-1 U (32 B per bus) of every resident instance slot to global memory
-  plan.mscratch_bytes = solver == GFR_SOLVER_NEWTON ? (size_t)grid * E * newton_scratch_doubles(lay.P) * 8 : 0;
+  plan.mscratch_bytes = solver == GFR_SOLVER_NEWTON ? (size_t)grid * E * newton_scratch_doubles(lay.P, kind == K_SOLVE_PQ) * 8 : 0;
   *out = plan;
-  *fn_out = kernel_fn(step, solver, lanes, plan.img_smem, lay.n_tie > 0);
+  *fn_out = kernel_fn(kind, solver, lanes, plan.img_smem, lay.n_tie > 0);
   return GFR_OK;
 }
 
@@ -492,15 +517,18 @@ int launch_step(const gfr_env* e, const double* actions, const double* noise, co
   return GFR_OK;
 }
 
+// solve_kernel, or solve_pq_kernel when q_inj is given
 int launch_solve(const ImageDev* im, const LaunchPlan& p, const void* fn, const EnvCfg& cfg,
-                 const double* p_inj, const SolOut& o, long long B, cudaStream_t s) {
+                 const double* p_inj, const double* q_inj, const SolOut& o, long long B, cudaStream_t s) {
   const void* img = im->d_img;
   int slot = p.slot_bytes;
   D2* ms = nullptr;
   if (p.mscratch_bytes) GFR_CUDA(cudaMallocAsync((void**)&ms, p.mscratch_bytes, s));   // stream-ordered scratch
   void* args[] = {(void*)&im->lay, (void*)&cfg, (void*)&img, (void*)&slot, (void*)&ms, (void*)&p_inj, (void*)&o,
                   (void*)&B};
-  cudaError_t le = cudaLaunchKernel(fn, dim3(p.grid), dim3(p.threads), args, p.smem, s);
+  void* args_pq[] = {(void*)&im->lay, (void*)&cfg, (void*)&img, (void*)&slot, (void*)&ms, (void*)&p_inj,
+                     (void*)&q_inj, (void*)&o, (void*)&B};
+  cudaError_t le = cudaLaunchKernel(fn, dim3(p.grid), dim3(p.threads), q_inj ? args_pq : args, p.smem, s);
   if (ms) cudaFreeAsync(ms, s);
   if (le != cudaSuccess) return cuda_fail(le, "cudaLaunchKernel(solve)");
   g_launches.fetch_add(1);
@@ -617,7 +645,7 @@ int gfr_env_create(const gfr_feeder* f, int64_t n_envs, const gfr_env_cfg* cfg, 
   LaunchPlan plan;
   const void* fn = nullptr;
   const ImageDev* im = nullptr;
-  if (int rc = plan_launch(f, true, cfg->solver.solver, cfg->solver.lanes, n_envs, &plan, &fn, &im)) return rc;
+  if (int rc = plan_launch(f, K_STEP, cfg->solver.solver, cfg->solver.lanes, n_envs, &plan, &fn, &im)) return rc;
   auto* e = new gfr_env();
   e->f = f; e->img = im; e->B = n_envs; e->cfg = ec; e->solver = cfg->solver.solver;
   e->lanes = plan.lanes; e->threads = plan.threads; e->grid = plan.grid; e->smem = plan.smem; e->fn = fn;
@@ -757,6 +785,11 @@ int gfr_env_reset_outputs(gfr_env* e, const uint8_t* mask, const gfr_step_out* o
 
 int gfr_solve(const gfr_feeder* f, int64_t B, const double* p_inj, const gfr_solver_cfg* cfg,
               const gfr_sol_out* out, void* stream) {
+  return gfr_solve_pq(f, B, p_inj, nullptr, cfg, out, stream);
+}
+
+int gfr_solve_pq(const gfr_feeder* f, int64_t B, const double* p_inj, const double* q_inj, const gfr_solver_cfg* cfg,
+                 const gfr_sol_out* out, void* stream) {
   if (!f || !p_inj || !cfg || !out) return fail(GFR_E_ARG, "null argument");
   if (B < 1) return fail(GFR_E_ARG, "B must be >= 1");
   if (int rc = check_solver_cfg(f, cfg)) return rc;
@@ -765,8 +798,8 @@ int gfr_solve(const gfr_feeder* f, int64_t B, const double* p_inj, const gfr_sol
   LaunchPlan plan;
   const void* fn = nullptr;
   const ImageDev* im = nullptr;
-  if (int rc = plan_launch(f, false, cfg->solver, cfg->lanes, B, &plan, &fn, &im)) return rc;
-  return launch_solve(im, plan, fn, env_cfg_of(cfg), p_inj, *out, B, (cudaStream_t)stream);
+  if (int rc = plan_launch(f, q_inj ? K_SOLVE_PQ : K_SOLVE, cfg->solver, cfg->lanes, B, &plan, &fn, &im)) return rc;
+  return launch_solve(im, plan, fn, env_cfg_of(cfg), p_inj, q_inj, *out, B, (cudaStream_t)stream);
 }
 
 int gfr_network_create(const gfr_network_desc* d, int device, gfr_network** out) {
@@ -859,19 +892,27 @@ int gfr_network_unknowns(const gfr_network* net) { return net ? net->nd.N : 0; }
 
 int gfr_network_solve(const gfr_network* net, int64_t B, const double* p_inj, const gfr_solver_cfg* cfg,
                       const gfr_sol_out* out, void* stream) {
+  return gfr_network_solve_pq(net, B, p_inj, nullptr, cfg, out, stream);
+}
+
+int gfr_network_solve_pq(const gfr_network* net, int64_t B, const double* p_inj, const double* q_inj,
+                         const gfr_solver_cfg* cfg, const gfr_sol_out* out, void* stream) {
   if (!net || !p_inj || !cfg || !out) return fail(GFR_E_ARG, "null argument");
   if (B < 1) return fail(GFR_E_ARG, "B must be >= 1");
   if (int rc = check_stopping(cfg)) return rc;
   DeviceGuard guard(net->device);
   if (!guard.ok) return no_device();
   // kernel choice: [J | mismatch] in registers up to 127 unknowns (cfg->lanes: 0 = this choice, 1 = always the
-  // shared-memory kernel, 2 = the register kernel or GFR_E_LIMIT)
+  // shared-memory kernel, 2 = the register kernel or GFR_E_LIMIT); with q_inj, their specified-Q instantiations
   typedef void (*dense_fn)(const NetDev, const double, const int, const double, const double*, const SolOut, const long long);
+  typedef void (*dense_pq_fn)(const NetDev, const double, const int, const double, const double*, const double*,
+                              const SolOut, const long long);
   const int N = net->nd.N;
   if (cfg->lanes < 0 || cfg->lanes > 2) return fail(GFR_E_ARG, "lanes must be 0 (auto), 1 (shared-memory LU) or 2 (register LU) for a network solve");
   if (cfg->lanes == 2 && N > 127) return fail(GFR_E_LIMIT, "the register-resident elimination takes at most 127 unknowns");
   const bool in_regs = cfg->lanes != 1 && N <= 127;
   dense_fn fn = dense_solve_kernel;
+  dense_pq_fn fn_pq = dense_solve_pq_kernel;
   int threads = N <= 48 ? 128 : 256;
   size_t smem = dense_smem_bytes(net->nd.n, N);
   if (in_regs) {
@@ -883,18 +924,26 @@ int gfr_network_solve(const gfr_network* net, int64_t B, const double* p_inj, co
                                      K<16, 8>, K<16, 9>, K<16, 10>, K<16, 11>, K<16, 12>,
                                      K<32, 13>, K<32, 14>, K<32, 15>, K<32, 16> };
 #undef K
+#define K dense_solve_reg_pq_kernel
+    static const dense_pq_fn by_r_pq[] = { nullptr, K<8, 1>, K<8, 2>, K<8, 3>, K<8, 4>, K<8, 5>, K<8, 6>, K<8, 7>,
+                                           K<16, 8>, K<16, 9>, K<16, 10>, K<16, 11>, K<16, 12>,
+                                           K<32, 13>, K<32, 14>, K<32, 15>, K<32, 16> };
+#undef K
     const int tx = N <= 56 ? 8 : N <= 96 ? 16 : 32;
     fn = by_r[(N + 7) / 8];
+    fn_pq = by_r_pq[(N + 7) / 8];
     threads = 8 * tx;
   }
-  GFR_CUDA(cudaFuncSetAttribute((const void*)fn, cudaFuncAttributeMaxDynamicSharedMemorySize, net->smem_optin));
+  const void* kfn = q_inj ? (const void*)fn_pq : (const void*)fn;
+  GFR_CUDA(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, net->smem_optin));
   int per_sm = 0;
-  GFR_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, (const void*)fn, threads, smem));
+  GFR_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kfn, threads, smem));
   if (per_sm < 1) return fail(GFR_E_LIMIT, "the dense Jacobian of this network exceeds the shared memory of an SM");
   long long grid = (long long)net->sm_count * per_sm;
   if (grid > B) grid = B;
   const EnvCfg k = env_cfg_of(cfg);
-  fn<<<(int)grid, threads, smem, (cudaStream_t)stream>>>(net->nd, k.tol, k.max_it, k.accel, p_inj, *out, (long long)B);
+  if (q_inj) fn_pq<<<(int)grid, threads, smem, (cudaStream_t)stream>>>(net->nd, k.tol, k.max_it, k.accel, p_inj, q_inj, *out, (long long)B);
+  else fn<<<(int)grid, threads, smem, (cudaStream_t)stream>>>(net->nd, k.tol, k.max_it, k.accel, p_inj, *out, (long long)B);
   g_launches.fetch_add(1);
   GFR_CUDA(cudaGetLastError());
   return GFR_OK;

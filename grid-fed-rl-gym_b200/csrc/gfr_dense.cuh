@@ -71,9 +71,12 @@ __device__ __forceinline__ void dense_flat_start(const NetDev& net, D2* ef, int 
   }
 }
 
-// calculated injections and mismatch (:150-166); returns the NaN-propagating maximum over the CTA
+// calculated injections and mismatch (:150-166); returns the NaN-propagating maximum over the CTA.
+// SPEC_Q: PQ buses have a specified Q (qspec); without it Q_spec = 0, as in the reference.
+template <bool SPEC_Q = false>
 __device__ __forceinline__ double dense_mismatch(const NetDev& net, const D2* ef, D2* pq, double* rhs,
-                                                 const double* __restrict__ pspec, double* red, int tid, int nt) {
+                                                 const double* __restrict__ pspec, const double* __restrict__ qspec,
+                                                 double* red, int tid, int nt) {
   double mm = 0.0;
   for (int i = tid; i < net.n; i += nt) {
     const D2 vi = ef[i];
@@ -92,7 +95,7 @@ __device__ __forceinline__ double dense_mismatch(const NetDev& net, const D2* ef
     const int rt = net.col_theta[i], rv = net.col_vm[i];
     double aP = 0.0, aQ = 0.0;
     if (rt >= 0) { const double d = pspec[i] - P; rhs[rt] = d; aP = fabs(d); }
-    if (rv >= 0) { const double d = 0.0 - Q; rhs[rv] = d; aQ = fabs(d); }
+    if (rv >= 0) { const double d = (SPEC_Q ? qspec[i] : 0.0) - Q; rhs[rv] = d; aQ = fabs(d); }
     const double loc = (aQ > aP || aQ != aQ) ? aQ : aP;
     mm = (loc > mm || loc != loc) ? loc : mm;
   }
@@ -142,8 +145,10 @@ __device__ __forceinline__ void dense_jacobian(const NetDev& net, const D2* ef, 
 // Mismatch and Jacobian in ONE pass over the adjacency lists (the register kernel): the same arithmetic, term
 // by term, as dense_mismatch + dense_jacobian; J must be zero on entry (the caller clears it while the
 // elimination result is scattered).  The Jacobian of the converged iterate is wasted, once per solve.
+template <bool SPEC_Q = false>
 __device__ __forceinline__ double dense_mismatch_jacobian(const NetDev& net, const D2* ef, double* J, int ld,
                                                           double* rhs, const double* __restrict__ pspec,
+                                                          const double* __restrict__ qspec,
                                                           double* red, int tid, int nt) {
   double mm = 0.0;
   for (int i = tid; i < net.n; i += nt) {
@@ -181,7 +186,7 @@ __device__ __forceinline__ double dense_mismatch_jacobian(const NetDev& net, con
         J[rv + rv * ld] = fma(-yd.y, v2, Q);                         // V dQ/dV:       Q - B v2
       }
     }
-    if (rv >= 0) { const double d = 0.0 - Q; rhs[rv] = d; aQ = fabs(d); }
+    if (rv >= 0) { const double d = (SPEC_Q ? qspec[i] : 0.0) - Q; rhs[rv] = d; aQ = fabs(d); }
     const double loc = (aQ > aP || aQ != aQ) ? aQ : aP;
     mm = (loc > mm || loc != loc) ? loc : mm;
   }
@@ -253,9 +258,11 @@ __device__ __forceinline__ bool pivot_takes(double ob, int oi, double best, int 
 }
 
 // ---- kernel 1: Jacobian factorised in shared memory (any N that fits; used for N >= 128) ---------------------
-__global__ void __launch_bounds__(256)
-dense_solve_kernel(const NetDev net, const double tol, const int max_it, const double accel,
-                   const double* __restrict__ p_inj, const SolOut o, const long long B) {
+// (SPEC_Q: q_inj [B, n] specified Q at the PQ buses; dense_solve_pq_kernel)
+template <bool SPEC_Q>
+__device__ __forceinline__ void dense_solve(const NetDev& net, const double tol, const int max_it, const double accel,
+                                            const double* __restrict__ p_inj, const double* __restrict__ q_inj,
+                                            const SolOut& o, const long long B) {
   extern __shared__ __align__(16) unsigned char smem[];
   const int n = net.n, N = net.N;
   const int ld = N | 1;
@@ -269,12 +276,13 @@ dense_solve_kernel(const NetDev net, const double tol, const int max_it, const d
 
   for (long long env = blockIdx.x; env < B; env += gridDim.x) {
     const double* pspec = p_inj + env * n;
+    const double* qspec = SPEC_Q ? q_inj + env * n : nullptr;
     dense_flat_start(net, ef, tid, nt);
     __syncthreads();
     int converged = 0, iterations = max_it;
     double max_mismatch = INFINITY;
     for (int it = 0; it < max_it; ++it) {
-      const double mm = dense_mismatch(net, ef, pq, rhs, pspec, red, tid, nt);
+      const double mm = dense_mismatch<SPEC_Q>(net, ef, pq, rhs, pspec, qspec, red, tid, nt);
       max_mismatch = mm;
       if (mm < tol) { converged = 1; iterations = it + 1; break; }      // checked before the update (:168-171)
       dense_jacobian(net, ef, pq, J, ld, tid, nt);
@@ -359,6 +367,17 @@ dense_solve_kernel(const NetDev net, const double tol, const int max_it, const d
     }
     dense_results(net, ef, red, o, env, converged, iterations, max_mismatch, tid, nt);
   }
+}
+__global__ void __launch_bounds__(256)
+dense_solve_kernel(const NetDev net, const double tol, const int max_it, const double accel,
+                   const double* __restrict__ p_inj, const SolOut o, const long long B) {
+  dense_solve<false>(net, tol, max_it, accel, p_inj, nullptr, o, B);
+}
+__global__ void __launch_bounds__(256)
+dense_solve_pq_kernel(const NetDev net, const double tol, const int max_it, const double accel,
+                      const double* __restrict__ p_inj, const double* __restrict__ q_inj, const SolOut o,
+                      const long long B) {
+  dense_solve<true>(net, tol, max_it, accel, p_inj, q_inj, o, B);
 }
 
 // ---- kernel 2: [J | mismatch] in REGISTERS, N <= 127 ----------------------------------------------------------
@@ -469,10 +488,10 @@ constexpr int dense_reg_min_blocks(int TX, int R) {
   return regs > 96 ? 0 : b > 24 ? 24 : b;   // 0 = no request
 }
 
-template <int TX, int R>
-__global__ void __launch_bounds__(8 * TX, dense_reg_min_blocks(TX, R))
-dense_solve_reg_kernel(const NetDev net, const double tol, const int max_it, const double accel,
-                       const double* __restrict__ p_inj, const SolOut o, const long long B) {
+template <int TX, int R, bool SPEC_Q>
+__device__ __forceinline__ void dense_solve_reg(const NetDev& net, const double tol, const int max_it,
+                                                const double accel, const double* __restrict__ p_inj,
+                                                const double* __restrict__ q_inj, const SolOut& o, const long long B) {
   constexpr int TY = 8, C = 8 * R / TX + 1, nt = TY * TX;
   static_assert(R >= 1 && R <= 16 && C >= 1 && C <= 10 && nt % 32 == 0, "8 R rows <= 128; whole warps");
   extern __shared__ __align__(16) unsigned char smem[];
@@ -496,13 +515,14 @@ dense_solve_reg_kernel(const NetDev net, const double tol, const int max_it, con
 
   for (long long env = blockIdx.x; env < B; env += gridDim.x) {
     const double* pspec = p_inj + env * n;
+    const double* qspec = SPEC_Q ? q_inj + env * n : nullptr;
     dense_flat_start(net, ef, tid, nt);
     for (int q = tid; q < ld * N; q += nt) J[q] = 0.0;
     __syncthreads();
     int converged = 0, iterations = max_it;
     double max_mismatch = INFINITY;
     for (int it = 0; it < max_it; ++it) {
-      const double mm = dense_mismatch_jacobian(net, ef, J, ld, rhs, pspec, red, tid, nt);   // ends with a barrier
+      const double mm = dense_mismatch_jacobian<SPEC_Q>(net, ef, J, ld, rhs, pspec, qspec, red, tid, nt);   // ends with a barrier
       max_mismatch = mm;
       if (mm < tol) { converged = 1; iterations = it + 1; break; }
       double a[R][C];
@@ -549,6 +569,19 @@ dense_solve_reg_kernel(const NetDev net, const double tol, const int max_it, con
     }
     dense_results(net, ef, red, o, env, converged, iterations, max_mismatch, tid, nt);
   }
+}
+template <int TX, int R>
+__global__ void __launch_bounds__(8 * TX, dense_reg_min_blocks(TX, R))
+dense_solve_reg_kernel(const NetDev net, const double tol, const int max_it, const double accel,
+                       const double* __restrict__ p_inj, const SolOut o, const long long B) {
+  dense_solve_reg<TX, R, false>(net, tol, max_it, accel, p_inj, nullptr, o, B);
+}
+template <int TX, int R>
+__global__ void __launch_bounds__(8 * TX, dense_reg_min_blocks(TX, R))
+dense_solve_reg_pq_kernel(const NetDev net, const double tol, const int max_it, const double accel,
+                          const double* __restrict__ p_inj, const double* __restrict__ q_inj, const SolOut o,
+                          const long long B) {
+  dense_solve_reg<TX, R, true>(net, tol, max_it, accel, p_inj, q_inj, o, B);
 }
 #undef GFR_LIVE_CASE
 

@@ -52,7 +52,7 @@ enum { GEN_SOLAR = 0, GEN_WIND = 1 };
 //            again in the back-substitution, and the specified injections live in a per-slot scratch
 //            in global memory, by position, that stays L2 resident; the back-substitution loads them
 //            two rows ahead into registers.
-//   sweep:   40 B per bus in three arrays: e + jf | Jr + jJi (branch current) | P
+//   sweep:   40 B per bus in three arrays: e + jf | Jr + jJi (branch current) | P  (P + jQ, 48 B: solve with Q)
 // Before the solve the same space (Newton: ef + pool; sweep: the J fields) carries the load /
 // generator / battery powers into the per-position injection sums.
 enum { F_E = 0, F_F = 1, F_SCRATCH = 2 };
@@ -295,6 +295,9 @@ struct SGrp : Lanes<LANES> {
   GFR_HD D2& ef(int k) const { return efp[k]; }
   GFR_HD double pspec(int k) const { return pp[k]; }
   GFR_HD void set_pspec(int k, double v) const { pp[k] = v; }
+  // kernels with specified Q: (P, Q) of bus k, 16 B per bus where the P-only kernels keep 8
+  GFR_HD D2 pqspec(int k) const { return reinterpret_cast<const D2*>(pp)[k]; }
+  GFR_HD void set_pqspec(int k, D2 v) const { reinterpret_cast<D2*>(pp)[k] = v; }
   GFR_HD double& scr(int j) const { return reinterpret_cast<double*>(jrp)[j]; }           // sources: the J array, flat (2 n doubles)
 };
 
@@ -313,8 +316,26 @@ struct NGrp : Lanes<LANES> {
   GFR_HD D2& ef(int k) const { return efp[k]; }
   GFR_HD double pspec(int p) const { return ld_scratch1(pp + p, pol); }
   GFR_HD void set_pspec(int p, double v) const { st_scratch1(pp + p, v, pol); }
+  // kernels with specified Q: (P, Q) of position p, in the same place (2 P doubles instead of P)
+  GFR_HD D2 pqspec(int p) const { return ld_scratch(reinterpret_cast<const D2*>(pp) + p, pol); }
+  GFR_HD void set_pqspec(int p, D2 v) const { st_scratch(reinterpret_cast<D2*>(pp) + p, v, pol); }
   GFR_HD double& scr(int j) const { return reinterpret_cast<double*>(efp)[j]; }   // ef + pool, flat
 };
+
+// The specified injection of a position (Newton) or bus (sweep): P (a double), or (P, Q) in the kernels compiled
+// with SPEC_Q.  The P-only kernels keep a plain double (a D2 with a constant 0 changed their register allocation),
+// and spec_q() of it is the reference's Q_spec = 0.
+template <bool SPEC_Q> struct SpecT { typedef double type; };
+template <> struct SpecT<true> { typedef D2 type; };
+template <bool SPEC_Q, class G>
+GFR_HD typename SpecT<SPEC_Q>::type spec_of(const G& g, int p) {
+  if constexpr (SPEC_Q) return g.pqspec(p);
+  else return g.pspec(p);
+}
+GFR_HD double spec_p(double s) { return s; }
+GFR_HD double spec_p(const D2& s) { return s.x; }
+GFR_HD double spec_q(double) { return 0.0; }
+GFR_HD double spec_q(const D2& s) { return s.y; }
 
 template <int LANES, int SOLVER> struct GroupOf { typedef NGrp<LANES> type; };
 template <int LANES> struct GroupOf<LANES, SOLVER_SWEEP> { typedef SGrp<LANES> type; };
@@ -326,20 +347,26 @@ GFR_HD size_t newton_slot_bytes(int n, int n_pool, int n_src) {
   return (size_t)n * 16 + (size_t)n_pool * (16 * POOL_D2);
 }
 // doubles of global scratch per instance slot (Newton): D^-1 U, D^-1 r (48 B per position) + specified injections
-// (a whole number of 128-byte lines per slot: a slot's lines can be dropped from L2 without touching a neighbour's)
-GFR_HD size_t newton_scratch_doubles(int P) { return (((size_t)P * 6 + (((size_t)P + 1) / 2) * 2) + 15) & ~(size_t)15; }
+// (a whole number of 128-byte lines per slot: a slot's lines can be dropped from L2 without touching a neighbour's).
+// The kernels with specified Q keep (P, Q) pairs there: 16 B per position instead of 8.
+GFR_HD size_t newton_scratch_doubles(int P, bool spec_q = false) {
+  return (((size_t)P * 6 + (spec_q ? 2 * (size_t)P : (((size_t)P + 1) / 2) * 2)) + 15) & ~(size_t)15;
+}
 // One thread per instance on a small feeder: the specified injections move to a per-thread local array (L1,
-// interleaved by thread), 32 B per bus stay in shared memory - 40 % more resident instances per SM
+// interleaved by thread), 32 B per bus stay in shared memory - 40 % more resident instances per SM.  The kernels with
+// specified Q keep (P, Q) in the slot instead (48 B per bus): they serve the solve entry points, not the step, and a
+// second local array would be one more placement of the injections to keep in step with the slot layout.
 enum { SWEEP_P_LOCAL_MAX = 20 };
 GFR_HD bool sweep_p_local(int lanes, int n) { return lanes == 1 && n <= SWEEP_P_LOCAL_MAX; }
-GFR_HD size_t sweep_slot_bytes(int n, int n_src, bool p_local = false, int n_tie = 0) {
+GFR_HD size_t sweep_slot_bytes(int n, int n_src, bool p_local = false, int n_tie = 0, bool spec_q = false) {
   if (n_src > SCRATCH_FIELDS_SWEEP * n) return 0;
-  const size_t units = ((size_t)n * (p_local ? 32 : 40) + 15) / 16 + 2 * (size_t)n_tie;   // 16-byte units, made odd: neighbouring instances'
+  const size_t units = ((size_t)n * (spec_q ? 48 : p_local ? 32 : 40) + 15) / 16 + 2 * (size_t)n_tie;   // 16-byte units, made odd: neighbouring instances'
   return (units | 1) * 16;                                // slots then start 4 banks apart (conflict-free 128-bit accesses)
 }
 // Points a group at its instance slot: `slot` in shared memory, `mg` its global scratch (Newton), `p_local` the
 // thread's own array of SWEEP_P_LOCAL_MAX doubles (sweep, one lane; a caller that passes none points g.pp at its own)
-template <int LANES>
+// (SPEC_Q: the kernels with specified Q, see sweep_slot_bytes)
+template <int LANES, bool SPEC_Q = false>
 GFR_HD void bind_slot(NGrp<LANES>& g, unsigned char* slot, const Layout& lay, D2* mg, double* = nullptr) {
   g.np = lay.n_pool;
   g.efp = reinterpret_cast<D2*>(slot);
@@ -348,17 +375,17 @@ GFR_HD void bind_slot(NGrp<LANES>& g, unsigned char* slot, const Layout& lay, D2
   g.mg = mg;
   g.pol = scratch_policy();
 }
-template <int LANES>
+template <int LANES, bool SPEC_Q = false>
 GFR_HD void bind_slot(SGrp<LANES>& g, unsigned char* slot, const Layout& lay, D2*, double* p_local = nullptr) {
   const int n = lay.n;
   g.efp = reinterpret_cast<D2*>(slot);
   g.jrp = g.efp + n;
   g.pp = reinterpret_cast<double*>(g.jrp + n);
-  g.jt = g.jrp + n + (sweep_p_local(LANES, n) ? 0 : (n + 1) / 2);      // after the injections, when they live here
+  g.jt = g.jrp + n + (SPEC_Q ? n : sweep_p_local(LANES, n) ? 0 : (n + 1) / 2);      // after the injections, when they live here
   g.n = n;
   // one thread per instance on a small feeder: the specified injections live in the thread's local array (the host
   // sized the shared-memory slot without them)
-  if (sweep_p_local(LANES, n)) g.pp = p_local;
+  if (!SPEC_Q && sweep_p_local(LANES, n)) g.pp = p_local;
 }
 
 
@@ -670,7 +697,8 @@ GFR_HD void put_hand_off(D2* e, int np, const D2 h0, const D2 h1, const D2 hc, c
 // schedule: every branch is evaluated ONCE, by the bus below it, which keeps its own share (ga, al) and hands the
 // parent's share (gl, ll) up - in registers to an heir's parent, through field 3 of its pool slot otherwise.
 // Same arithmetic, term by term and in the same order, as the elimination pass.
-template <int LANES>
+// SPEC_Q: PQ buses have a specified Q (the reference's Q_spec row filled in); without it Q_spec = 0, as there.
+template <int LANES, bool SPEC_Q = false>
 GFR_HD double newton_mismatch(const NGrp<LANES>& g, const Layout& lay, const int* simg, const double* dimg) {
   const int nrows = lay.nrows, np = lay.n_pool;
   const I4* sched = reinterpret_cast<const I4*>(simg + lay.o_sched);
@@ -680,7 +708,7 @@ GFR_HD double newton_mismatch(const NGrp<LANES>& g, const Layout& lay, const int
   const I4* kids = reinterpret_cast<const I4*>(simg + (wide_group<LANES>() ? lay.o_kids : 0));
   double mm = 0.0;
   D2 hf; hf.x = hf.y = 0.0;                             // (gl, ll) of the bus this lane handled in the previous row
-  double ps_next = g.pspec((nrows - 1) * LANES + g.lane);
+  typename SpecT<SPEC_Q>::type ps_next = spec_of<SPEC_Q>(g, (nrows - 1) * LANES + g.lane);
   const auto row_in = [&](int p) {
     RowIn r = {sched[p], I4(), gb[p], gbd[p]};
     if (wide_group<LANES>()) r.kq = kids[p];
@@ -693,8 +721,8 @@ GFR_HD double newton_mismatch(const NGrp<LANES>& g, const Layout& lay, const int
     const RowIn in = ahead.take(row_in, p, row > 0, p - LANES);
     const I4 t = in.t;                                  // idle positions: record 0 -> bus 0, harmless
     const D2 vk = g.ef(rec_bus(t)), vp = g.ef(rec_parent(t));
-    const double ps = ps_next;
-    if (row > 0) ps_next = g.pspec(p - LANES);
+    const auto ps = ps_next;
+    if (row > 0) ps_next = spec_of<SPEC_Q>(g, p - LANES);
     if (t.z & FL_VALID) {
       const double v2 = fma(vk.x, vk.x, vk.y * vk.y);
       const BranchT bt = branch_terms(vk, vp, in.y);
@@ -704,7 +732,7 @@ GFR_HD double newton_mismatch(const NGrp<LANES>& g, const Layout& lay, const int
         hf.x += fl.x; hf.y += fl.y;
       });
       const double P = fma(in.yd.x, v2, bt.ga) + hf.x, Q = fma(-in.yd.y, v2, bt.al) + hf.y;
-      double aP = fabs(ps - P), aQ = fabs(Q);
+      double aP = fabs(spec_p(ps) - P), aQ = SPEC_Q ? fabs(spec_q(ps) - Q) : fabs(Q);
       if ((t.z & (FL_PQ | FL_THETA)) != (FL_PQ | FL_THETA)) {   // slack: no equations; PV: no Q equation
         if (!(t.z & FL_THETA)) aP = 0.0;
         if (!(t.z & FL_PQ)) aQ = 0.0;
@@ -794,7 +822,9 @@ GFR_HD void newton_back_update(const NGrp<LANES>& g, const Layout& lay, const in
   }
 }
 
-template <int LANES>
+// SPEC_Q: PQ buses have a specified Q (right-hand side and mismatch only: the flat-start factors f0 do not depend on
+// the injections)
+template <int LANES, bool SPEC_Q = false>
 GFR_HD void newton_solve(const NGrp<LANES>& g, const Layout& lay, const int* simg,
                          const double* dimg, double tol, int max_it, double accel,
                          SolveStat* out) {
@@ -822,7 +852,8 @@ GFR_HD void newton_solve(const NGrp<LANES>& g, const Layout& lay, const int* sim
       for (int p = g.lane; p < P; p += LANES) {
         const int fl = sched[p].z;
         const D2 pc = f0[5 * P + p];
-        double aP = fabs(g.pspec(p) - pc.x), aQ = fabs(pc.y);
+        const auto s = spec_of<SPEC_Q>(g, p);
+        double aP = fabs(spec_p(s) - pc.x), aQ = SPEC_Q ? fabs(spec_q(s) - pc.y) : fabs(pc.y);
         if (!(fl & FL_THETA)) aP = 0.0;
         if (!(fl & FL_PQ)) aQ = 0.0;
         const double loc = max_nan(aP, aQ);
@@ -836,7 +867,7 @@ GFR_HD void newton_solve(const NGrp<LANES>& g, const Layout& lay, const int* sim
         break;
       }
       D2 hc; hc.x = hc.y = 0.0;                         // L v of the bus this lane eliminated in the previous row
-      double ps_next = g.pspec((nrows - 1) * LANES + g.lane);     // the specified injection, one row ahead (an L2 round trip)
+      typename SpecT<SPEC_Q>::type ps_next = spec_of<SPEC_Q>(g, (nrows - 1) * LANES + g.lane);   // the specified injection, one row ahead (an L2 round trip)
       struct F0In { I4 t, kq; D2 pc, i0, i1, lp; };   // record, packed tails, flat-profile (P, Q), D^-1 rows, (ll, gl)
       const auto f0_in = [&](int p) {
         F0In r = {sched[p], I4(), f0[5 * P + p], f0[p], f0[P + p], f0[4 * P + p]};
@@ -849,8 +880,8 @@ GFR_HD void newton_solve(const NGrp<LANES>& g, const Layout& lay, const int* sim
         const int p = row * LANES + g.lane;
         const F0In in = ahead.take(f0_in, p, row > 0, p - LANES);
         const I4 t = in.t;
-        const double ps = ps_next;
-        if (row > 0) ps_next = g.pspec(p - LANES);
+        const auto ps = ps_next;
+        if (row > 0) ps_next = spec_of<SPEC_Q>(g, p - LANES);
         if (t.z & FL_VALID) {
           if (!(t.z & FL_C_REG)) { hc.x = hc.y = 0.0; }
           for_each_tail<LANES>(t, in.kq, child_slot, [&](int slot) {
@@ -858,7 +889,7 @@ GFR_HD void newton_solve(const NGrp<LANES>& g, const Layout& lay, const int* sim
             hc.x += cc.x; hc.y += cc.y;
           });
           const D2 sc = hc;
-          double r0 = ps - in.pc.x - sc.x, r1 = 0.0 - in.pc.y - sc.y;
+          double r0 = spec_p(ps) - in.pc.x - sc.x, r1 = spec_q(ps) - in.pc.y - sc.y;
           if (!(t.z & FL_THETA)) r0 = 0.0;
           if (!(t.z & FL_PQ)) r1 = 0.0;
           D2 v;
@@ -880,7 +911,7 @@ GFR_HD void newton_solve(const NGrp<LANES>& g, const Layout& lay, const int* sim
       // ---- the iterate is expected to have converged (quadratic rate seen so far): a mismatch-only
       //      pass settles it without the elimination
       if (rate * mm_prev * mm_prev < 0.25 * tol) {
-        mm = newton_mismatch(g, lay, simg, dimg);
+        mm = newton_mismatch<LANES, SPEC_Q>(g, lay, simg, dimg);
         if (mm < tol) {
           out->max_mismatch = mm;
           out->converged = 1;
@@ -894,7 +925,7 @@ GFR_HD void newton_solve(const NGrp<LANES>& g, const Layout& lay, const int* sim
       int singular = 0;
       D2 h0, h1, hc, hf;                               // what the bus this lane eliminated in the previous row hands up
       h0.x = h0.y = h1.x = h1.y = hc.x = hc.y = hf.x = hf.y = 0.0;
-      double ps_next = g.pspec((nrows - 1) * LANES + g.lane);     // the specified injection, one row ahead (an L2 round trip)
+      typename SpecT<SPEC_Q>::type ps_next = spec_of<SPEC_Q>(g, (nrows - 1) * LANES + g.lane);   // the specified injection, one row ahead (an L2 round trip)
       const auto row_in = [&](int p) {
         RowIn r = {sched[p], I4(), gb[p], gbd[p]};
         if (wide_group<LANES>()) r.kq = kids[p];
@@ -907,8 +938,8 @@ GFR_HD void newton_solve(const NGrp<LANES>& g, const Layout& lay, const int* sim
         const RowIn in = ahead.take(row_in, p, row > 0, p - LANES);
         const I4 t = in.t;
         const D2 vk = g.ef(rec_bus(t)), vp = g.ef(rec_parent(t)), yd = in.yd;
-        const double ps = ps_next;
-        if (row > 0) ps_next = g.pspec(p - LANES);
+        const auto ps = ps_next;
+        if (row > 0) ps_next = spec_of<SPEC_Q>(g, p - LANES);
         if (t.z & FL_VALID) {
           const double v2 = fma(vk.x, vk.x, vk.y * vk.y);
           const BranchT bt = branch_terms(vk, vp, in.y);
@@ -918,9 +949,9 @@ GFR_HD void newton_solve(const NGrp<LANES>& g, const Layout& lay, const int* sim
           const D2 s0 = h0, s1 = h1, sc = hc, sf = hf;
           const double Pk = fma(yd.x, v2, bt.ga) + sf.x, Q = fma(-yd.y, v2, bt.al) + sf.y;
           D2 d0, d1, r;
-          r.x = ps - Pk;
-          r.y = 0.0 - Q;
-          double aP = fabs(r.x), aQ = fabs(Q);
+          r.x = spec_p(ps) - Pk;
+          r.y = spec_q(ps) - Q;
+          double aP = fabs(r.x), aQ = SPEC_Q ? fabs(r.y) : fabs(Q);
           r.x -= sc.x; r.y -= sc.y;
           d0.x = fma(-yd.y, v2, -Q) - s0.x;             // -Q - B v2
           d0.y = fma(yd.x, v2, Pk) - s0.y;              //  P + G v2
@@ -1025,7 +1056,13 @@ GFR_HD void add_tie_current(const int* tie_ptr, const int* tie_inc, const D2* jt
     else { a.x -= j.x; a.y -= j.y; }
   }
 }
-template <int LANES, bool TIES>
+// SPEC_Q: PQ buses inject P + jQ, a current conj(S / V) = (P - jQ) V / |V|^2 (added to a); else Q = 0.
+GFR_HD void add_pq_current(const D2 s, const D2 v, D2& a) {
+  const double r = rcp_fast(fma(v.x, v.x, v.y * v.y)), wp = s.x * r, wq = s.y * r;
+  a.x = fma(wp, v.x, fma(wq, v.y, a.x));
+  a.y = fma(wp, v.y, fma(-wq, v.x, a.y));
+}
+template <int LANES, bool TIES, bool SPEC_Q = false>
 GFR_HD void sweep_solve(const SGrp<LANES>& g, const Layout& lay, const int* simg,
                         const double* dimg, double tol, int max_it, SolveStat* out) {
   const int n = lay.n, nrows = lay.sw_rows, ks = lay.k_slack, nt = TIES ? lay.n_tie : 0;
@@ -1050,15 +1087,21 @@ GFR_HD void sweep_solve(const SGrp<LANES>& g, const Layout& lay, const int* simg
       // hands each subtree current to the parent needs no child lists (and no barriers)
       D2 z0; z0.x = z0.y = 0.0;
       for (int k = 0; k < n; ++k) g.at2(S_JR, k) = z0;
-      double p_next = g.at(S_P, n - 1);                // the injections may live in local memory (L1 / L2): one bus ahead
+      double p_next = SPEC_Q ? 0.0 : g.at(S_P, n - 1);  // the injections may live in local memory (L1 / L2): one bus ahead
       for (int k = n - 1; k >= 0; --k) {
         const I4 t = topo[k];
         const D2 v = g.at2(F_E, k);
-        const double p_k = p_next;
-        if (k > 0) p_next = g.at(S_P, k - 1);
-        const double w = (t.w & FL_THETA) ? p_k * rcp_fast(fma(v.x, v.x, v.y * v.y)) : 0.0;
-        D2 a = g.at2(S_JR, k);
-        a.x = fma(w, v.x, a.x); a.y = fma(w, v.y, a.y);
+        D2 a;
+        if constexpr (SPEC_Q) {                        // (P, Q) in the shared-memory slot: nothing to fetch ahead
+          a = g.at2(S_JR, k);
+          if (t.w & FL_THETA) add_pq_current(g.pqspec(k), v, a);
+        } else {
+          const double p_k = p_next;
+          if (k > 0) p_next = g.at(S_P, k - 1);
+          const double w = (t.w & FL_THETA) ? p_k * rcp_fast(fma(v.x, v.x, v.y * v.y)) : 0.0;
+          a = g.at2(S_JR, k);
+          a.x = fma(w, v.x, a.x); a.y = fma(w, v.y, a.y);
+        }
         add_tie_current(tie_ptr, tie_inc, g.jt, nt, k, a);
         g.at2(S_JR, k) = a;
         if (k > 0) { D2& ap = g.at2(S_JR, t.x); ap.x += a.x; ap.y += a.y; }
@@ -1073,9 +1116,14 @@ GFR_HD void sweep_solve(const SGrp<LANES>& g, const Layout& lay, const int* simg
         if (t.w & FL_VALID) {
           const int k = t.x & 0xffff;
           const D2 v = g.at2(F_E, k);
-          const double w = (t.w & FL_THETA) ? g.at(S_P, k) * rcp_fast(fma(v.x, v.x, v.y * v.y)) : 0.0;   // conj(S / V) = P V / |V|^2
           D2 a;
-          a.x = w * v.x; a.y = w * v.y;
+          if constexpr (SPEC_Q) {
+            a.x = a.y = 0.0;
+            if (t.w & FL_THETA) add_pq_current(g.pqspec(k), v, a);
+          } else {
+            const double w = (t.w & FL_THETA) ? g.at(S_P, k) * rcp_fast(fma(v.x, v.x, v.y * v.y)) : 0.0;   // conj(S / V) = P V / |V|^2
+            a.x = w * v.x; a.y = w * v.y;
+          }
           add_tie_current(tie_ptr, tie_inc, g.jt, nt, k, a);
 #pragma unroll 1
           for (int q = t.y; q < t.z; ++q) {
@@ -1254,30 +1302,36 @@ GFR_HD void line_flow(const G& g, const Layout& lay, const int* simg, const doub
 
 typedef gfr_sol_out SolOut;      // the caller's output table, as the C ABI declares it
 
-template <int SOLVER, int LANES>
+template <int SOLVER, bool SPEC_Q = false, int LANES>
 GFR_HD void run_solver(const NGrp<LANES>& g, const Layout& lay, const int* simg, const double* dimg,
                        const EnvCfg& cfg, SolveStat* st) {
-  newton_solve(g, lay, simg, dimg, cfg.tol, cfg.max_it, cfg.accel, st);
+  newton_solve<LANES, SPEC_Q>(g, lay, simg, dimg, cfg.tol, cfg.max_it, cfg.accel, st);
 }
-template <int SOLVER, int LANES>
+template <int SOLVER, bool SPEC_Q = false, int LANES>
 GFR_HD void run_solver(const SGrp<LANES>& g, const Layout& lay, const int* simg, const double* dimg,
                        const EnvCfg& cfg, SolveStat* st) {
-  sweep_solve<LANES, SOLVER == SOLVER_SWEEP_TIES>(g, lay, simg, dimg, cfg.tol, cfg.max_it, st);
+  sweep_solve<LANES, SOLVER == SOLVER_SWEEP_TIES, SPEC_Q>(g, lay, simg, dimg, cfg.tol, cfg.max_it, st);
 }
 
-template <int LANES, int SOLVER>
+// One solve: p_inj [B, n] (and, SPEC_Q, q_inj [B, n]) pu in ref bus order; the results into `o`
+template <int LANES, int SOLVER, bool SPEC_Q = false>
 GFR_HD void solve_instance(const typename GroupOf<LANES, SOLVER>::type& g, const Layout& lay,
                            const int* simg, const double* dimg, const EnvCfg& cfg, long long env,
-                           const double* p_inj, const SolOut& o) {
+                           const double* p_inj, const SolOut& o, const double* q_inj = nullptr) {
   const int n = lay.n, m = lay.m;
   const int* rank = simg + lay.o_rank;
   const int* rankp = simg + lay.o_rankp;
   const double* pin = p_inj + env * n;
-  for (int i = g.lane; i < n; i += LANES) g.set_pspec(rankp[i], pin[i]);
+  if constexpr (SPEC_Q) {
+    const double* qin = q_inj + env * n;
+    for (int i = g.lane; i < n; i += LANES) { D2 s; s.x = pin[i]; s.y = qin[i]; g.set_pqspec(rankp[i], s); }
+  } else {
+    for (int i = g.lane; i < n; i += LANES) g.set_pspec(rankp[i], pin[i]);
+  }
   g.sync();          // a position's injection is read by the lane that owns the position, not the one that owns ref bus i
   flat_start(g, lay, simg, dimg);
   SolveStat st;
-  run_solver<SOLVER>(g, lay, simg, dimg, cfg, &st);
+  run_solver<SOLVER, SPEC_Q>(g, lay, simg, dimg, cfg, &st);
   for (int i = g.lane; i < n; i += LANES) {
     int k = rank[i];
     const D2 vv = g.ef(k);

@@ -11,6 +11,11 @@ Both call shapes are accepted.  Quantities are taken in the units the caller use
 like the reference solver (which never converts): pass per-unit injections with per-unit
 impedances.  The two-argument form with a ``{'loads': {bus: W}, 'generation': {bus: W}}`` dict
 divides by the feeder's base power first (deviation D1, DESIGN.md).
+
+Specified reactive power (the reference's ``Q_spec`` row, which it leaves at 0) goes in as ``q_inj``
+[B, n] pu next to ``p_inj``, as a ``(p, q)`` tuple in place of ``p_inj``, or as ``'reactive_loads'`` /
+``'reactive_generation'`` ({bus: var}) in the two-argument form's dict.  Q entries of the slack and of PV
+buses are ignored.  The reference's four-argument form stays active power only, as its signature is.
 """
 
 from __future__ import annotations
@@ -67,6 +72,28 @@ class NativeNetwork:
             self.close()
         except Exception:
             pass
+
+
+def _injections(p_inj, q_inj, n: int, dev):
+    """(p, q) as [B, n] float64 tensors on ``dev`` (q None when no reactive power is given); ``p_inj`` may be a
+    ``(p, q)`` pair."""
+    if q_inj is None and isinstance(p_inj, tuple) and len(p_inj) == 2:
+        p_inj, q_inj = p_inj
+
+    def one(x, name):
+        t = torch.as_tensor(x)
+        if t.dim() == 1:
+            t = t[None, :]
+        if t.dim() != 2 or t.shape[1] != n:
+            raise InvalidConfigurationError(f"{name} must be [B, {n}], got {tuple(t.shape)}")
+        return t.to(device=dev, dtype=torch.float64).contiguous()
+    p = one(p_inj, "p_inj")
+    if q_inj is None:
+        return p, None
+    q = one(q_inj, "q_inj")
+    if q.shape != p.shape:
+        raise InvalidConfigurationError(f"q_inj must have the shape of p_inj {tuple(p.shape)}, got {tuple(q.shape)}")
+    return p, q
 
 
 def is_radial(buses, lines) -> bool:
@@ -149,15 +176,11 @@ class B200PowerFlowSolver:
             self._cache[key] = net
         return net
 
-    def solve_network_batch(self, net: NativeNetwork, p_inj) -> PowerFlowSolution:
-        """The dense path: ``p_inj`` [B, n] per-unit injections in the network's bus order."""
+    def solve_network_batch(self, net: NativeNetwork, p_inj, q_inj=None) -> PowerFlowSolution:
+        """The dense path: ``p_inj`` (and ``q_inj``, or None for Q_spec = 0) [B, n] per-unit injections in the
+        network's bus order."""
         dev, lib = net.device, net.lib
-        p = torch.as_tensor(p_inj)
-        if p.dim() == 1:
-            p = p[None, :]
-        if p.shape[1] != net.n_bus:
-            raise InvalidConfigurationError(f"p_inj must be [B, {net.n_bus}], got {tuple(p.shape)}")
-        p = p.to(device=dev, dtype=torch.float64).contiguous()
+        p, q = _injections(p_inj, q_inj, net.n_bus, dev)
         B, n, m = p.shape[0], net.n_bus, net.n_line
         f64 = dict(dtype=torch.float64, device=dev)
         out = dict(converged=torch.zeros(B, dtype=torch.uint8, device=dev),
@@ -168,21 +191,24 @@ class B200PowerFlowSolver:
         so = nat.SolOut(*[out[k].data_ptr() for k, _ in nat.SolOut._fields_])
         cfg = nat.make_solver_cfg("newton", self.tolerance, self.max_iterations, self.acceleration_factor,
                                   self.dense_kernel)
-        nat.check(lib, lib.gfr_network_solve(net.handle, B, p.data_ptr(), C.byref(cfg), C.byref(so),
-                                             torch.cuda.current_stream(dev).cuda_stream))
+        nat.check(lib, lib.gfr_network_solve_pq(net.handle, B, p.data_ptr(), None if q is None else q.data_ptr(),
+                                                C.byref(cfg), C.byref(so), torch.cuda.current_stream(dev).cuda_stream))
         out["converged"] = out["converged"].view(torch.bool)
         return PowerFlowSolution(**out)
 
-    def solve_batch(self, feeder, p_inj) -> PowerFlowSolution:
-        """``p_inj`` [B, n] per-unit injections (generation minus load) in ``feeder.buses`` order;
+    def solve_batch(self, feeder, p_inj, q_inj=None) -> PowerFlowSolution:
+        """``p_inj`` [B, n] per-unit injections (generation minus load) in ``feeder.buses`` order, and
+        ``q_inj`` [B, n] their reactive parts (None: Q_spec = 0; ``p_inj`` may also be a ``(p, q)`` pair);
         returns a ``PowerFlowSolution`` of tensors with a leading B axis."""
+        if q_inj is None and isinstance(p_inj, tuple) and len(p_inj) == 2:
+            p_inj, q_inj = p_inj
         if isinstance(feeder, NativeNetwork):
-            return self.solve_network_batch(feeder, p_inj)
+            return self.solve_network_batch(feeder, p_inj, q_inj)
         sweep_ties = False
         if not isinstance(feeder, (NativeFeeder, FeederSoA)) and self._use_dense(feeder.buses, feeder.lines):
             s_base = float(feeder.parameters.base_power) * 1e6
             try:
-                return self.solve_network_batch(self._network(feeder.buses, feeder.lines, s_base), p_inj)
+                return self.solve_network_batch(self._network(feeder.buses, feeder.lines, s_base), p_inj, q_inj)
             except GridLimitError:
                 # the dense Jacobian does not fit an SM (e.g. IEEE-123 with its 26 tie lines: 244 unknowns):
                 # "auto" falls back to the sweep on the spanning tree with the loops restored by compensation
@@ -200,12 +226,7 @@ class B200PowerFlowSolver:
             nf = self._native(("feeder", id(feeder), _signature(feeder.buses, feeder.lines)),
                               lambda: self._compile(feeder))
         dev, soa, lib = nf.device, nf.soa, nf.lib
-        p = torch.as_tensor(p_inj)
-        if p.dim() == 1:
-            p = p[None, :]
-        if p.shape[1] != soa.n_bus:
-            raise InvalidConfigurationError(f"p_inj must be [B, {soa.n_bus}], got {tuple(p.shape)}")
-        p = p.to(device=dev, dtype=torch.float64).contiguous()
+        p, q = _injections(p_inj, q_inj, soa.n_bus, dev)
         B, n, m = p.shape[0], soa.n_bus, soa.n_line
         f64 = dict(dtype=torch.float64, device=dev)
         out = dict(converged=torch.zeros(B, dtype=torch.uint8, device=dev),
@@ -220,8 +241,8 @@ class B200PowerFlowSolver:
         cfg = nat.make_solver_cfg(method, self.tolerance if not sweep_ties else min(self.tolerance, 1e-9), self.max_iterations if not sweep_ties else max(self.max_iterations, 200),
                                   self.acceleration_factor,
                                   self.lanes or getattr(soa, "lanes_hint", 0) or auto_lanes(soa.n_bus, method))
-        nat.check(lib, lib.gfr_solve(nf.handle, B, p.data_ptr(), C.byref(cfg), C.byref(so),
-                                     torch.cuda.current_stream(dev).cuda_stream))
+        nat.check(lib, lib.gfr_solve_pq(nf.handle, B, p.data_ptr(), None if q is None else q.data_ptr(), C.byref(cfg),
+                                        C.byref(so), torch.cuda.current_stream(dev).cuda_stream))
         out["converged"] = out["converged"].view(torch.bool)
         return PowerFlowSolution(**out)
 
@@ -260,7 +281,14 @@ class B200PowerFlowSolver:
                 p[0, index[bus]] -= v / s_base
             for bus, v in loading_conditions.get("generation", {}).items():
                 p[0, index[bus]] += v / s_base
-            return self._unwrap(self.solve_batch(feeder, p))
+            q = None
+            if "reactive_loads" in loading_conditions or "reactive_generation" in loading_conditions:
+                q = np.zeros((1, len(feeder.buses)))
+                for bus, v in loading_conditions.get("reactive_loads", {}).items():
+                    q[0, index[bus]] -= v / s_base
+                for bus, v in loading_conditions.get("reactive_generation", {}).items():
+                    q[0, index[bus]] += v / s_base
+            return self._unwrap(self.solve_batch(feeder, p, q))
         return self.solve_batch(feeder, loading_conditions)
 
     def _unwrap(self, sol: PowerFlowSolution) -> PowerFlowSolution:

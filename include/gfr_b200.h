@@ -237,6 +237,11 @@ int gfr_env_step(gfr_env* e, const double* actions, const double* noise, const g
  * p_inj [B,n] pu in ref bus order (generation minus load; the slack entry is ignored). */
 int gfr_solve(const gfr_feeder* f, int64_t B, const double* p_inj, const gfr_solver_cfg* cfg,
               const gfr_sol_out* out, void* stream);
+/* gfr_solve with specified reactive power: q_inj [B,n] pu in ref bus order (generation minus load, like p_inj).
+ * The Q entries of the slack and of PV buses are ignored (those buses have no Q equation).  q_inj = NULL is
+ * gfr_solve: Q_spec = 0 through the same kernels.  p_inj = NULL -> GFR_E_ARG. */
+int gfr_solve_pq(const gfr_feeder* f, int64_t B, const double* p_inj, const double* q_inj,
+                 const gfr_solver_cfg* cfg, const gfr_sol_out* out, void* stream);
 
 /* ---- meshed networks: the reference's dense Newton-Raphson as written ------------------------
  * NewtonRaphsonSolver.solve on ANY connected network (cycles allowed): dense Ybus
@@ -266,6 +271,10 @@ int gfr_network_unknowns(const gfr_network* net);          /* order of the dense
  * GFR_E_LIMIT. */
 int gfr_network_solve(const gfr_network* net, int64_t B, const double* p_inj, const gfr_solver_cfg* cfg,
                       const gfr_sol_out* out, void* stream);
+/* gfr_network_solve with specified reactive power q_inj [B, n_bus] pu (NULL: Q_spec = 0, as gfr_network_solve);
+ * the slack's and PV buses' entries are ignored. */
+int gfr_network_solve_pq(const gfr_network* net, int64_t B, const double* p_inj, const double* q_inj,
+                         const gfr_solver_cfg* cfg, const gfr_sol_out* out, void* stream);
 
 /* The noise rows the in-kernel generator yields: out [B, n_slots] for keys seeds[B] and draw
  * counters draws[B] (slot 0 uniform, slots 1.. standard normal). */
