@@ -267,7 +267,8 @@ class PortEnv:
                  stochastic_loads: bool = True, renewable_sources: Optional[Sequence[str]] = None,
                  weather_variation: bool = True, voltage_limits=(0.95, 1.05),
                  frequency_limits=(59.5, 60.5), safety_penalty: float = 100.0,
-                 tolerance: float = 1e-6, max_iterations: int = 50) -> None:
+                 tolerance: float = 1e-6, max_iterations: int = 50, acceleration: float = 1.0) -> None:
+        """``acceleration``: the factor of the Newton update (the reference's ``acceleration_factor``)."""
         self.B = int(num_envs)
         self.net = DenseNetwork(feeder.buses, feeder.lines)
         self.s_base = float(feeder.parameters.base_power) * 1e6
@@ -276,7 +277,7 @@ class PortEnv:
         self.v_lo, self.v_hi = voltage_limits
         self.f_lo, self.f_hi = frequency_limits
         self.penalty = float(safety_penalty)
-        self.tol, self.max_it = tolerance, max_iterations
+        self.tol, self.max_it, self.accel = tolerance, max_iterations, float(acceleration)
         idx = self.net.index
         self.load_bus = np.array([idx[l.bus] for l in feeder.loads], dtype=np.int64)
         self.load_base = np.array([float(l.base_power) for l in feeder.loads])
@@ -448,7 +449,7 @@ class PortEnv:
         p_spec = np.zeros((b, self.n))
         p_spec -= loads_w / self.s_base
         p_spec += gen_w / self.s_base
-        sol = newton_raphson(self.net, p_spec, self.tol, self.max_it)
+        sol = newton_raphson(self.net, p_spec, self.tol, self.max_it, self.accel)
         flows_w = sol["line_flows"] * self.s_base
         losses_w = sol["losses"] * self.s_base
         # --- state update (grid_env.py:722-739, base.py:261-264)

@@ -92,7 +92,8 @@ class EmuEnv:
         return out
 
 
-def emu_solve(feeder, p_inj, solver="newton", tolerance=1e-6, max_iterations=50, lanes=0, emu_lanes=None):
+def emu_solve(feeder, p_inj, solver="newton", tolerance=1e-6, max_iterations=50, lanes=0, emu_lanes=None,
+              acceleration=1.0):
     soa, used = compile_for_solver(feeder, solver, lanes, with_components=False)
     if emu_lanes is None:
         emu_lanes = used if used in EMU_LANES else 1
@@ -103,7 +104,7 @@ def emu_solve(feeder, p_inj, solver="newton", tolerance=1e-6, max_iterations=50,
                bus_voltages=np.zeros((B, n)), bus_angles=np.zeros((B, n)), line_flows=np.zeros((B, m)),
                line_loadings=np.zeros((B, m)), losses=np.zeros(B), max_mismatch=np.zeros(B))
     so = nat.SolOut(*[out[k].ctypes.data for k, _ in nat.SolOut._fields_])
-    cfg = nat.make_solver_cfg(solver, tolerance, max_iterations, lanes=emu_lanes)
+    cfg = nat.make_solver_cfg(solver, tolerance, max_iterations, acceleration, lanes=emu_lanes)
     rc = lib().emu_solve(C.byref(desc), B, p.ctypes.data, C.byref(cfg), C.byref(so))
     assert rc == 0
     return out

@@ -41,9 +41,10 @@ def lib():
     return _LIB
 
 
-def emu_solve_pq(feeder, p_inj, q_inj, solver="newton", tolerance=1e-6, max_iterations=50, lanes=0, emu_lanes=None):
+def emu_solve_pq(feeder, p_inj, q_inj, solver="newton", tolerance=1e-6, max_iterations=50, lanes=0, emu_lanes=None,
+                 acceleration=1.0):
     """The Q kernels' solve of ``p_inj`` / ``q_inj`` [B, n] (pu, ``feeder.buses`` order) on the host; same arguments
-    and result dict as ``emu.emu_solve``."""
+    and result dict as ``emu.emu_solve``, and the acceleration factor of the Newton update."""
     soa, used = compile_for_solver(feeder, solver, lanes, with_components=False)
     if emu_lanes is None:
         emu_lanes = used if used in EMU_LANES else 1
@@ -55,7 +56,7 @@ def emu_solve_pq(feeder, p_inj, q_inj, solver="newton", tolerance=1e-6, max_iter
                bus_voltages=np.zeros((B, n)), bus_angles=np.zeros((B, n)), line_flows=np.zeros((B, m)),
                line_loadings=np.zeros((B, m)), losses=np.zeros(B), max_mismatch=np.zeros(B))
     so = nat.SolOut(*[out[k].ctypes.data for k, _ in nat.SolOut._fields_])
-    cfg = nat.make_solver_cfg(solver, tolerance, max_iterations, lanes=emu_lanes)
+    cfg = nat.make_solver_cfg(solver, tolerance, max_iterations, acceleration, lanes=emu_lanes)
     rc = lib().emu_solve_pq(C.byref(desc), B, p.ctypes.data, q.ctypes.data, C.byref(cfg), C.byref(so))
     assert rc == 0
     return out

@@ -744,10 +744,12 @@ def test_dense_and_tree_solvers_agree_on_radial_feeders():
 @pytest.mark.parametrize("num_buses,conn,seed", [(9, 0.3, 1), (14, 0.2, 2), (28, 0.08, 3), (33, 0.06, 4),
                                                  (47, 0.04, 5), (49, 0.04, 6), (60, 0.03, 7), (70, 0.03, 8)])
 def test_dense_register_and_shared_memory_kernels_agree(num_buses, conn, seed):
-    """The register-resident Gauss-Jordan elimination (every tile shape: <= 31, <= 63, <= 95, <= 127
-    unknowns, sizes on both sides of each boundary) against the shared-memory LU: same pivots, so
-    the same convergence flags and iteration counts and the same state to rounding; above 127
-    unknowns "auto" is the shared-memory kernel and "registers" is refused."""
+    """The register-resident Gauss-Jordan elimination against the shared-memory LU on eight meshes with 16, 26, 54,
+    64, 92, 96, 118 and 138 unknowns (register tiles R = 2, 4, 7, 8, 12, 12, 15: both sides of the switches from 8 to
+    16 to 32 thread columns at 56 and 96 unknowns, and one network beyond the register kernel's 127): same pivots,
+    so the same convergence flags and iteration counts and the same state to rounding; above 127 unknowns "auto" is
+    the shared-memory kernel and "registers" is refused.  Every R, odd and even N, against the oracle:
+    tests/test_gpu_newton_iterates.py."""
     import grid_fed_rl_b200 as m
     f = m.repair_topology(m.SyntheticFeeder(m.NetworkConfig(num_buses=num_buses, connectivity=conn,
                                                             load_probability=0.9, dg_probability=0.3), seed=seed),

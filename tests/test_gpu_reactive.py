@@ -24,7 +24,9 @@ def _pf_batch(f, B, seed, lo=0.3, hi=1.0):
     return s * p0, s * q0
 
 
-def _check(sol, ref, iterations=True, rows=slice(None)):
+def _check(sol, ref, f, tol, iterations=True, rows=slice(None)):
+    """Converged rows: the state and losses within TOL_PU; line loadings (|S| s_base / rating on the solve surface,
+    |S| / rating in the oracle) within what a TOL_PU error of |S| allows; the mismatch below the tolerance ``tol``."""
     ok = ref["converged"]
     assert ok.any()
     conv = sol.converged.cpu().numpy()[rows]
@@ -32,8 +34,14 @@ def _check(sol, ref, iterations=True, rows=slice(None)):
     if iterations:
         assert np.array_equal(conv, ok)
         assert np.all(np.abs(sol.iterations.cpu().numpy()[rows].astype(int) - ref["iterations"]) <= 1)
-    for k in ("bus_voltages", "bus_angles", "line_flows"):
+    for k in ("bus_voltages", "bus_angles", "line_flows", "losses"):
         assert np.max(np.abs(getattr(sol, k).cpu().numpy()[rows][ok] - ref[k][ok])) <= TOL_PU, k
+    s_base = float(f.parameters.base_power) * 1e6
+    got, want = sol.line_loadings.cpu().numpy()[rows][ok], ref["line_loadings"][ok] * s_base
+    with np.errstate(divide="ignore", invalid="ignore"):
+        per_pu = np.where(ref["line_s_abs"][ok] > 0, want / ref["line_s_abs"][ok], 0.0)   # s_base / rating
+    assert np.all(np.abs(got - want) <= TOL_PU * per_pu + 1e-12), "line_loadings"
+    assert np.all(sol.max_mismatch.cpu().numpy()[rows][ok] < tol), "max_mismatch"
 
 
 def _solver(**kw):
@@ -53,7 +61,7 @@ def test_newton_with_q_matches_oracle(spec, lanes):
         sol = _solver(tolerance=1e-10, lanes=lanes).solve_batch(f, p, q)
     except m.GridLimitError as exc:            # one thread per instance on a 123-bus feeder
         pytest.skip(str(exc))
-    _check(sol, ref)
+    _check(sol, ref, f, 1e-10)
 
 
 @pytest.mark.parametrize("lanes", [1, 8, 32, 64])
@@ -67,7 +75,7 @@ def test_sweep_with_q_matches_oracle(spec, lanes):
         sol = _solver(method="sweep", tolerance=1e-11, max_iterations=300, lanes=lanes).solve_batch(f, p, q)
     except m.GridLimitError as exc:
         pytest.skip(str(exc))
-    _check(sol, ref, iterations=False)
+    _check(sol, ref, f, 1e-11, iterations=False)
 
 
 @pytest.mark.parametrize("where", ["shared", "registers"])
@@ -80,7 +88,7 @@ def test_dense_with_q_matches_oracle(name, where):
     p, q = _pf_batch(f, 12, seed=7, hi=0.7)
     ref = newton_raphson_pq(net, p, q, 1e-10, 30)
     sol = _solver(method="dense", dense_kernel=where, tolerance=1e-10, max_iterations=30).solve_batch(f, p, q)
-    _check(sol, ref)
+    _check(sol, ref, f, 1e-10)
 
 
 @pytest.mark.parametrize("spec", ["ieee34", "meshieee34", "mesh40:3:0.05", "meshieee123"])
@@ -91,7 +99,7 @@ def test_auto_with_q_matches_oracle(spec):
     p, q = _pf_batch(f, 8, seed=3, hi=0.7)
     ref = newton_raphson_pq(port.DenseNetwork(f.buses, f.lines), p, q, 1e-10, 50)
     sol = _solver(method="auto", tolerance=1e-10).solve_batch(f, p, q)
-    _check(sol, ref, iterations=spec != "meshieee123")
+    _check(sol, ref, f, 1e-10, iterations=spec != "meshieee123")
 
 
 def test_full_size_ieee123_newton_8_lanes():
@@ -103,7 +111,7 @@ def test_full_size_ieee123_newton_8_lanes():
     assert bool(sol.converged.all())
     rows = np.sort(np.random.RandomState(12).choice(B, 64, replace=False))
     ref = newton_raphson_pq(port.DenseNetwork(f.buses, f.lines), p[rows], q[rows], 1e-8, 50)
-    _check(sol, ref, rows=rows)
+    _check(sol, ref, f, 1e-8, rows=rows)
 
 
 # ----------------------------------------------------------------------------- P-only callers
@@ -222,7 +230,7 @@ def test_pv_and_slack_q_entries_change_nothing(method, kw):
     ref = newton_raphson_pq(port.DenseNetwork(f.buses, f.lines), p, q, 1e-10, 50)
     s = _solver(method=method, tolerance=1e-10, **kw)
     a = s.solve_batch(f, p, q)
-    _check(a, ref)
+    _check(a, ref, f, 1e-10)
     q2 = q.copy(); q2[:, [0, 4, 7]] = rs.uniform(-1, 1, size=(32, 3))
     b = s.solve_batch(f, p, q2)
     for k in ("bus_voltages", "bus_angles", "line_flows", "iterations", "converged"):
